@@ -17,11 +17,14 @@ OPT_AUTO_RESET = 1
 OPT_SHARE_SM = 2
 OPT_COMPACT = 4
 FLAG_DONE, FLAG_COLLISION = 1, 2
+POLICY_RANDOM, POLICY_JOINT, POLICY_AGENTS = 0, 1, 2
+EPISODE_TIMEOUT, EPISODE_COLLISION, EPISODE_GOAL, EPISODE_TERMINAL_START = 0, 1, 2, 3
 
 EXPORTS = ["mapf_ctx_create", "mapf_ctx_destroy", "mapf_ctx_info", "mapf_ctx_moves", "mapf_ctx_reward_table", "mapf_decode_states",
            "mapf_encode_states", "mapf_count_rows", "mapf_scan_scratch_bytes", "mapf_scan_rows", "mapf_count_scan_rows",
            "mapf_count_scan_range", "mapf_expand",
            "mapf_count_range", "mapf_expand_range", "mapf_checksum", "mapf_step", "mapf_step_lanes", "mapf_rollout", "mapf_step_host", "mapf_step_host_resident",
+           "mapf_evaluate_scratch_bytes", "mapf_evaluate",
            "mapf_backup", "mapf_backup_range", "mapf_greedy", "mapf_greedy_bcast", "mapf_count_predecessors", "mapf_predecessors",
            "mapf_projected_words", "mapf_project_states", "mapf_parse_map_text", "mapf_parse_scen_text", "mapf_ctx_create_from_text", "mapf_ctx_grid",
            "mapf_group_create", "mapf_group_destroy", "mapf_group_size", "mapf_group_step", "mapf_last_error",
@@ -97,6 +100,9 @@ def lib():
         L.mapf_rollout.argtypes = [vp, vp, vp, i64, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp, vp]
         L.mapf_step_host.argtypes = [vp, vp, vp, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp]
         L.mapf_step_host_resident.argtypes = [vp, vp, vp, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp]
+        L.mapf_evaluate_scratch_bytes.argtypes = []
+        L.mapf_evaluate_scratch_bytes.restype = i64
+        L.mapf_evaluate.argtypes = [vp, i32, vp, i64, i64, i64, C.c_double, u64, u64, i64, vp, vp, vp, vp, vp]
         L.mapf_backup.argtypes = [vp, vp, vp, i64, vp, i64, C.c_double, vp, vp]
         L.mapf_backup_range.argtypes = [vp, C.POINTER(u64 * 2), i64, vp, i64, C.c_double, vp, vp]
         L.mapf_greedy.argtypes = [vp, vp, i64, vp, vp, vp]
@@ -466,6 +472,53 @@ class Engine:
         ns, reward, prob, done, coll = out
         check(lib().mapf_step_host_resident(self._h, _ptr(states_dev), _ptr(actions), B, _ptr(uniforms), seed, step_index,
                                             env_offset, opts, _ptr(ns), _ptr(reward), _ptr(prob), _ptr(done), _ptr(coll)))
+        return out
+
+    # ---- closed-loop policy evaluation -----------------------------------------------------------------------
+    def evaluate(self, policy, n_episodes, max_steps, gamma=1.0, seed=0, step_index=0, episode_offset=0, out=None):
+        """`n_episodes` episodes from the start state under `policy`, each cut at its first done or after `max_steps`
+        steps, in one launch (mapf_evaluate).  Episode e draws what env `episode_offset + e` of `step` draws from
+        `step_index` on.  `policy`: None (uniformly random joint actions, as `rollout` draws them), an int32[nS] tensor
+        of joint actions indexed by the joint state, or an integer [n_agents, L] tensor of per-agent actions indexed by
+        the agent's cell.  Returns (returns f64[E], lengths i32[E], outcomes u8[E]) with outcomes EPISODE_*."""
+        import torch
+        E = int(n_episodes)
+        if E < 0:
+            raise ValueError("n_episodes must be >= 0 (got %d)" % E)
+        if policy is None:
+            kind, table, n_entries = POLICY_RANDOM, None, 0
+        elif not isinstance(policy, torch.Tensor) or policy.dim() not in (1, 2):
+            raise ValueError("policy must be None, an int32[nS] tensor or an integer [n_agents, L] tensor")
+        elif policy.dim() == 1:
+            self._check_tensor("policy", policy, torch.int32)
+            if policy.shape[0] < self.nS:
+                raise ValueError("a joint-state policy needs nS = %d entries (got %d)" % (self.nS, policy.shape[0]))
+            kind, table, n_entries = POLICY_JOINT, policy, policy.shape[0]
+        else:
+            if policy.dtype.is_floating_point or policy.dtype.is_complex or policy.dtype is torch.bool or \
+                    tuple(policy.shape) != (self.n, self.L) or policy.device != self.torch_device:
+                raise ValueError("a per-agent policy must be an integer tensor of shape (%d, %d) on %s (got %s %s on %s)"
+                                 % (self.n, self.L, self.torch_device, policy.dtype, tuple(policy.shape), policy.device))
+            kind, table, n_entries = POLICY_AGENTS, policy, policy.numel()
+        if table is not None and table.numel() > 0:
+            hi = self.nA if kind == POLICY_JOINT else 5
+            lo_v, hi_v = torch.aminmax(table)
+            if int(lo_v) < 0 or int(hi_v) >= hi:
+                raise ValueError("policy entries must lie in [0, %d) (got [%d, %d])" % (hi, int(lo_v), int(hi_v)))
+        if kind == POLICY_AGENTS:
+            table = table.to(torch.uint8).contiguous()
+        dev = self.torch_device
+        if out is None:
+            out = (torch.empty(E, dtype=torch.float64, device=dev), torch.empty(E, dtype=torch.int32, device=dev),
+                   torch.empty(E, dtype=torch.uint8, device=dev))
+        ret, length, outcome = out
+        self._check_tensor("returns", ret, torch.float64, (E,))
+        self._check_tensor("lengths", length, torch.int32, (E,))
+        self._check_tensor("outcomes", outcome, torch.uint8, (E,))
+        scratch = torch.empty((int(lib().mapf_evaluate_scratch_bytes()) + 7) // 8, dtype=torch.int64, device=dev)
+        check(lib().mapf_evaluate(self._h, kind, _ptr(table), n_entries, E, int(max_steps), float(gamma), int(seed),
+                                  int(step_index), int(episode_offset), _ptr(scratch), _ptr(ret), _ptr(length),
+                                  _ptr(outcome), self._stream()))
         return out
 
     # ---- rows next to the hot path (SURVEY.md 8f) ----------------------------------------------------------

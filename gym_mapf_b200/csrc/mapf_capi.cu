@@ -71,6 +71,7 @@ struct mapf_ctx {
     int grid_lanes = 0, grid_lanes_tape = 0;
     LaneConsts lanes;                   // per-lane constants of the lane-per-agent step (k_step_lanes)
     int grid_expand = 0, grid_expand_range = 0, grid_plain = 0, grid_backup = 0, grid_backup_range = 0;
+    int grid_evaluate[3] = {0, 0, 0};   // k_evaluate by policy kind
     KernelSet ks;
     u32 pat_triple[MAPF_MAX_PATTERNS];  // merge patterns (see PatternList)
     int n_patterns = 0;
@@ -627,7 +628,10 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
         {ctx->ks.expand, ctx->smem_expand, &ctx->grid_expand, ctx->threads_expand},
         {ctx->ks.expand_range, ctx->smem_expand, &ctx->grid_expand_range, ctx->threads_expand},
         {ctx->ks.backup, ctx->smem_backup, &ctx->grid_backup},
-        {ctx->ks.backup_range, ctx->smem_backup, &ctx->grid_backup_range}};
+        {ctx->ks.backup_range, ctx->smem_backup, &ctx->grid_backup_range},
+        {ctx->ks.evaluate[MAPF_POLICY_RANDOM], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_RANDOM]},
+        {ctx->ks.evaluate[MAPF_POLICY_JOINT], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_JOINT]},
+        {ctx->ks.evaluate[MAPF_POLICY_AGENTS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_AGENTS]}};
     for (auto &pl : plan) {
         if (!pl.fn) continue;  // two-word states have no backup kernels; the lane-per-agent step covers 2..8 agents
         if (pl.smem > smem_limit) {
@@ -1219,6 +1223,49 @@ extern "C" int mapf_rollout(const mapf_ctx *ctx, void *states_inout, const int32
         LAUNCH(given ? ctx->ks.rollout_philox : ctx->ks.rollout_philox_rnd, grid_for(B, ctx->threads, ctx->grid_rollout),
                ctx->threads, ctx->smem_base, stream, args);
     }
+    return MAPF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// closed-loop policy evaluation
+// ---------------------------------------------------------------------------------------------------------------
+extern "C" int64_t mapf_evaluate_scratch_bytes(void) { return 16; }  // the u32 episode queue counter, padded
+
+extern "C" int mapf_evaluate(const mapf_ctx *ctx, int32_t policy_kind, const void *policy, int64_t policy_len,
+                             int64_t n_episodes, int64_t max_steps, double gamma, uint64_t seed, uint64_t step_index0,
+                             int64_t episode_offset, void *scratch, double *ret, int32_t *length, uint8_t *outcome,
+                             void *stream) {
+    if (!ctx || policy_kind < MAPF_POLICY_RANDOM || policy_kind > MAPF_POLICY_AGENTS || n_episodes < 0 ||
+        (policy_kind != MAPF_POLICY_RANDOM && !policy) || (n_episodes > 0 && (!scratch || !ret || !length || !outcome)))
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate: bad argument");
+    if (max_steps < 1 || max_steps >= (1ll << 31))
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate: max_steps = %lld, must be in [1, 2**31)", (long long)max_steps);
+    if (n_episodes > MAPF_LAUNCH_MAX_ENVS) return fail(MAPF_ERR_INVALID, "mapf_evaluate: at most 2**30 episodes per call");
+    if (policy_kind == MAPF_POLICY_JOINT) {
+        if (ctx->sp.words != 1)
+            return fail(MAPF_ERR_UNSUPPORTED, "mapf_evaluate: a joint-state policy over L**n = %d**%d states cannot exist; "
+                                              "use MAPF_POLICY_AGENTS", ctx->sp.L, ctx->sp.n);
+        if (policy_len < 0 || (u64)policy_len <= ctx->sp.smax[0])
+            return fail(MAPF_ERR_INVALID, "mapf_evaluate: a joint-state policy needs nS = %llu entries (policy_len = %lld)",
+                        (unsigned long long)ctx->sp.smax[0] + 1, (long long)policy_len);
+    }
+    if (policy_kind == MAPF_POLICY_AGENTS && policy_len != (int64_t)ctx->sp.n * ctx->sp.L)
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate: a per-agent policy has n * L = %lld entries (policy_len = %lld)",
+                    (long long)ctx->sp.n * ctx->sp.L, (long long)policy_len);
+    if (!ctx->philox_ok)
+        return fail(MAPF_ERR_UNSUPPORTED, "device-side sampling needs slip probabilities that add up to 1");
+    if (n_episodes == 0) return MAPF_OK;
+    const void *fn = ctx->ks.evaluate[policy_kind];
+    if (!fn) return fail(MAPF_ERR_UNSUPPORTED, "mapf_evaluate: no kernel for policy kind %d", policy_kind);
+    DeviceGuard g(ctx->device);
+    CUDA_TRY(cudaMemsetAsync(scratch, 0, sizeof(u32), (cudaStream_t)stream));
+    DevSpec sp = ctx->sp;
+    PhiloxKeys keys = make_keys(seed);
+    u32 E = (u32)n_episodes, T = (u32)max_steps;
+    u64 st = step_index0, e0 = (u64)episode_offset;
+    void *args[] = {&sp, &keys, &policy, &E, &T, &gamma, &st, &e0, &scratch, &ret, &length, &outcome};
+    LAUNCH(fn, grid_for(n_episodes, ctx->threads, ctx->grid_evaluate[policy_kind]), ctx->threads, ctx->smem_base, stream,
+           args);
     return MAPF_OK;
 }
 

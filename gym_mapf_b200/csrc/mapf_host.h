@@ -23,6 +23,7 @@ struct KernelSet {
     int compact_len_bytes = 0;
     const void *decode = nullptr, *encode = nullptr;
     const void *backup = nullptr, *backup_range = nullptr;  // k_backup<N, LUTS, RANGE>; one-word states only
+    const void *evaluate[3] = {nullptr, nullptr, nullptr};  // k_evaluate<N, W, LUTS, POLICY> by MAPF_POLICY_* kind
     const void *pred_count = nullptr, *pred_emit = nullptr, *project = nullptr;
     size_t expand_slab_bytes = 0;        // per warp
     int expand_threads = 0;              // CTA size of k_expand (0: the context's)

@@ -1497,6 +1497,100 @@ k_rollout(DevSpec sp, PhiloxKeys keys, u64 *states, const int *__restrict__ acti
 }
 
 // =====================================================================================================
+// Closed-loop policy evaluation: whole episodes in registers, one 13-byte record per episode
+// =====================================================================================================
+// Episode e (< E) starts on the start state and takes at most T steps; step t is the step of env e0 + e at step index
+// step0 + t of k_step's Philox stream without auto-reset, with the action the policy picks for the current state:
+//   POLICY 0 (MAPF_POLICY_RANDOM)  the uniform joint action k_rollout draws (random_action)
+//   POLICY 1 (MAPF_POLICY_JOINT)   int32 policy[s], indexed by the one-word joint state
+//   POLICY 2 (MAPF_POLICY_AGENTS)  u8 policy[i * L + cell of agent i]: each agent's action from its own cell
+// The return G = G + disc * r, disc = disc * gamma is accumulated with single binary64 operations (no FMA), and the
+// episode stops at its first done.  Nothing is stored per step: ret / length / outcome of episode e are written when it
+// ends (outcome = the step's kind: 1 clash, 2 goal, 3 the start state was terminal; 0 = no done within T steps).
+// A lane whose episode ends takes the next episode index of the queue (`counter`, one warp-aggregated atomic per warp
+// and refill), so a warp's lanes stay busy until the queue drains instead of waiting for the warp's longest episode.
+// MAPF_EVAL_STATIC (experiment builds only) deals episodes out by grid stride instead.
+template <int N, int WORDS, bool LUTS, int POLICY>
+__global__ void __launch_bounds__(MAPF_MAX_THREADS, MAPF_MIN_BLOCKS(N))
+k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, u32 T, double gamma, u64 step0, u64 e0,
+           u32 *__restrict__ counter, double *__restrict__ ret, int *__restrict__ length, u8 *__restrict__ outcome) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    SmemTables tb = tables_begin<LUTS>(sp, smem);
+    const u32 n_threads = gridDim.x * blockDim.x;
+    u32 e = blockIdx.x * blockDim.x + threadIdx.x;  // the first n_threads episodes are dealt out statically
+    bool live = e < E;
+    EnvIn<N> in;
+    u32 t = 0;
+    double G = 0.0, disc = 1.0;
+    in.lo = sp.s0[0];
+    in.hi = sp.s0[1];
+#pragma unroll
+    for (int i = 0; i < N; ++i) in.cell[i] = (int)sp.start[i];
+    tables_wait<LUTS>(smem);
+#ifndef MAPF_EVAL_STATIC
+    const u32 lane = threadIdx.x & 31u;
+#endif
+    // every lane of a warp stays in the loop until none is live: the refill below is a warp-wide collective
+    while (__any_sync(0xffffffffu, live)) {
+        bool ended = false;
+        if (live) {
+            const u64 env = e0 + (u64)e, stp = step0 + (u64)t;
+            if (POLICY == 0) {
+                load_actions<N>(sp, tb, random_action(sp, keys, env, stp), in.actv);
+            } else if (POLICY == 1) {
+                load_actions<N>(sp, tb, (u32)__ldg(reinterpret_cast<const int *>(policy) + in.lo), in.actv);
+            } else {
+                const u8 *table = reinterpret_cast<const u8 *>(policy);
+#pragma unroll
+                for (int i = 0; i < N; ++i)  // (an out-of-range entry is clamped to LEFT, like load_actions clamps)
+                    in.actv[i] = min((u32)__ldg(table + (u32)i * (u32)sp.L + (u32)in.cell[i]), 4u) * 8u + tb.act0;
+            }
+            env_draws<N>(keys, env, stp, in);
+            int nxt[N];
+            // after a step that was not done the state is not terminal (see env_step): only step 0 needs the test
+            const EnvOut o = env_step<N, WORDS, LUTS, false>(sp, tb, in, nullptr, 0u, nxt, t > 0);
+            G = __dadd_rn(G, __dmul_rn(disc, o.reward));
+            disc = __dmul_rn(disc, gamma);
+            ++t;
+            in.lo = o.lo;
+            in.hi = o.hi;
+#pragma unroll
+            for (int i = 0; i < N; ++i) in.cell[i] = nxt[i];
+            if (o.kind != 0u || t == T) {
+                ret[e] = G;
+                length[e] = (int)t;
+                outcome[e] = (u8)o.kind;
+                ended = true;
+            }
+        }
+#ifdef MAPF_EVAL_STATIC
+        if (ended) e += n_threads;
+#else
+        const u32 fin = __ballot_sync(0xffffffffu, ended);
+        if (fin) {
+            u32 base = 0;
+            if (lane == (u32)(__ffs(fin) - 1)) base = atomicAdd(counter, (u32)__popc(fin));
+            base = __shfl_sync(0xffffffffu, base, __ffs(fin) - 1);
+            if (ended) e = n_threads + base + (u32)__popc(fin & ((1u << lane) - 1u));
+        }
+#endif
+        if (ended) {
+            live = e < E;
+            t = 0;
+            G = 0.0;
+            disc = 1.0;
+            in.lo = sp.s0[0];
+            in.hi = sp.s0[1];
+#pragma unroll
+            for (int i = 0; i < N; ++i) in.cell[i] = (int)sp.start[i];
+        }
+    }
+#ifdef MAPF_EVAL_STATIC
+    (void)counter;
+#endif
+}
+
+// =====================================================================================================
 // Heterogeneous batches (SURVEY.md 8f row 4): envs of DIFFERENT specs (grid, starts/goals, rewards) in one launch
 // =====================================================================================================
 // The batch is a concatenation of per-spec segments (seg_begin[i] .. seg_begin[i + 1] belong to spec i).  Every CTA

@@ -95,6 +95,19 @@ def get_local_view(env: MapfEnv, agent_indexes: list, **kwargs):
                    device=env.device)
 
 
+def independent_policy(env: MapfEnv, gamma=1.0, eps=1e-6, max_iter=1000):
+    """The product of single-agent optimal policies: for each agent i, `value_iteration` of the one-agent view
+    `get_local_view(env, [i])` (same grid, so its states are the joint env's cell ids).  Returns int32[n_agents, L]:
+    agent i on cell c intends action [i, c] -- the per-agent policy `VecMapfEnv.evaluate` takes."""
+    import torch
+    from .vec_env import VecMapfEnv
+    rows = []
+    for i in range(env.n_agents):
+        _, pi, _ = VecMapfEnv(get_local_view(env, [i]), 1).value_iteration(gamma=gamma, eps=eps, max_iter=max_iter)
+        rows.append(pi)
+    return torch.stack(rows).contiguous()
+
+
 def mapf_env_load_from_json(json_str: str) -> MapfEnv:
     raise NotImplementedError()
 

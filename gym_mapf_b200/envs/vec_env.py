@@ -12,6 +12,21 @@ import numpy as np
 
 Transitions = collections.namedtuple("Transitions", "row_ptr next_state prob reward flags")
 Rollout = collections.namedtuple("Rollout", "next_state reward prob done collision")
+# per episode: return f64, length i32 (steps taken), outcome u8 (0 timeout, 1 collision, 2 goal, 3 the start was terminal)
+Evaluation = collections.namedtuple("Evaluation", "returns lengths outcomes")
+
+
+def evaluation_summary(ev):
+    """dict of the usual policy statistics of an Evaluation: mean / (population) standard deviation of the return, the
+    shares of episodes that reached the goal, collided or ran out of steps, and the mean episode length."""
+    from .. import _native
+    n = ev.returns.numel()
+    if n == 0:
+        raise ValueError("an empty Evaluation has no statistics")
+    rate = lambda code: float((ev.outcomes == code).sum().item()) / n  # noqa: E731
+    return dict(mean_return=float(ev.returns.mean().item()), std_return=float(ev.returns.std(correction=0).item()),
+                success_rate=rate(_native.EPISODE_GOAL), collision_rate=rate(_native.EPISODE_COLLISION),
+                timeout_rate=rate(_native.EPISODE_TIMEOUT), mean_length=float(ev.lengths.double().mean().item()))
 
 
 class VecMapfEnv:
@@ -113,6 +128,17 @@ class VecMapfEnv:
                                        auto_reset=self.auto_reset)
         self.step_count += 1
         return tuple(out)
+
+    def evaluate(self, policy, n_episodes, max_steps, gamma=1.0, seed=None):
+        """Runs `policy` for `n_episodes` episodes from the start state, in one launch: episode e is env e of this
+        batch stepped from a reset with `actions = policy(states)` and no auto-reset, cut at its first done or after
+        `max_steps` steps.  It draws from the Philox stream of `self.seed` (or `seed`) at `self.env_offset + e`, from
+        step `self.step_count` on.  `policy`: None (uniformly random joint actions), int32[nS] joint actions by joint
+        state (`value_iteration`'s policy), or an integer [n_agents, L] table of per-agent actions by cell
+        (`independent_policy`).  Returns an Evaluation; `self.states` and `step_count` are left as they are."""
+        out = self.engine.evaluate(policy, n_episodes, max_steps, gamma=gamma, seed=self.seed if seed is None else seed,
+                                   step_index=self.step_count, episode_offset=self.env_offset)
+        return Evaluation(*out)
 
     # ---- transition table --------------------------------------------------------------------------------------
     def transitions(self, states, actions):

@@ -181,6 +181,35 @@ int mapf_rollout(const mapf_ctx *ctx, void *states_inout, const int32_t *actions
                  const double *uniforms, uint64_t seed, uint64_t step_index0, int64_t env_offset, uint32_t options,
                  void *next_states, double *reward, double *prob, uint8_t *done, uint8_t *collision, void *stream);
 
+/* ---- closed-loop policy evaluation --------------------------------------------------------------------------- */
+
+/* outcome of an episode: the kind of its last step, or TIMEOUT when no step within max_steps was done */
+enum { MAPF_EPISODE_TIMEOUT = 0, MAPF_EPISODE_COLLISION = 1, MAPF_EPISODE_GOAL = 2, MAPF_EPISODE_TERMINAL_START = 3 };
+/* policy kinds of mapf_evaluate */
+enum {
+    MAPF_POLICY_RANDOM = 0, /* a uniformly random joint action per step, drawn as mapf_rollout draws it (policy unused) */
+    MAPF_POLICY_JOINT = 1,  /* int32 policy[policy_len], indexed by the joint state (policy_len >= nS; one-word states) */
+    MAPF_POLICY_AGENTS = 2  /* uint8 policy[n_agents * L]: agent i on cell c intends action policy[i * L + c] */
+};
+
+/* Bytes of device scratch mapf_evaluate needs (its work counter).  Concurrent calls need separate scratch. */
+int64_t mapf_evaluate_scratch_bytes(void);
+/* n_episodes closed-loop episodes of a policy in one launch.  Episode e is exactly
+ *     s = start state; G = 0; disc = 1
+ *     for t in range(max_steps):
+ *         a = policy(s); s, r, done = mapf_step(s, a) with Philox counter (episode_offset + e, step_index0 + t), no auto-reset
+ *         G = G + disc * r; disc = disc * gamma        (single binary64 operations, no fused multiply-add)
+ *         if done: break
+ * i.e. env e of a mapf_step batch with env_offset = episode_offset, cut at its first done.  ret[e] = G (f64),
+ * length[e] = t + 1 (int32), outcome[e] = MAPF_EPISODE_*.  Nothing is stored per step.  Out-of-range policy entries are
+ * clamped.  Device sampling only: a context whose slip probabilities do not add up to 1 is MAPF_ERR_UNSUPPORTED.
+ * Rejected (MAPF_ERR_INVALID): NULL pointers, max_steps < 1 or >= 2**31, n_episodes < 0 or > 2**30, AGENTS with
+ * policy_len != n_agents * L, JOINT with policy_len < nS; JOINT on a two-word context is MAPF_ERR_UNSUPPORTED.
+ * n_episodes == 0 launches nothing.  `scratch` (mapf_evaluate_scratch_bytes) is reset on `stream` by the call. */
+int mapf_evaluate(const mapf_ctx *ctx, int32_t policy_kind, const void *policy, int64_t policy_len, int64_t n_episodes,
+                  int64_t max_steps, double gamma, uint64_t seed, uint64_t step_index0, int64_t episode_offset,
+                  void *scratch, double *ret, int32_t *length, uint8_t *outcome, void *stream);
+
 /* Host-buffer convenience call (end-to-end path): copies states/actions from HOST memory, steps, copies the five
  * results back to HOST memory, on the context's own streams; returns when the results are in host memory. */
 int mapf_step_host(mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B, const double *uniforms,
