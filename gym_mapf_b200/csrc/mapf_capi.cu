@@ -1053,6 +1053,26 @@ static PhiloxKeys make_keys(uint64_t seed) {
 #define MAPF_SMALL_HOST_BATCH 1024         // mapf_step_host: batches up to this size go through the pinned scratch
 #define MAPF_LAUNCH_MAX_ENVS (1ll << 30)  // kernels index envs with 32 bits; larger batches are split
 
+// CTA size of a grid-stride k_step launch over `items` work items (envs / EPT) on at most `*grid` CTAs of at most
+// `max_threads` threads, for a kernel of which `per_sm` CTAs are resident on an SM.  The items need
+// rounds = ceil(items / (grid * max_threads)) grid-stride rounds; the CTA is then the smallest size that covers the items
+// in that many rounds, so that all threads run the same number of rounds, give or take one, and no part of the grid
+// idles through a last round that only some CTAs have.  Example: one pool of 2**19 C2 envs (2**18 pairs) on 148 CTAs:
+// 512 threads run 3.46 rounds each (68 CTAs run a 4th, 80 sit it out), 448 threads run 3.95.  The size is a multiple of
+// 4 / gcd(per_sm, 4) warps, so that the resident warps of an SM split evenly over its four schedulers (measured on
+// 2**20 C2 envs: 416 and 480 threads, 26 and 30 warps per SM, are 10 % slower than 448 and 512).  The grid shrinks only
+// where CTAs would get no item.  A smaller CTA is always legal under the kernel's __launch_bounds__ and keeps the
+// occupancy the grid was sized for; results depend on the env index only.
+static int plan_step_cta(u32 items, int max_threads, int per_sm, int *grid) {
+    const int quantum = 32 * (per_sm % 4 == 0 ? 1 : per_sm % 2 == 0 ? 2 : 4);
+    const int64_t g = *grid, rounds = ((int64_t)items + g * max_threads - 1) / (g * max_threads);
+    int threads = (int)(((int64_t)items + g * rounds * quantum - 1) / (g * rounds * quantum)) * quantum;
+    if (threads > max_threads) threads = max_threads;  // a max_threads that is not a multiple of the quantum
+    const int64_t used = ((int64_t)items + threads - 1) / threads;
+    if (used < g) *grid = (int)used;
+    return threads;
+}
+
 // Picks the step-kernel variant: replayed uniforms -> TAPE; otherwise the 2-envs-per-thread kernel with 128-bit
 // loads/stores when the batch is even and every buffer is suitably aligned, else the scalar one.
 static int launch_step(const mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B, const double *uniforms,
@@ -1099,24 +1119,33 @@ static int launch_step(const mapf_ctx *ctx, const void *states, const int32_t *a
         const void *fn;
         int grid;
         const KernelSet &ks = ctx->ks;
-        int threads = ctx->threads;
+        int max_threads = ctx->threads;
+        u32 items = nb;  // grid-stride work items: envs / EPT
         if (uniforms) {
             fn = keep ? (compact ? ks.step_tape_ck : ks.step_tape_k) : (compact ? ks.step_tape_c : ks.step_tape);
-            threads = ctx->threads_step;
-            grid = grid_for(nb, threads, ctx->grid_step_tape);
+            max_threads = ctx->threads_step;
+            grid = ctx->grid_step_tape;
         } else if (force_ept != 1 && (!ks.step_threads || ks.step_wide_ept2) && (nb & 1) == 0 && aligned(a_states, 16) && aligned(a_ns, 16) && aligned(a_actions, 8) &&
                    aligned(a_r, compact ? 2 : 16) && aligned(a_p, 16) && aligned(a_d, 2) && (compact || aligned(a_c, 2)) &&
                    aligned(a_keep, 16)) {
             fn = keep ? (compact ? ks.step_philox2ck : ks.step_philox2k) : (compact ? ks.step_philox2c : ks.step_philox2);
-            if (ks.step_wide_ept2) threads = ctx->threads_step;
-            grid = grid_for(nb / 2, threads, ctx->grid_step2);
+            if (ks.step_wide_ept2) max_threads = ctx->threads_step;
+            grid = ctx->grid_step2;
+            items = nb / 2;
         } else {
             fn = keep ? (compact ? ks.step_philox1ck : ks.step_philox1k) : (compact ? ks.step_philox1c : ks.step_philox1);
-            threads = ctx->threads_step;
-            grid = grid_for(nb, threads, ctx->grid_step1);
+            max_threads = ctx->threads_step;
+            grid = ctx->grid_step1;
         }
+        const int per_sm = grid / ctx->info.sm_count;  // the grids above are the kernels' resident CTAs on every SM
         if (grid_limit > 0 && grid > grid_limit) grid = grid_limit;
         if ((options & MAPF_OPT_SHARE_SM) && grid > ctx->info.sm_count) grid = ctx->info.sm_count;
+        // Only the pools' launches (one CTA per SM each) are sized by plan_step_cta: two pools of 2**19 C2 envs step in
+        // 8.89 us instead of 9.18 with 448-thread CTAs, while a single chain of 2**20 envs (two CTAs of one launch per SM)
+        // runs 1.0 % slower at 448 threads than at 512 (profiles/r04_launch_shape.txt).
+        int threads = max_threads;
+        if (options & MAPF_OPT_SHARE_SM) threads = plan_step_cta(items, max_threads, per_sm, &grid);
+        else grid = grid_for(items, threads, grid);
 #ifdef MAPF_TUNING
         static int use_pdl = -1;
         if (use_pdl < 0) {
