@@ -23,7 +23,7 @@ EPISODE_TIMEOUT, EPISODE_COLLISION, EPISODE_GOAL, EPISODE_TERMINAL_START = 0, 1,
 EXPORTS = ["mapf_ctx_create", "mapf_ctx_destroy", "mapf_ctx_info", "mapf_ctx_moves", "mapf_ctx_reward_table", "mapf_decode_states",
            "mapf_encode_states", "mapf_count_rows", "mapf_scan_scratch_bytes", "mapf_scan_rows", "mapf_count_scan_rows",
            "mapf_count_scan_range", "mapf_expand",
-           "mapf_count_range", "mapf_expand_range", "mapf_checksum", "mapf_step", "mapf_step_lanes", "mapf_rollout", "mapf_step_host", "mapf_step_host_resident",
+           "mapf_count_range", "mapf_expand_range", "mapf_checksum", "mapf_step", "mapf_rollout", "mapf_step_host", "mapf_step_host_resident",
            "mapf_evaluate_scratch_bytes", "mapf_evaluate",
            "mapf_backup", "mapf_backup_range", "mapf_greedy", "mapf_greedy_bcast", "mapf_count_predecessors", "mapf_predecessors",
            "mapf_projected_words", "mapf_project_states", "mapf_parse_map_text", "mapf_parse_scen_text", "mapf_ctx_create_from_text", "mapf_ctx_grid",
@@ -96,7 +96,6 @@ def lib():
         L.mapf_expand_range.argtypes = [vp, C.POINTER(u64 * 2), i64, vp, vp, vp, vp, vp, vp]
         L.mapf_checksum.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp, vp]
         L.mapf_step.argtypes = [vp, vp, vp, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp, vp]
-        L.mapf_step_lanes.argtypes = L.mapf_step.argtypes
         L.mapf_rollout.argtypes = [vp, vp, vp, i64, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp, vp]
         L.mapf_step_host.argtypes = [vp, vp, vp, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp]
         L.mapf_step_host_resident.argtypes = [vp, vp, vp, i64, vp, u64, u64, i64, u32, vp, vp, vp, vp, vp]
@@ -371,10 +370,9 @@ class Engine:
 
     # ---- step / rollout
     def step(self, states, actions, uniforms=None, seed=0, step_index=0, env_offset=0, auto_reset=False, out=None,
-             mapping="thread", share_sm=False, compact=False):
-        """`mapping`: "thread" (one thread per env, the shipped kernel) or "lanes" (one warp lane per agent, the measured
-        alternative; 2..8 agents, one-word states).  `share_sm`: one resident CTA per SM (MAPF_OPT_SHARE_SM), for env
-        pools that are stepped concurrently on separate streams.  `compact` (MAPF_OPT_COMPACT): the result is
+             share_sm=False, compact=False):
+        """`share_sm`: one resident CTA per SM (MAPF_OPT_SHARE_SM), for env pools that are stepped concurrently on
+        separate streams.  `compact` (MAPF_OPT_COMPACT): the result is
         (next_states, reward_code u8[B], prob, flags u8[B]) -- reward = reward_table()[code], flags = done | collision << 1."""
         B = states.shape[0]
         self._check_batch(states, actions, uniforms)
@@ -387,12 +385,10 @@ class Engine:
                    torch.empty(B, dtype=torch.float64, device=dev), torch.empty(B, dtype=torch.bool, device=dev),
                    torch.empty(B, dtype=torch.bool, device=dev))
         ns, reward, prob, done, coll = out
-        fn = self._mapf_step if mapping == "thread" else lib().mapf_step_lanes
-        rc = fn(self._h, states.data_ptr(), actions.data_ptr(), B,
-                None if uniforms is None else uniforms.data_ptr(), seed, step_index, env_offset,
-                (OPT_AUTO_RESET if auto_reset else 0) | (OPT_SHARE_SM if share_sm else 0), ns.data_ptr(),
-                reward.data_ptr(), prob.data_ptr(),
-                done.data_ptr(), coll.data_ptr(), self._stream())
+        rc = self._mapf_step(self._h, states.data_ptr(), actions.data_ptr(), B,
+                             None if uniforms is None else uniforms.data_ptr(), seed, step_index, env_offset,
+                             (OPT_AUTO_RESET if auto_reset else 0) | (OPT_SHARE_SM if share_sm else 0), ns.data_ptr(),
+                             reward.data_ptr(), prob.data_ptr(), done.data_ptr(), coll.data_ptr(), self._stream())
         if rc:
             check(rc)
         return out

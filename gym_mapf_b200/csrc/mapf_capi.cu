@@ -68,8 +68,6 @@ struct mapf_ctx {
     size_t smem_backup = 0;      // smem_base + per-warp backup slabs
     int threads_step = 0;  // CTA size of k_step (ks.step_threads, else `threads`)
     int grid_step1 = 0, grid_step2 = 0, grid_step_tape = 0, grid_rollout = 0, grid_rollout2 = 0, grid_rollout_tape = 0;
-    int grid_lanes = 0, grid_lanes_tape = 0;
-    LaneConsts lanes;                   // per-lane constants of the lane-per-agent step (k_step_lanes)
     int grid_expand = 0, grid_expand_range = 0, grid_plain = 0, grid_backup = 0, grid_backup_range = 0;
     int grid_evaluate[3] = {0, 0, 0};   // k_evaluate by policy kind
     KernelSet ks;
@@ -81,9 +79,6 @@ struct mapf_ctx {
     unsigned char *d_image = nullptr;   // DevSpec::image; the move table is its tail
     u64 *d_lut = nullptr;               // = d_image + (MAPF_SMEM_LUT - MAPF_SMEM_IMG)
     u32 *d_cell_rc = nullptr, *d_colbits = nullptr, *d_colbase = nullptr;
-#ifdef MAPF_BITMAP_ENTRIES
-    unsigned char *d_image_bm = nullptr;  // experiment build: pattern tables + the obstacle bitmap blob
-#endif
     std::vector<u64> h_lut;
     std::vector<u32> h_cell_rc;
     // mapf_step_host staging
@@ -165,9 +160,6 @@ extern "C" void mapf_ctx_destroy(mapf_ctx *ctx) {
         cudaFree(ctx->d_image);
         cudaFree(ctx->d_cell_rc);
         cudaFree(ctx->d_colbits);
-#ifdef MAPF_BITMAP_ENTRIES
-        cudaFree(ctx->d_image_bm);
-#endif
         cudaFree(ctx->d_colbase);
         cudaFree(ctx->d_stage);
         if (ctx->h_small) cudaFreeHost(ctx->h_small);
@@ -479,9 +471,6 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
 
     // ---- launch geometry: stage the move table in shared memory when it leaves room for the per-warp scratch
     const size_t smem_limit = (size_t)prop.sharedMemPerBlockOptin;
-#ifdef MAPF_BITMAP_ENTRIES
-    size_t bm_blob = 0;
-#endif
     KernelSet probe;
     if (!pick_kernels(n, sp.words, true, &probe)) {
         mapf_ctx_destroy(ctx);
@@ -530,73 +519,9 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
         CTX_TRY(cudaMemcpy(ctx->d_image, head.data(), image_head, cudaMemcpyHostToDevice));
         sp.image = ctx->d_image;
         sp.image_bytes = (u32)(image_head + (luts ? lut_pad : 0));
-#ifdef MAPF_BITMAP_ENTRIES
-        // Experiment build (make variant EXTRA=-DMAPF_BITMAP_ENTRIES; tools/bitmap_entries_check.py): when the move table is
-        // not staged, stage the obstacle bitmap instead (words, word ranks, cell positions) and derive the entries on the
-        // fly (bm_lut_entry).  Bit-exact, measured 3.2x slower than the L2 gathers in the step: not shipped (DESIGN 7b).
-        if (!luts && sp.cand_mask == 7 && H <= 256 && W <= 256) {
-            const size_t nw = (size_t)W * wpc;
-            const size_t off_rank = nw * 4, off_pos = (off_rank + nw * 2 + 3) & ~(size_t)3;
-            bm_blob = (off_pos + (size_t)L * 2 + 15) & ~(size_t)15;
-            std::vector<unsigned char> blob(bm_blob, 0);
-            memcpy(blob.data(), colbits.data(), nw * 4);
-            uint16_t *wr = reinterpret_cast<uint16_t *>(blob.data() + off_rank);
-            for (int c = 0; c < W; ++c) {
-                u32 acc = colbase[c];
-                for (int w = 0; w < wpc; ++w) { wr[(size_t)c * wpc + w] = (uint16_t)acc; acc += (u32)__builtin_popcount(colbits[(size_t)c * wpc + w]); }
-            }
-            uint16_t *ps = reinterpret_cast<uint16_t *>(blob.data() + off_pos);
-            for (int id = 0; id < L; ++id) ps[id] = (uint16_t)((ctx->h_cell_rc[id] >> 16) | ((ctx->h_cell_rc[id] & 0xffffu) << 8));
-            CTX_TRY(cudaMalloc(&ctx->d_image_bm, image_head + bm_blob));
-            CTX_TRY(cudaMemcpy(ctx->d_image_bm, head.data(), image_head, cudaMemcpyHostToDevice));
-            CTX_TRY(cudaMemcpy(ctx->d_image_bm + image_head, blob.data(), bm_blob, cudaMemcpyHostToDevice));
-            sp.image = ctx->d_image_bm;
-            sp.image_bytes = (u32)(image_head + bm_blob);
-            sp.bm_wrank_off = (u32)off_rank;
-            sp.bm_pos_off = (u32)off_pos;
-            sp.bm_wpc = (u32)wpc;
-            auto pat_of = [&](u32 triple) {
-                for (int p = 0; p < ctx->n_patterns; ++p)
-                    if (ctx->pat_triple[p] == triple) return (u32)(p * MAPF_PAT_STRIDE);
-                return 0u;
-            };
-            const u32 none = pat_of(1u | (2u << 3) | (4u << 6)) | (3u << 8);
-            sp.bm_pat[0] = sp.bm_pat[1] = sp.bm_pat[2] = sp.bm_pat[4] = (u16)none;
-            sp.bm_pat[3] = (u16)(pat_of(3u | (4u << 3)) | (2u << 8));
-            sp.bm_pat[5] = (u16)(pat_of(5u | (2u << 3)) | (2u << 8));
-            sp.bm_pat[6] = (u16)(pat_of(1u | (6u << 3)) | (2u << 8));
-            sp.bm_pat[7] = (u16)(pat_of(7u) | (1u << 8));
-            sp.bm_pat_stay = (pat_of(7u) << 16) | (1u << 24);
-            ctx->threads = 512;
-        }
-#endif
     }
     pick_kernels(n, sp.words, luts, &ctx->ks);
-    memset(&ctx->lanes, 0, sizeof(ctx->lanes));
-    if (ctx->ks.step_lanes_philox) {
-        u128 pw = 1;
-        u32 p5 = 1;
-        for (int i = 0; i < 8; ++i) {
-            if (i < n) {  // L**i < nS < 2**63
-                const FastDiv f = make_fastdiv((u64)pw);
-                ctx->lanes.div_magic[i] = f.magic;
-                ctx->lanes.div_shift[i] = f.shift;
-                ctx->lanes.powL[i] = (u64)pw;
-                pw *= (u128)L;
-            }
-            if (i >= 1) {  // floor(a / 5**i) for a < 2**20: round-up magic with s = 32 + floor(log2 d)
-                const int fl = 31 - __builtin_clz(p5);
-                const u64 two_s = 1ull << (32 + fl);
-                ctx->lanes.act_magic[i] = (u32)((two_s + p5 - 1) / p5);
-                ctx->lanes.act_shift[i] = (u32)fl;
-            }
-            p5 *= 5u;
-        }
-    }
     ctx->smem_base = MAPF_SMEM_LUT + (luts ? lut_pad : 0);  // barrier + image
-#ifdef MAPF_BITMAP_ENTRIES
-    ctx->smem_base += bm_blob;
-#endif
     ctx->threads_step = ctx->ks.step_threads ? ctx->ks.step_threads : ctx->threads;
     ctx->threads_expand = ctx->ks.expand_threads ? ctx->ks.expand_threads : ctx->threads;
     if (ctx->smem_base + (size_t)(ctx->threads_expand / 32) * ctx->ks.expand_slab_bytes > smem_limit)
@@ -606,16 +531,16 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
     int grid_keep = 0;  // the KEEP kernels are launched with their plain twins' grids (host-link-bound callers)
     struct { const void *fn; size_t smem; int *grid; int threads; } plan[] = {
         {ctx->ks.step_philox1k, ctx->smem_base, &grid_keep, ctx->threads_step},
-        {ctx->ks.step_philox2k, ctx->smem_base, &grid_keep, ctx->ks.step_wide_ept2 ? ctx->threads_step : 0},
+        {ctx->ks.step_philox2k, ctx->smem_base, &grid_keep},
         {ctx->ks.step_tape_k, ctx->smem_base, &grid_keep, ctx->threads_step},
         {ctx->ks.step_philox1ck, ctx->smem_base, &grid_keep, ctx->threads_step},
-        {ctx->ks.step_philox2ck, ctx->smem_base, &grid_keep, ctx->ks.step_wide_ept2 ? ctx->threads_step : 0},
+        {ctx->ks.step_philox2ck, ctx->smem_base, &grid_keep},
         {ctx->ks.step_tape_ck, ctx->smem_base, &grid_keep, ctx->threads_step},
         {ctx->ks.step_philox1, ctx->smem_base, &ctx->grid_step1, ctx->threads_step},
-        {ctx->ks.step_philox2, ctx->smem_base, &ctx->grid_step2, ctx->ks.step_wide_ept2 ? ctx->threads_step : 0},
+        {ctx->ks.step_philox2, ctx->smem_base, &ctx->grid_step2},
         {ctx->ks.step_tape, ctx->smem_base, &ctx->grid_step_tape, ctx->threads_step},
         {ctx->ks.step_philox1c, ctx->smem_base, &ctx->grid_step1, ctx->threads_step},
-        {ctx->ks.step_philox2c, ctx->smem_base, &ctx->grid_step2, ctx->ks.step_wide_ept2 ? ctx->threads_step : 0},
+        {ctx->ks.step_philox2c, ctx->smem_base, &ctx->grid_step2},
         {ctx->ks.step_tape_c, ctx->smem_base, &ctx->grid_step_tape, ctx->threads_step},
         {ctx->ks.rollout_philox, ctx->smem_base, &ctx->grid_rollout},
         {ctx->ks.rollout_philox2, ctx->smem_base, &ctx->grid_rollout2, MAPF_ROLLOUT2_THREADS},
@@ -623,8 +548,6 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
         {ctx->ks.rollout_philox_rnd, ctx->smem_base, &ctx->grid_rollout},
         {ctx->ks.rollout_tape_rnd, ctx->smem_base, &ctx->grid_rollout_tape},
         {ctx->ks.rollout_tape, ctx->smem_base, &ctx->grid_rollout_tape},
-        {ctx->ks.step_lanes_philox, ctx->smem_base, &ctx->grid_lanes},
-        {ctx->ks.step_lanes_tape, ctx->smem_base, &ctx->grid_lanes_tape},
         {ctx->ks.expand, ctx->smem_expand, &ctx->grid_expand, ctx->threads_expand},
         {ctx->ks.expand_range, ctx->smem_expand, &ctx->grid_expand_range, ctx->threads_expand},
         {ctx->ks.backup, ctx->smem_backup, &ctx->grid_backup},
@@ -633,7 +556,7 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
         {ctx->ks.evaluate[MAPF_POLICY_JOINT], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_JOINT]},
         {ctx->ks.evaluate[MAPF_POLICY_AGENTS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_AGENTS]}};
     for (auto &pl : plan) {
-        if (!pl.fn) continue;  // two-word states have no backup kernels; the lane-per-agent step covers 2..8 agents
+        if (!pl.fn) continue;  // two-word states have no backup kernels; wide step CTAs have no EPT = 2 k_step
         if (pl.smem > smem_limit) {
             mapf_ctx_destroy(ctx);
             return fail(MAPF_ERR_UNSUPPORTED, "a hot kernel needs %zu B of shared memory, the device offers %zu", pl.smem, smem_limit);
@@ -1125,11 +1048,10 @@ static int launch_step(const mapf_ctx *ctx, const void *states, const int32_t *a
             fn = keep ? (compact ? ks.step_tape_ck : ks.step_tape_k) : (compact ? ks.step_tape_c : ks.step_tape);
             max_threads = ctx->threads_step;
             grid = ctx->grid_step_tape;
-        } else if (force_ept != 1 && (!ks.step_threads || ks.step_wide_ept2) && (nb & 1) == 0 && aligned(a_states, 16) && aligned(a_ns, 16) && aligned(a_actions, 8) &&
+        } else if (force_ept != 1 && ks.step_philox2 && (nb & 1) == 0 && aligned(a_states, 16) && aligned(a_ns, 16) && aligned(a_actions, 8) &&
                    aligned(a_r, compact ? 2 : 16) && aligned(a_p, 16) && aligned(a_d, 2) && (compact || aligned(a_c, 2)) &&
                    aligned(a_keep, 16)) {
             fn = keep ? (compact ? ks.step_philox2ck : ks.step_philox2k) : (compact ? ks.step_philox2c : ks.step_philox2);
-            if (ks.step_wide_ept2) max_threads = ctx->threads_step;
             grid = ctx->grid_step2;
             items = nb / 2;
         } else {
@@ -1188,36 +1110,6 @@ extern "C" int mapf_step(const mapf_ctx *ctx, const void *states, const int32_t 
     DeviceGuard g(ctx->device);
     return launch_step(ctx, states, actions, B, uniforms, seed, step_index, env_offset, options, next_states, reward, prob,
                        done, collision, (cudaStream_t)stream);
-}
-
-extern "C" int mapf_step_lanes(const mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B,
-                               const double *uniforms, uint64_t seed, uint64_t step_index, int64_t env_offset,
-                               uint32_t options, void *next_states, double *reward, double *prob, uint8_t *done,
-                               uint8_t *collision, void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !actions || !next_states || !reward || !prob || !done || !collision)))
-        return fail(MAPF_ERR_INVALID, "mapf_step_lanes: bad argument");
-    if (!ctx->ks.step_lanes_philox)
-        return fail(MAPF_ERR_UNSUPPORTED, "the lane-per-agent step covers 2..8 agents, one-word states and move tables staged "
-                                          "in shared memory; use mapf_step");
-    if (B == 0) return MAPF_OK;
-    if (B > MAPF_LAUNCH_MAX_ENVS) return fail(MAPF_ERR_INVALID, "mapf_step_lanes: at most 2**30 envs per call");
-    if (!uniforms && !ctx->philox_ok)
-        return fail(MAPF_ERR_UNSUPPORTED, "device-side sampling needs slip probabilities that add up to 1; pass uniforms");
-    DeviceGuard g(ctx->device);
-    DevSpec sp = ctx->sp;
-    LaneConsts lc = ctx->lanes;
-    PhiloxKeys keys = make_keys(seed);
-    u32 nb = (u32)B, op = options;
-    u64 st = step_index, e0 = (u64)env_offset;
-    void *args[] = {&sp, &lc, &keys, &states, &actions, &nb, &uniforms, &st, &e0, &op, &next_states, &reward, &prob, &done,
-                    &collision};
-    // one warp steps 32 envs per round
-    const int64_t warps_needed = (B + 31) / 32, per_cta = ctx->threads / 32;
-    int grid = (int)((warps_needed + per_cta - 1) / per_cta);
-    const int gmax = uniforms ? ctx->grid_lanes_tape : ctx->grid_lanes;
-    if (grid > gmax) grid = gmax;
-    LAUNCH(uniforms ? ctx->ks.step_lanes_tape : ctx->ks.step_lanes_philox, grid, ctx->threads, ctx->smem_base, stream, args);
-    return MAPF_OK;
 }
 
 extern "C" int mapf_rollout(const mapf_ctx *ctx, void *states_inout, const int32_t *actions, int64_t T, int64_t B,

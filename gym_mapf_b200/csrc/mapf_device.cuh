@@ -101,12 +101,6 @@ struct DevSpec {
     u32 image_bytes;   // multiple of 16; ends after the action table when the move table is not staged
     u32 smem_window;   // shared-window address of a hot kernel's dynamic shared memory (probed at context creation;
                        // the action table holds absolute shared-window addresses)
-#ifdef MAPF_BITMAP_ENTRIES  // experiment build (DESIGN 7b): moves derived from the obstacle bitmap in shared memory
-    u32 bm_wrank_off, bm_pos_off;  // byte offsets of the word ranks / the cell positions behind the bitmap words
-    u32 bm_wpc;                    // 32-bit words per column
-    u16 bm_pat[8];                 // blocked bits (intended | right << 1 | left << 2) -> pattern-row offset | k << 8
-    u32 bm_pat_stay;               // the same for STAY
-#endif
 };
 
 // Host-side staging of the per-pattern tables (one MAPF_PAT_STRIDE-byte row per merge pattern):
@@ -390,9 +384,6 @@ __device__ __forceinline__ u32 count_below(u32 w, u32 na, u32 nb) {
 }
 
 // ---- Philox4x32-10 (Salmon et al., SC'11), the counter-based generator of the device-side sampling mode -------
-#ifndef MAPF_PHILOX_ROUNDS
-#define MAPF_PHILOX_ROUNDS 10  // experiments only: anything else changes the stream
-#endif
 struct Philox4 {
     u32 v[4];
 };
@@ -403,16 +394,12 @@ struct PhiloxKeys {
 };
 __device__ __forceinline__ Philox4 philox4x32_10(u32 c0, u32 c1, u32 c2, u32 c3, const PhiloxKeys &K) {
 #pragma unroll
-    for (int r = 0; r < MAPF_PHILOX_ROUNDS; ++r) {
-#ifndef MAPF_PHILOX_NARROW  // one wide multiply per product (measured faster than separate hi/lo multiplies)
+    for (int r = 0; r < 10; ++r) {
+        // one wide multiply per product (measured faster than separate hi/lo multiplies)
         u64 p0, p1;
         asm("mul.wide.u32 %0, %1, %2;" : "=l"(p0) : "r"(c0), "r"(0xD2511F53u));
         asm("mul.wide.u32 %0, %1, %2;" : "=l"(p1) : "r"(c2), "r"(0xCD9E8D57u));
         const u32 hi0 = (u32)(p0 >> 32), lo0 = (u32)p0, hi1 = (u32)(p1 >> 32), lo1 = (u32)p1;
-#else
-        const u32 hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const u32 hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-#endif
         const u32 n0 = hi1 ^ c1 ^ K.k[2 * r], n2 = hi0 ^ c3 ^ K.k[2 * r + 1];
         c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
     }
@@ -459,9 +446,6 @@ struct SmemTables {
     u32 lut;           // shared-window address of the staged move table
     u32 act0;          // what the action table holds for STAY: the staged table's address, or 0
     const u64 *lut_g;  // the move table in global memory
-#ifdef MAPF_BITMAP_ENTRIES
-    const DevSpec *sp;
-#endif
 };
 
 __device__ __forceinline__ u32 smem_u32(const void *p) { return (u32)__cvta_generic_to_shared(p); }
@@ -514,9 +498,6 @@ __device__ __forceinline__ SmemTables tables_begin(const DevSpec &sp, unsigned c
     t.act0 = LUTS ? t.lut : 0u;
     asm volatile("" : "+r"(t.base), "+r"(t.lut));  // opaque: keep both in registers instead of re-deriving them
     t.lut_g = sp.lut;
-#ifdef MAPF_BITMAP_ENTRIES
-    t.sp = &sp;
-#endif
     return t;
 }
 
@@ -543,15 +524,6 @@ __device__ __forceinline__ u32 lds_u16(u32 addr) {
 // Joint action -> per agent `action * 8 (+ the staged move table's address)`, straight from the action table.
 template <int N>
 __device__ __forceinline__ void load_actions(const DevSpec &sp, const SmemTables &tb, u32 a, u32 (&actv)[N]) {
-#if defined(MAPF_ACTION_ARITH)  // experiment: base-5 digits by multiply-high instead of the shared-memory table
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-        const u32 q = a / 5u;
-        actv[i] = (a - q * 5u) * 8u + tb.act0;
-        a = q;
-    }
-    return;
-#endif
     a = min(a, (u32)sp.nA - 1u);  // an invalid action (rejected by the host API) must not index outside the table
 #pragma unroll
     for (int c = 0; c < (N + 3) / 4; ++c) {
@@ -569,74 +541,15 @@ __device__ __forceinline__ void load_actions(const DevSpec &sp, const SmemTables
     }
 }
 
-#ifdef MAPF_BITMAP_ENTRIES
-template <int OFF>
-__device__ __forceinline__ u32 lds_u32(u32 addr) {
-    u32 v;
-    asm volatile("ld.shared.u32 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(OFF));
-    return v;
-}
-// The entry of (cell, action) derived on the fly from the obstacle bitmap staged in shared memory (grid.py:37-40 numbering,
-// mapf_env.py:43-94 moves, :163-184 merge): position of the cell, three clamped moves with a bitmap test each, the rank
-// (word prefix + popcount) of a lateral destination, and the merge pattern from the three "blocked" bits -- two of the
-// three destinations coincide only when both moves are blocked (both stay on the cell).  fail_prob in (0, 1) only.
-__device__ __forceinline__ u64 bm_lut_entry(const SmemTables &tb, u32 cell, u32 act8) {
-    const DevSpec &sp = *tb.sp;
-    const u32 a = act8 >> 3;
-    if (a == 0u) {
-        u32 hi = cell | sp.bm_pat_stay;  // dest 2 | pattern row << 16 | k << 24
-#pragma unroll
-        for (int i = 0; i < ENT_PARK_AGENTS; ++i)
-            if (i < sp.n && cell == (u32)sp.goal[i]) hi |= 1u << (ENT_PARK_SHIFT - 32 + i);
-        return ((u64)hi << 32) | (u64)(cell | (cell << 16));
-    }
-    const u32 pos = lds_u16<0>(tb.lut + sp.bm_pos_off + cell * 2u);
-    const int r = (int)(pos & 0xffu), c = (int)(pos >> 8);
-    u32 dest[3], blocked = 0;
-#pragma unroll
-    for (int j = 0; j < 3; ++j) {
-        // intended, right slip, left slip (POSSIBILITIES, __init__.py:19-25): UP=1 RIGHT=2 DOWN=3 LEFT=4
-        const u32 d = j == 0 ? a : (j == 1 ? (a & 3u) + 1u : ((a + 2u) & 3u) + 1u);
-        const int dr = (d == 3u) - (d == 1u), dc = (d == 2u) - (d == 4u);
-        const int tr = r + dr, tc = c + dc;
-        const bool inb = (u32)tr < (u32)sp.H && (u32)tc < (u32)sp.Wd;
-        const u32 widx = inb ? (u32)tc * sp.bm_wpc + ((u32)tr >> 5) : 0u;
-        const u32 word = lds_u32<0>(tb.lut + widx * 4u);
-        const bool free_ = inb && ((word >> (tr & 31)) & 1u);
-        u32 id = cell;
-        if (free_) {
-            if (dc == 0) id = cell + (u32)dr;  // column-major numbering: the vertical neighbour is the next / previous id
-            else id = lds_u16<0>(tb.lut + sp.bm_wrank_off + widx * 2u) + (u32)__popc(word & ((1u << (tr & 31)) - 1u));
-        } else {
-            blocked |= 1u << j;
-        }
-        dest[j] = id;
-    }
-    const u32 pk = sp.bm_pat[blocked];  // pattern-row offset | k << 8
-    const u32 k = pk >> 8;
-    const u32 e1 = (blocked & 3u) == 3u ? dest[2] : dest[1];
-    const u32 e2 = k == 3u ? dest[2] : dest[0];
-    const u32 e1k = k >= 2u ? e1 : dest[0];
-    const u32 hi = e2 | ((pk & 0xffu) << 16) | (k << 24);
-    return ((u64)hi << 32) | (u64)(dest[0] | (e1k << 16));
-}
-#endif
-
 // bytes of shared memory the staged table occupies behind MAPF_SMEM_LUT (kernel scratch follows it)
 template <bool LUTS>
 __device__ __forceinline__ u32 staged_table_bytes(const DevSpec &sp) {
-#ifdef MAPF_BITMAP_ENTRIES
-    if (!LUTS) return sp.image_bytes - (u32)(MAPF_SMEM_LUT - MAPF_SMEM_IMG);
-#endif
     return LUTS ? sp.lut_bytes : 0u;
 }
 
 // move-table entry of (cell, action): `act8` is action * 8 (+ the table's shared-window address when staged)
 template <bool LUTS>
 __device__ __forceinline__ u64 lut_entry(const SmemTables &tb, u32 cell, u32 act8) {
-#ifdef MAPF_BITMAP_ENTRIES
-    if (!LUTS) return bm_lut_entry(tb, cell, act8);
-#endif
     if (LUTS) return lds_u64<0>(cell * 40u + act8);
     return __ldg(reinterpret_cast<const u64 *>(reinterpret_cast<const unsigned char *>(tb.lut_g) + (cell * 40u + act8)));
 }

@@ -5,7 +5,7 @@
 
 struct KernelSet {
     const void *step_philox1 = nullptr;  // k_step<N, W, LUTS, TAPE=false, EPT=1>
-    const void *step_philox2 = nullptr;  // ... EPT=2 (128-bit I/O)
+    const void *step_philox2 = nullptr;  // ... EPT=2 (128-bit I/O); null when step_threads != 0
     const void *step_tape = nullptr;     // k_step<N, W, LUTS, TAPE=true, EPT=1>
     const void *step_philox1c = nullptr, *step_philox2c = nullptr, *step_tape_c = nullptr;  // ... COMPACT outputs
     // ... KEEP = true (mapf_step_host_resident: next states also stored to the device-resident array), plain / COMPACT
@@ -14,7 +14,6 @@ struct KernelSet {
     const void *rollout_philox = nullptr, *rollout_tape = nullptr;  // k_rollout<N, W, LUTS, TAPE, EPT=1>
     const void *rollout_philox2 = nullptr;                            // ... EPT=2 (128-bit stores)
     const void *rollout_philox_rnd = nullptr, *rollout_philox2_rnd = nullptr, *rollout_tape_rnd = nullptr;  // actions == NULL
-    const void *step_lanes_philox = nullptr, *step_lanes_tape = nullptr;  // k_step_lanes<N, TAPE>: 2..8 agents, one-word states
     const void *step_group_philox = nullptr, *step_group_tape = nullptr;  // k_step_group<N, W, TAPE>; staged move tables only
     const void *expand = nullptr, *expand_range = nullptr;
     const void *count = nullptr, *count_range = nullptr;
@@ -27,7 +26,6 @@ struct KernelSet {
     const void *pred_count = nullptr, *pred_emit = nullptr, *project = nullptr;
     size_t expand_slab_bytes = 0;        // per warp
     int expand_threads = 0;              // CTA size of k_expand (0: the context's)
-    int step_wide_ept2 = 0;              // experiment builds: the wide CTAs also run the EPT = 2 kernels
     int step_threads = 0;                // CTA size of the EPT = 1 k_step kernels, which are then always used (0: the context's)
     size_t backup_slab_bytes = 0;        // per warp
 };

@@ -10,17 +10,20 @@
 template <int N, int W, bool LUTS>
 static void fill(KernelSet *k) {
     k->step_philox1 = (const void *)k_step<N, W, LUTS, false, 1>;
-    k->step_philox2 = (const void *)k_step<N, W, LUTS, false, 2>;
     k->step_tape = (const void *)k_step<N, W, LUTS, true, 1>;
     k->step_philox1c = (const void *)k_step<N, W, LUTS, false, 1, true>;
-    k->step_philox2c = (const void *)k_step<N, W, LUTS, false, 2, true>;
     k->step_tape_c = (const void *)k_step<N, W, LUTS, true, 1, true>;
     k->step_philox1k = (const void *)k_step<N, W, LUTS, false, 1, false, true>;
-    k->step_philox2k = (const void *)k_step<N, W, LUTS, false, 2, false, true>;
     k->step_tape_k = (const void *)k_step<N, W, LUTS, true, 1, false, true>;
     k->step_philox1ck = (const void *)k_step<N, W, LUTS, false, 1, true, true>;
-    k->step_philox2ck = (const void *)k_step<N, W, LUTS, false, 2, true, true>;
     k->step_tape_ck = (const void *)k_step<N, W, LUTS, true, 1, true, true>;
+    // EPT = 2; with a staged move table, from STEP_WIDE_MIN_AGENTS agents on the step runs one env per thread instead
+    if constexpr (!(LUTS && N >= STEP_WIDE_MIN_AGENTS)) {
+        k->step_philox2 = (const void *)k_step<N, W, LUTS, false, 2>;
+        k->step_philox2c = (const void *)k_step<N, W, LUTS, false, 2, true>;
+        k->step_philox2k = (const void *)k_step<N, W, LUTS, false, 2, false, true>;
+        k->step_philox2ck = (const void *)k_step<N, W, LUTS, false, 2, true, true>;
+    }
     k->rollout_philox = (const void *)k_rollout<N, W, LUTS, false, 1, true>;
     k->rollout_philox_rnd = (const void *)k_rollout<N, W, LUTS, false, 1, false>;
     if constexpr (N <= 6) {
@@ -29,10 +32,6 @@ static void fill(KernelSet *k) {
     }
     k->rollout_tape = (const void *)k_rollout<N, W, LUTS, true, 1, true>;
     k->rollout_tape_rnd = (const void *)k_rollout<N, W, LUTS, true, 1, false>;
-    if constexpr (LUTS && W == 1 && N >= 2 && N <= 8) {
-        k->step_lanes_philox = (const void *)k_step_lanes<N, false>;
-        k->step_lanes_tape = (const void *)k_step_lanes<N, true>;
-    }
     if (LUTS) {
         k->step_group_philox = (const void *)k_step_group<N, W, false>;
         k->step_group_tape = (const void *)k_step_group<N, W, true>;
@@ -67,7 +66,6 @@ static void fill(KernelSet *k) {
     k->project = (const void *)k_project<N, W>;
     k->expand_slab_bytes = sizeof(ExpandSlab<N>);
     k->expand_threads = LUTS ? EXPAND_THREADS(N) : 0;  // 0: the context's CTA size
-    k->step_wide_ept2 = STEP_WIDE_EPT2;
     k->step_threads = LUTS && N >= STEP_WIDE_MIN_AGENTS ? STEP_WIDE_THREADS : 0;  // != 0: one env per thread, wide CTAs
     k->backup_slab_bytes = sizeof(BackupSlab<N>);
 }

@@ -1,6 +1,6 @@
 // mapf_kernels.cuh -- the sm_100a kernels of the joint-transition engine.
 //
-// Mapping ("T" family): one thread per emitted unit -- one env-step in step/rollout mode, one P[s][a] record in
+// Mapping: one thread per emitted unit -- one env-step in step/rollout mode, one P[s][a] record in
 // expand mode.  All per-agent loops are unrolled over the template parameter N, so an agent's cell, move-table
 // entry and outcome digit live in registers.  The per-(cell, action) move table is staged in shared memory by one
 // bulk asynchronous copy (TMA engine) per CTA.
@@ -9,9 +9,6 @@
 #pragma once
 #include "mapf_device.cuh"
 
-#ifndef MAPF_ABLATE
-#define MAPF_ABLATE 0  // timing experiments only (tools/sweep8.sh); 0 = the real kernel
-#endif
 // Timeline builds only (-DMAPF_TRACE, tools/trace_step.py): thread 0 of every CTA of the Philox-mode k_step stamps
 // %globaltimer at its phase boundaries into the buffer passed in place of the (unused) `uniforms` pointer:
 // buf[0] = next free slot; slot = {tag << 48 | (step & 0xffff) << 32 | smid << 16 | blockIdx, nanoseconds}.
@@ -1155,11 +1152,7 @@ __device__ __forceinline__ EnvOut env_step(const DevSpec &sp, const SmemTables &
     u32 ehi[N];
 #pragma unroll
     for (int i = 0; i < N; ++i) {
-#if MAPF_ABLATE == 1  // experiment: no move-table gather (a made-up entry keeps the data flow alive)
-        const u64 e = ((u64)in.cell[i] * 0x0001000100010001ull + in.actv[i]) & 0x0000ffffffffffffull;
-#else
         const u64 e = lut_entry<LUTS>(tb, (u32)in.cell[i], in.actv[i]);
-#endif
         ehi[i] = (u32)(e >> 32);
         const u32 row = ent_row(ehi[i], tb.base);
         u32 pick;
@@ -1268,9 +1261,6 @@ __device__ __forceinline__ void step_item(const DevSpec &sp, const SmemTables &t
         int nxt[N];
         o[q] = env_step<N, WORDS, LUTS, TAPE>(sp, tb, in[q], TAPE ? uniforms + (size_t)(b + q) * N : nullptr, opts, nxt);
     }
-#if MAPF_ABLATE == 3  // experiment: almost no stores (the condition is never true, but the compiler cannot know)
-    if (o[0].prob < -1.0)
-#endif
     if (KEEP) {
         if (EPT == 2 && WORDS == 1) reinterpret_cast<ulonglong2 *>(keep)[it] = make_ulonglong2(o[0].lo, o[EPT - 1].lo);
         else {
@@ -1323,7 +1313,7 @@ __device__ __forceinline__ void item_draws(const PhiloxKeys &keys, u64 env0, u64
 
 // From STEP_WIDE_MIN_AGENTS agents on (one CTA per SM: two envs per thread want ~128 registers, which leaves 16 warps
 // per SM) the step kernel runs ONE env per thread in CTAs of STEP_WIDE_THREADS threads: <= 80 registers, 24 warps per SM.
-// The EPT = 2 instantiations of those agent counts are not launched (mapf_capi.cu: launch_step).  Measured against the
+// With a staged move table the EPT = 2 k_step of those agent counts is not instantiated (mapf_inst.cu).  Measured against the
 // 512-thread EPT = 2 launch (profiles/r02_ablations.txt): 7 agents +1.4 / +3.0 %, 8 agents (C4) +2.8 %, 9 agents +2.3 /
 // +8.6 %, 10 agents +8.9 %; 640 or 1024 threads and two envs per thread in 768-thread CTAs (a spill) are slower.
 #ifndef STEP_WIDE_MIN_AGENTS
@@ -1332,10 +1322,7 @@ __device__ __forceinline__ void item_draws(const PhiloxKeys &keys, u64 env0, u64
 #ifndef STEP_WIDE_THREADS
 #define STEP_WIDE_THREADS 768
 #endif
-#ifndef STEP_WIDE_EPT2
-#define STEP_WIDE_EPT2 0  // experiment: the wide CTAs keep two envs per thread (80 registers: a small spill)
-#endif
-#define STEP_THREADS(N, EPT) ((N) >= STEP_WIDE_MIN_AGENTS && ((EPT) == 1 || STEP_WIDE_EPT2) ? STEP_WIDE_THREADS : MAPF_MAX_THREADS)
+#define STEP_THREADS(N, EPT) ((N) >= STEP_WIDE_MIN_AGENTS && (EPT) == 1 ? STEP_WIDE_THREADS : MAPF_MAX_THREADS)
 template <int N, int WORDS, bool LUTS, bool TAPE, int EPT, bool COMPACT = false, bool KEEP = false>
 __global__ void __launch_bounds__(STEP_THREADS(N, EPT), MAPF_MIN_BLOCKS(N))
 k_step(DevSpec sp, PhiloxKeys keys, const u64 *states, const int *__restrict__ actions, u32 B,
@@ -1366,9 +1353,7 @@ k_step(DevSpec sp, PhiloxKeys keys, const u64 *states, const int *__restrict__ a
         asm volatile("prefetch.global.L2 [%0];" ::"l"(actions + (size_t)pf * EPT));
     }
     TRACE(2);
-#ifndef MAPF_NO_GRID_WAIT  // experiment builds only: launches whose inputs do not depend on the previous launch
     asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
     TRACE(3);
     RawIn<WORDS, EPT> raw;
     if (it < n_items) load_raw<WORDS, EPT>(states, actions, it, raw);
@@ -1509,7 +1494,6 @@ k_rollout(DevSpec sp, PhiloxKeys keys, u64 *states, const int *__restrict__ acti
 // ends (outcome = the step's kind: 1 clash, 2 goal, 3 the start state was terminal; 0 = no done within T steps).
 // A lane whose episode ends takes the next episode index of the queue (`counter`, one warp-aggregated atomic per warp
 // and refill), so a warp's lanes stay busy until the queue drains instead of waiting for the warp's longest episode.
-// MAPF_EVAL_STATIC (experiment builds only) deals episodes out by grid stride instead.
 template <int N, int WORDS, bool LUTS, int POLICY>
 __global__ void __launch_bounds__(MAPF_MAX_THREADS, MAPF_MIN_BLOCKS(N))
 k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, u32 T, double gamma, u64 step0, u64 e0,
@@ -1527,9 +1511,7 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
 #pragma unroll
     for (int i = 0; i < N; ++i) in.cell[i] = (int)sp.start[i];
     tables_wait<LUTS>(smem);
-#ifndef MAPF_EVAL_STATIC
     const u32 lane = threadIdx.x & 31u;
-#endif
     // every lane of a warp stays in the loop until none is live: the refill below is a warp-wide collective
     while (__any_sync(0xffffffffu, live)) {
         bool ended = false;
@@ -1563,9 +1545,6 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
                 ended = true;
             }
         }
-#ifdef MAPF_EVAL_STATIC
-        if (ended) e += n_threads;
-#else
         const u32 fin = __ballot_sync(0xffffffffu, ended);
         if (fin) {
             u32 base = 0;
@@ -1573,7 +1552,6 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
             base = __shfl_sync(0xffffffffu, base, __ffs(fin) - 1);
             if (ended) e = n_threads + base + (u32)__popc(fin & ((1u << lane) - 1u));
         }
-#endif
         if (ended) {
             live = e < E;
             t = 0;
@@ -1585,9 +1563,6 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
             for (int i = 0; i < N; ++i) in.cell[i] = (int)sp.start[i];
         }
     }
-#ifdef MAPF_EVAL_STATIC
-    (void)counter;
-#endif
 }
 
 // =====================================================================================================
@@ -1722,171 +1697,4 @@ k_step_group(const DevSpec *__restrict__ specs, const u32 *__restrict__ seg_begi
         }
         lo = hi;
     }
-}
-
-// =====================================================================================================
-// Step, lane-per-agent mapping ("A" family) -- the mapping BASELINE.json's north star describes, kept as a measured
-// alternative to the thread-per-env k_step (see DESIGN.md section 3 "Mapping" for the numbers).
-// =====================================================================================================
-// A group of G = 2, 4 or 8 lanes (the smallest power of two >= N) works on ONE env at a time, lane i of the group
-// being agent i: its digit of the state (one 64-bit division by L**i, the neighbour lane's quotient gives the
-// remainder), its action digit, its move-table entry, its slip draw and outcome.  Across the group:
-//   vertex conflicts   __match_any_sync on (group, next cell): any lane whose match mask has a second bit
-//   swap conflicts     __shfl_xor_sync of the reversed move word (next | prev << 16) against the own (prev | next << 16)
-//   duplicates in the current state (is_terminal)   __match_any_sync on (group, cell)
-//   clash / parked-agent counts                     __ballot_sync + the group's bit field
-//   probability        ((p0 * p1) * p2) ... in agent order, the factors fetched with __shfl_sync (mapf_env.py:250-257)
-//   next state         sum of next_i * L**i by a shuffle-xor butterfly
-// Global memory is still accessed one env per lane: a warp loads 32 consecutive envs (and draws their Philox words),
-// each group then steps through the G envs its own lanes hold (the env's state / action are broadcast from the holding
-// lane, its draws arrive by an in-register G x G transpose), lane j of the group keeps env j's results, and the warp
-// stores 32 consecutive results -- every load and store is as coalesced as in k_step.
-struct LaneConsts {
-    u64 div_magic[8];  // floor(x / L**i) for a 64-bit x: FastDiv of L**i (entry 0 unused: the quotient is x)
-    u32 div_shift[8];
-    u64 powL[8];       // L**i
-    u32 act_magic[8];  // floor(a / 5**i) = umulhi(a, magic) >> shift for a < 2**20 (entry 0 unused)
-    u32 act_shift[8];
-};
-
-template <int G>
-__device__ __forceinline__ void transpose_group(u32 (&m)[G], u32 li) {
-#pragma unroll
-    for (int s = 1; s < G; s <<= 1) {
-        const bool up = (li & (u32)s) != 0u;
-#pragma unroll
-        for (int k = 0; k < G; ++k) {
-            if (k & s) continue;
-            const u32 send = up ? m[k] : m[k | s];
-            const u32 recv = __shfl_xor_sync(0xffffffffu, send, s);
-            if (up) m[k] = recv;
-            else m[k | s] = recv;
-        }
-    }
-}
-
-template <int N, bool TAPE>
-__global__ void __launch_bounds__(MAPF_MAX_THREADS, 2)
-k_step_lanes(DevSpec sp, LaneConsts lc, PhiloxKeys keys, const u64 *states, const int *__restrict__ actions, u32 B,
-             const double *__restrict__ uniforms, u64 step, u64 env0, u32 opts, u64 *next_states,
-             double *__restrict__ reward, double *__restrict__ prob, u8 *__restrict__ done, u8 *__restrict__ coll) {
-    constexpr int G = N <= 2 ? 2 : (N <= 4 ? 4 : 8);
-    constexpr int NW = ((N + 3) / 4) * 4;
-    static_assert(N >= 2 && N <= 8, "lane-per-agent step: 2..8 agents");
-    extern __shared__ __align__(16) unsigned char smem[];
-    SmemTables tb = tables_begin<true>(sp, smem);
-    const u32 lane = threadIdx.x & 31u;
-    const u32 li = lane & (u32)(G - 1);   // agent of this lane
-    const u32 gbase = lane & ~(u32)(G - 1);
-    const bool active = li < (u32)N;
-    // per-lane constants
-    const u64 my_magic = lc.div_magic[li];
-    const u32 my_shift = lc.div_shift[li];
-    const u64 my_pow = active ? lc.powL[li] : 0ull;
-    const u32 my_amagic = lc.act_magic[li], my_ashift = lc.act_shift[li];
-    const u32 my_goal = sp.goal[li];
-    const u32 L = (u32)sp.L;
-    const u32 warps = (gridDim.x * blockDim.x) >> 5;
-    const u32 rounds = (B + 31u) >> 5;
-    bool ready = false;
-    for (u32 rd = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; rd < rounds; rd += warps) {
-        // ---- lane = env: coalesced loads, this env's draws
-        const u32 b = rd * 32u + lane;
-        const bool live = b < B;
-        const u64 s_mine = live ? states[b] : 0ull;
-        const u32 a_mine = live ? min((u32)actions[b], (u32)sp.nA - 1u) : 0u;
-        u32 wt[G];  // after the transpose: this agent's draw for env j of the group
-        if (!TAPE) {
-            EnvIn<N> tmp;
-            env_draws<N>(keys, env0 + (u64)b, step, tmp);
-#pragma unroll
-            for (int k = 0; k < G; ++k) wt[k] = k < NW ? tmp.w[k < NW ? k : 0] : 0u;
-            transpose_group<G>(wt, li);
-        }
-        if (!ready) { tables_wait<true>(smem); ready = true; }
-        u64 o_ns = 0;
-        double o_r = 0.0, o_p = 0.0;
-        u32 o_done = 0, o_coll = 0;
-#pragma unroll
-        for (int j = 0; j < G; ++j) {
-            // ---- lane = agent of env (gbase + j)
-            const u64 s = __shfl_sync(0xffffffffu, s_mine, j, G);
-            const u32 a = __shfl_sync(0xffffffffu, a_mine, j, G);
-            // my digit: q_i = s / L**i; cell_i = q_i - q_{i+1} * L (the neighbour lane holds q_{i+1}; q_N = 0)
-            u64 q = s;
-            if (li != 0u) {
-                const u64 h = __umul64hi(s, my_magic);
-                q = (((s - h) >> 1) + h) >> my_shift;
-            }
-            if (!active) q = 0ull;
-            u32 qn = __shfl_down_sync(0xffffffffu, (u32)q, 1, G);
-            if (li == (u32)(G - 1)) qn = 0u;
-            u32 cell = (u32)q - qn * L;
-            cell = min(cell, L - 1u);  // an out-of-range state (rejected by the host API) stays a valid table index
-            // my action digit, the same way
-            u32 qa = li == 0u ? a : (__umulhi(a, my_amagic) >> my_ashift);
-            u32 qan = __shfl_down_sync(0xffffffffu, qa, 1, G);
-            if (li == (u32)(G - 1)) qan = 0u;
-            const u32 act = active ? qa - qan * 5u : 0u;
-            const u64 e = lds_u64<0>(tb.lut + (active ? cell : 0u) * 40u + act * 8u);
-            const u32 row = ent_row((u32)(e >> 32), tb.base);
-            u32 pick;
-            if (TAPE) {
-                const u32 bj = rd * 32u + gbase + (u32)j;
-                const double ui = (active && bj < B) ? uniforms[(size_t)bj * N + li] : 0.0;
-                const double c0 = lds_f64<MAPF_SMEM_CUM>(row), c1 = lds_f64<MAPF_SMEM_CUM + 8>(row),
-                             c2 = lds_f64<MAPF_SMEM_CUM + 16>(row);
-                pick = c0 > ui ? 0u : (c1 > ui ? 1u : (c2 > ui ? 2u : 0u));
-            } else {
-                const uint2 t = lds_u32x2<MAPF_SMEM_THR>(row);
-                pick = count_below(wt[j], t.x, t.y);
-            }
-            const u32 nxt = ent_dest(e, pick);
-            const double p = lds_f64<MAPF_SMEM_PP>(row + pick * 8u);
-            // ---- conflicts across the group
-            const u32 gtag = gbase << 16;  // distinct per group; cells are 16-bit
-            const u32 k_cell = active ? (cell | gtag) : (0x80000000u | lane);
-            const u32 k_next = active ? (nxt | gtag) : (0x80000000u | lane);
-            const bool dup_here = __popc(__match_any_sync(0xffffffffu, k_cell)) > 1;   // is_terminal: a shared cell
-            bool clash_here = __popc(__match_any_sync(0xffffffffu, k_next)) > 1;       // vertex conflict
-            const u32 fw = active ? __byte_perm(cell, nxt, 0x5410) : 0xffffffffu;      // prev | next << 16
-            const u32 bw = active ? __byte_perm(nxt, cell, 0x5410) : 0xfffffffeu;      // next | prev << 16
-#pragma unroll
-            for (int d = 1; d < G; ++d) {  // swap: every lane takes part in every shuffle (no short-circuit around it)
-                const u32 other = __shfl_xor_sync(0xffffffffu, bw, d);
-                clash_here = clash_here | (other == fw);
-            }
-            const u32 gmask = ((1u << G) - 1u) << gbase;
-            const bool dup = (__ballot_sync(0xffffffffu, dup_here) & gmask) != 0u;
-            const bool clash = (__ballot_sync(0xffffffffu, clash_here) & gmask) != 0u;
-            u32 parked = 0;
-            if (sp.soc) parked = __popc(__ballot_sync(0xffffffffu, active && cell == my_goal && act == 0u) & gmask);
-            const bool term = dup || s == sp.sgoal[0];
-            // ---- probability in agent order, next state by a butterfly sum
-            double total = __shfl_sync(0xffffffffu, p, 0, G);
-#pragma unroll
-            for (int k = 1; k < N; ++k) total = __dmul_rn(total, __shfl_sync(0xffffffffu, p, k, G));
-            u64 ns = (u64)nxt * my_pow;
-#pragma unroll
-            for (int d = 1; d < G; d <<= 1) ns += __shfl_xor_sync(0xffffffffu, ns, d);
-            const bool goal = ns == sp.sgoal[0];
-            const int kind = term ? 3 : (clash ? 1 : (goal ? 2 : 0));
-            const double rw = lds_f64<MAPF_SMEM_REW>(tb.base + ((u32)(kind * MAPF_REW_STRIDE) + parked) * 8u);
-            if (term) { ns = s; total = 0.0; }
-            if ((opts & 1u) && kind != 0) ns = sp.s0[0];
-            if (li == (u32)j) {
-                o_ns = ns; o_r = rw; o_p = total;
-                o_done = kind != 0 ? 1u : 0u;
-                o_coll = kind == 1 ? 1u : 0u;
-            }
-        }
-        if (live) {
-            next_states[b] = o_ns;
-            reward[b] = o_r;
-            prob[b] = o_p;
-            done[b] = (u8)o_done;
-            coll[b] = (u8)o_coll;
-        }
-    }
-    if (!ready) tables_wait<true>(smem);
 }

@@ -166,14 +166,6 @@ int mapf_step(const mapf_ctx *ctx, const void *states, const int32_t *actions, i
  * their goal that chose STAY under the sum-of-costs criterion (mapf_env.py:441-446; 0 under Makespan). */
 int mapf_ctx_reward_table(const mapf_ctx *ctx, double out64[64]);
 
-/* The same step with the LANE-PER-AGENT mapping (a group of 2/4/8 warp lanes per env, lane i = agent i; vertex
- * conflicts by __match_any_sync, swaps by __shfl_xor_sync, counts by __ballot_sync).  Bit-identical results and the
- * same Philox stream as mapf_step; 2..8 agents, one-word states, staged move tables (else MAPF_ERR_UNSUPPORTED).  It
- * is the slower of the two mappings on every measured config (DESIGN.md section 3) and kept as a measured alternative. */
-int mapf_step_lanes(const mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B, const double *uniforms,
-                    uint64_t seed, uint64_t step_index, int64_t env_offset, uint32_t options, void *next_states,
-                    double *reward, double *prob, uint8_t *done, uint8_t *collision, void *stream);
-
 /* T consecutive steps of B envs in one launch; state lives in registers between steps.
  * actions: int32[T*B] (step-major) or NULL for a uniformly random joint action per env and step (Philox).
  * Outputs are step-major [T*B]; states_inout receives the final states.  Step t uses step_index0 + t. */

@@ -292,16 +292,15 @@ def test_multimap_vec_env():
             assert torch.equal(i1["prob"], info["prob"][lo:hi]) and torch.equal(i1["collision"], info["collision"][lo:hi])
 
 
-# ---- the lane-per-agent mapping of the step (mapf_step_lanes) --------------------------------------------------------
+# ---- the step on conflict-dense states (mapf_step) ------------------------------------------------------------------
 @gpu
 @pytest.mark.parametrize("n,map_name,scen", [(2, "empty-8-8", 1), (3, "room-32-32-4", 1), (4, "room-32-32-4", 1),
                                              (5, "empty-16-16", 2), (6, "maze-32-32-4", 10), (7, "empty-16-16", 4),
                                              (8, "empty-8-8", 3)])
 @pytest.mark.parametrize("soc", [True, False])
 @pytest.mark.timeout(180)
-def test_lane_mapping_matches_oracle_and_thread_mapping(n, map_name, scen, soc):
-    """k_step_lanes (one warp lane per agent, warp-primitive conflict detection) == the C oracle given the uniforms, and
-    == k_step draw for draw in device-sampling mode; ragged batch sizes, conflict-dense states."""
+def test_step_conflict_dense_matches_oracle(n, map_name, scen, soc):
+    """k_step == the C oracle given the uniforms; ragged batch sizes, conflict-dense states."""
     import torch
     from engine_util import make_engine, make_oracle, u64
     sp = _shipped_spec(map_name, scen, n, 0.2, -1000.0, 100.0, -1.0, soc)
@@ -323,30 +322,13 @@ def test_lane_mapping_matches_oracle_and_thread_mapping(n, map_name, scen, soc):
         states = torch.from_numpy(lo.view(np.int64).copy()).cuda()
         actions = torch.from_numpy(act).cuda()
         uniforms = torch.from_numpy(uni).cuda()
-        got = eng.step(states, actions, uniforms=uniforms, mapping="lanes")
+        got = eng.step(states, actions, uniforms=uniforms)
         w = ora.step(lo, hi, act.astype(np.int64), uni)
         assert np.array_equal(u64(got[0]), w["next_lo"])
         assert np.array_equal(u64(got[1]), G.f64_to_bits(w["reward"])) and np.array_equal(u64(got[2]), G.f64_to_bits(w["prob"]))
         assert np.array_equal(got[3].cpu().numpy().astype(np.uint8), w["done"])
         assert np.array_equal(got[4].cpu().numpy().astype(np.uint8), w["collision"])
         assert w["collision"].sum() > 0 or B < 1000
-        for auto_reset in (False, True):
-            a = eng.step(states, actions, seed=11, step_index=3, env_offset=77, auto_reset=auto_reset)
-            b = eng.step(states, actions, seed=11, step_index=3, env_offset=77, auto_reset=auto_reset, mapping="lanes")
-            for x, y in zip(a, b):
-                assert torch.equal(x, y)
-
-
-@gpu
-def test_lane_mapping_unsupported():
-    from engine_util import make_engine
-    from gym_mapf_b200 import _native
-    import torch
-    e8 = make_engine(_shipped_spec("room-64-64-8", 1, 8, 0.2, -1000.0, 100.0, -1.0, False))   # two-word states
-    st = e8.states_from_ints([e8.s0])
-    with pytest.raises(_native.NativeError) as ei:
-        e8.step(st, torch.zeros(1, dtype=torch.int32, device="cuda"), mapping="lanes")
-    assert ei.value.code == _native.MAPF_ERR_UNSUPPORTED
 
 
 # ---- exclusive scan of row lengths (mapf_scan_rows): folded and spine paths, aligned and unaligned buffers ------------
@@ -401,10 +383,10 @@ def test_multimap_shards_equal_the_whole_batch():
 
 @gpu
 @pytest.mark.timeout(300)
-def test_fuzz_group_and_lane_kernels_every_agent_count():
+def test_fuzz_group_and_step_kernels_every_agent_count():
     """Random small grids (obstacles, coinciding starts/goals, every noise level), 1..13 agents: groups of 2-4 random
-    specs per agent count stepped in one launch must equal the C oracle per spec; with 2..8 agents and one-word states
-    the lane-per-agent kernel must as well."""
+    specs per agent count stepped in one launch must equal the C oracle per spec, and each spec's segment must equal
+    mapf_step of that spec alone."""
     import torch
     from engine_util import make_engine, make_oracle, u64
     from gym_mapf_b200 import _native
@@ -465,10 +447,9 @@ def test_fuzz_group_and_lane_kernels_every_agent_count():
                 assert np.array_equal(u64(out[2][sl]), G.f64_to_bits(w["prob"])), (n, words, sp)
                 assert np.array_equal(out[3][sl].cpu().numpy().astype(np.uint8), w["done"])
                 assert np.array_equal(out[4][sl].cpu().numpy().astype(np.uint8), w["collision"])
-                if words == 1 and 2 <= n <= 8:
-                    one = eng.step(states[sl].clone(), actions[sl].clone(), uniforms=uniforms[sl].clone(), mapping="lanes")
-                    for x, y in zip(one, out):
-                        assert torch.equal(x, y[sl]), (n, sp)
+                one = eng.step(states[sl].clone(), actions[sl].clone(), uniforms=uniforms[sl].clone())
+                for x, y in zip(one, out):
+                    assert torch.equal(x, y[sl]), (n, sp)
                 at += c
             group.close()
             for e in engines:

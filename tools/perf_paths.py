@@ -176,9 +176,8 @@ def step_case(tag, env, B, ring):
 
 
 def mappings():
-    """The same batched step through (a) the shipped thread-per-env kernel, (b) the lane-per-agent kernel
-    (mapf_step_lanes: __match_any_sync / __shfl_xor_sync / __ballot_sync across an agent group) and (c) the grouped
-    kernel of heterogeneous batches with 1, 4 and 64 specs (mapf_group_step).  Stream launches, ring of buffers > L2."""
+    """The same batched step through (a) the shipped thread-per-env kernel and (b) the grouped kernel of heterogeneous
+    batches with 1, 4 and 64 specs (mapf_group_step).  Stream launches, ring of buffers > L2."""
     for map_name, scen, n, B in (("room-32-32-4", 1, 4, 1 << 20), ("empty-32-32", 1, 2, 1 << 20),
                                  ("room-32-32-4", 13, 6, 1 << 20), ("empty-16-16", 1, 7, 1 << 20)):
         env = make(map_name, scen, n)
@@ -196,9 +195,7 @@ def mappings():
         ref = eng.step(states[0], actions[0], seed=1, step_index=7)
         by = B * (2 * W + 22)
         K = ring * 4
-        variants = [("thread-per-env (k_step)", lambda j, i: eng.step(states[j], actions[j], seed=1, step_index=i, out=outs[j])),
-                    ("lane-per-agent (k_step_lanes)",
-                     lambda j, i: eng.step(states[j], actions[j], seed=1, step_index=i, out=outs[j], mapping="lanes"))]
+        variants = [("thread-per-env (k_step)", lambda j, i: eng.step(states[j], actions[j], seed=1, step_index=i, out=outs[j]))]
         for n_specs in (1, 4, 64):
             # copies of the same spec with different rewards: every CTA re-stages when its tile run crosses a segment
             envs = [create_mapf_env(map_name, scen, n, 0.2, -1000.0 - k, 100.0, -1.0, OptimizationCriteria.SoC, device=0)

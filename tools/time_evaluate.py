@@ -1,6 +1,5 @@
 """Closed-loop policy evaluation (`k_evaluate`, mapf_evaluate) timed with CUDA events (profiles/r03_evaluate.txt).
 
-    make -C gym_mapf_b200/csrc variant TAG=evalstatic VN=4 EXTRA=-DMAPF_EVAL_STATIC   # optional: the static schedule
     python tools/time_evaluate.py
 
 Workloads (SoC, fail 0.2, scenario 1, max_steps 256, 2**22 episodes, gamma 1):
@@ -11,16 +10,11 @@ Workloads (SoC, fail 0.2, scenario 1, max_steps 256, 2**22 episodes, gamma 1):
   (e) the loop a user writes without mapf_evaluate on workload (a): `vec.step(policy(states))` + torch accumulators
 Each call is warmed up twice and timed seven times between its own pair of events; median [min, max] are reported.
 The policy tables are small (2.7 KB for (a), 1.9 MB for (c)) and stay in L2 after the first step, as they do in use.
-With the variant library next to the release one, (a) and (b) are timed again with the static grid-stride schedule in a
-child process (it holds 4-agent kernels only, so it receives the per-agent table of (a) from this process).
 """
 import os
 import subprocess
 import sys
-import tempfile
 import time
-
-import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -31,7 +25,6 @@ from gym_mapf_b200.envs.utils import create_mapf_env, independent_policy  # noqa
 from gym_mapf_b200.envs.vec_env import Evaluation, VecMapfEnv, evaluation_summary  # noqa: E402
 
 E, T = 1 << 22, 256
-STATIC_LIB = os.path.join(ROOT, "gym_mapf_b200", "csrc", "libmapf_b200_evalstatic.so")
 
 
 def env_of(map_name, n):
@@ -90,50 +83,30 @@ def workload_b(c2):
 
 
 def main():
-    child = len(sys.argv) == 4 and sys.argv[1] == "--workloads"  # the static-schedule run: workloads, table of (a)
-    only = sys.argv[2].split(",") if child else list("abcde")
-    if not child:
-        gpu = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                             capture_output=True, text=True).stdout.strip()
-        print("GPU: %s" % gpu)
-        print("%d episodes, max_steps %d, gamma 1.0, SoC, fail 0.2; median [min, max] of 7 timed calls" % (E, T))
+    gpu = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                         capture_output=True, text=True).stdout.strip()
+    print("GPU: %s" % gpu)
+    print("%d episodes, max_steps %d, gamma 1.0, SoC, fail 0.2; median [min, max] of 7 timed calls" % (E, T))
     env2 = env_of("room-32-32-4", 4)
     c2 = VecMapfEnv(env2, 1, seed=11)
-    if child:
-        table_c2 = torch.from_numpy(np.load(sys.argv[3])).to(c2.device)
-    else:
-        table_c2 = independent_policy(env2)
-    ev_a = None
-    if "a" in only:
-        ev_a = workload_a(c2, table_c2)
-    if "b" in only:
-        workload_b(c2)
-    if "c" in only:
-        env = env_of("room-32-32-4", 2)
-        vec = VecMapfEnv(env, 1, seed=11)
-        torch.cuda.synchronize()
-        t0 = time.perf_counter()
-        _, pi, iters = vec.value_iteration(gamma=1.0)
-        torch.cuda.synchronize()
-        print("(c) value_iteration, room-32-32-4, 2 agents (nS = %d): %d sweeps in %.3f s" % (env.nS, iters,
-                                                                                            time.perf_counter() - t0))
-        fn, ev = run_eval(vec, pi)
-        report("(c) JOINT 2 agents, value_iteration policy", timed(fn), ev)
-    if "d" in only:
-        env = env_of("room-64-64-8", 8)
-        vec = VecMapfEnv(env, 1, seed=11)
-        fn, ev = run_eval(vec, independent_policy(env))
-        report("(d) C4 AGENTS 8 agents (128-bit states), independent_policy", timed(fn), ev)
-    if "e" in only:
-        user_loop(env2, table_c2, ev_a)
-    if not child and os.path.exists(STATIC_LIB):
-        print("static grid-stride schedule (-DMAPF_EVAL_STATIC), same workloads:")
-        sys.stdout.flush()
-        with tempfile.TemporaryDirectory() as tmp:
-            path = os.path.join(tmp, "table_a.npy")
-            np.save(path, table_c2.cpu().numpy())
-            subprocess.run([sys.executable, os.path.abspath(__file__), "--workloads", "a,b", path],
-                           env=dict(os.environ, MAPF_B200_LIB=STATIC_LIB), check=True)
+    table_c2 = independent_policy(env2)
+    ev_a = workload_a(c2, table_c2)
+    workload_b(c2)
+    env = env_of("room-32-32-4", 2)
+    vec = VecMapfEnv(env, 1, seed=11)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    _, pi, iters = vec.value_iteration(gamma=1.0)
+    torch.cuda.synchronize()
+    print("(c) value_iteration, room-32-32-4, 2 agents (nS = %d): %d sweeps in %.3f s" % (env.nS, iters,
+                                                                                        time.perf_counter() - t0))
+    fn, ev = run_eval(vec, pi)
+    report("(c) JOINT 2 agents, value_iteration policy", timed(fn), ev)
+    env = env_of("room-64-64-8", 8)
+    vec = VecMapfEnv(env, 1, seed=11)
+    fn, ev = run_eval(vec, independent_policy(env))
+    report("(d) C4 AGENTS 8 agents (128-bit states), independent_policy", timed(fn), ev)
+    user_loop(env2, table_c2, ev_a)
 
 
 def user_loop(env, table, ev_a):
