@@ -637,8 +637,12 @@ static int grid_for(int64_t work_items, int threads, int grid_max) {
         if (_e != cudaSuccess) return fail(MAPF_ERR_CUDA, "launch %s: %s", #fn, cudaGetErrorString(_e));      \
     } while (0)
 
+// Two-word states are read and written as 16-byte vectors (load_state / store_state), so arrays of them must be
+// 16-byte aligned: a misaligned one is rejected instead of faulting in the kernel.
+static inline bool states_misaligned(int words, const void *p) { return words == 2 && ((uintptr_t)p & 15u) != 0; }
+
 extern "C" int mapf_decode_states(const mapf_ctx *ctx, const void *states, int64_t B, int32_t *cells, void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !cells))) return fail(MAPF_ERR_INVALID, "mapf_decode_states: bad argument");
+    if (!ctx || B < 0 || (B > 0 && (!states || !cells || states_misaligned(ctx->sp.words, states)))) return fail(MAPF_ERR_INVALID, "mapf_decode_states: bad argument");
     if (B == 0) return MAPF_OK;
     DeviceGuard g(ctx->device);
     DevSpec sp = ctx->sp;
@@ -648,7 +652,7 @@ extern "C" int mapf_decode_states(const mapf_ctx *ctx, const void *states, int64
 }
 
 extern "C" int mapf_encode_states(const mapf_ctx *ctx, const int32_t *cells, int64_t B, void *states, void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !cells))) return fail(MAPF_ERR_INVALID, "mapf_encode_states: bad argument");
+    if (!ctx || B < 0 || (B > 0 && (!states || !cells || states_misaligned(ctx->sp.words, states)))) return fail(MAPF_ERR_INVALID, "mapf_encode_states: bad argument");
     if (B == 0) return MAPF_OK;
     DeviceGuard g(ctx->device);
     DevSpec sp = ctx->sp;
@@ -669,7 +673,7 @@ static int count_impl(const mapf_ctx *ctx, bool range, const void *states, const
 
 extern "C" int mapf_count_rows(const mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B,
                                int64_t *row_len, void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !actions || !row_len)))
+    if (!ctx || B < 0 || (B > 0 && (!states || !actions || !row_len || states_misaligned(ctx->sp.words, states))))
         return fail(MAPF_ERR_INVALID, "mapf_count_rows: bad argument");
     return count_impl(ctx, false, states, actions, 0, 0, B, row_len, stream);
 }
@@ -752,7 +756,8 @@ static int count_scan_impl(const mapf_ctx *ctx, bool range, const void *states, 
 
 extern "C" int mapf_count_scan_rows(const mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B,
                                     int64_t *row_len, int64_t *row_ptr, void *scratch, void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !actions))) return fail(MAPF_ERR_INVALID, "mapf_count_scan_rows: bad argument");
+    if (!ctx || B < 0 || (B > 0 && (!states || !actions || states_misaligned(ctx->sp.words, states))))
+        return fail(MAPF_ERR_INVALID, "mapf_count_scan_rows: bad argument");
     return count_scan_impl(ctx, false, states, actions, 0, 0, B, row_len, row_ptr, scratch, stream);
 }
 
@@ -814,7 +819,9 @@ static int expand_impl(const mapf_ctx *ctx, bool range, const void *states, cons
 extern "C" int mapf_expand(const mapf_ctx *ctx, const void *states, const int32_t *actions, int64_t B,
                            const int64_t *row_ptr, void *next_state, double *prob, double *reward, uint8_t *flags,
                            void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !actions))) return fail(MAPF_ERR_INVALID, "mapf_expand: bad argument");
+    if (!ctx || B < 0 || (B > 0 && (!states || !actions || states_misaligned(ctx->sp.words, states) ||
+                                     states_misaligned(ctx->sp.words, next_state))))
+        return fail(MAPF_ERR_INVALID, "mapf_expand: bad argument");
     return expand_impl(ctx, false, states, actions, 0, 0, B, row_ptr, next_state, prob, reward, flags, stream);
 }
 
@@ -830,7 +837,8 @@ extern "C" int mapf_expand_range(const mapf_ctx *ctx, const uint64_t s_begin[2],
 
 extern "C" int mapf_checksum(const mapf_ctx *ctx, int64_t n_records, int64_t index_base, const void *next_state,
                              const double *prob, const double *reward, const uint8_t *flags, uint64_t *out8, void *stream) {
-    if (!ctx || n_records < 0 || !out8 || (n_records > 0 && (!next_state || !prob || !reward || !flags)))
+    if (!ctx || n_records < 0 || !out8 ||
+        (n_records > 0 && (!next_state || !prob || !reward || !flags || states_misaligned(ctx->sp.words, next_state))))
         return fail(MAPF_ERR_INVALID, "mapf_checksum: bad argument");
     if (n_records == 0) return MAPF_OK;
     DeviceGuard g(ctx->device);
@@ -910,7 +918,8 @@ extern "C" int mapf_greedy_bcast(const mapf_ctx *ctx, const double *Q, int64_t n
 }
 
 extern "C" int mapf_count_predecessors(const mapf_ctx *ctx, const void *states, int64_t B, int64_t *row_len, void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !row_len))) return fail(MAPF_ERR_INVALID, "mapf_count_predecessors: bad argument");
+    if (!ctx || B < 0 || (B > 0 && (!states || !row_len || states_misaligned(ctx->sp.words, states))))
+        return fail(MAPF_ERR_INVALID, "mapf_count_predecessors: bad argument");
     if (B == 0) return MAPF_OK;
     DeviceGuard g(ctx->device);
     DevSpec sp = ctx->sp;
@@ -921,7 +930,9 @@ extern "C" int mapf_count_predecessors(const mapf_ctx *ctx, const void *states, 
 
 extern "C" int mapf_predecessors(const mapf_ctx *ctx, const void *states, int64_t B, const int64_t *row_ptr, void *pred,
                                  void *stream) {
-    if (!ctx || B < 0 || (B > 0 && (!states || !row_ptr || !pred))) return fail(MAPF_ERR_INVALID, "mapf_predecessors: bad argument");
+    if (!ctx || B < 0 || (B > 0 && (!states || !row_ptr || !pred || states_misaligned(ctx->sp.words, states) ||
+                                     states_misaligned(ctx->sp.words, pred))))
+        return fail(MAPF_ERR_INVALID, "mapf_predecessors: bad argument");
     if (B == 0) return MAPF_OK;
     DeviceGuard g(ctx->device);
     DevSpec sp = ctx->sp;
@@ -939,7 +950,9 @@ extern "C" int mapf_projected_words(const mapf_ctx *ctx, int32_t n_sub) {
 
 extern "C" int mapf_project_states(const mapf_ctx *ctx, const void *states, int64_t B, const int32_t *agents, int32_t n_sub,
                                    void *out_states, void *stream) {
-    if (!ctx || B < 0 || !agents || n_sub < 1 || n_sub > ctx->sp.n || (B > 0 && (!states || !out_states)))
+    if (!ctx || B < 0 || !agents || n_sub < 1 || n_sub > ctx->sp.n ||
+        (B > 0 && (!states || !out_states || states_misaligned(ctx->sp.words, states) ||
+                   states_misaligned(mapf_projected_words(ctx, n_sub), out_states))))
         return fail(MAPF_ERR_INVALID, "mapf_project_states: bad argument");
     AgentList sub;
     memset(&sub, 0, sizeof(sub));
@@ -1104,7 +1117,8 @@ extern "C" int mapf_step(const mapf_ctx *ctx, const void *states, const int32_t 
                          uint32_t options, void *next_states, double *reward, double *prob, uint8_t *done,
                          uint8_t *collision, void *stream) {
     if (!ctx || B < 0 || (B > 0 && (!states || !actions || !next_states || !reward || !prob || !done ||
-                                     (!collision && !(options & MAPF_OPT_COMPACT)))))
+                                     (!collision && !(options & MAPF_OPT_COMPACT)) ||
+                                     states_misaligned(ctx->sp.words, states) || states_misaligned(ctx->sp.words, next_states))))
         return fail(MAPF_ERR_INVALID, "mapf_step: bad argument");
     if (B == 0) return MAPF_OK;
     DeviceGuard g(ctx->device);
@@ -1117,7 +1131,8 @@ extern "C" int mapf_rollout(const mapf_ctx *ctx, void *states_inout, const int32
                             uint32_t options, void *next_states, double *reward, double *prob, uint8_t *done,
                             uint8_t *collision, void *stream) {
     if (!ctx || B < 0 || T < 0 ||
-        (B > 0 && T > 0 && (!states_inout || !next_states || !reward || !prob || !done || !collision)))
+        (B > 0 && T > 0 && (!states_inout || !next_states || !reward || !prob || !done || !collision ||
+                            states_misaligned(ctx->sp.words, states_inout) || states_misaligned(ctx->sp.words, next_states))))
         return fail(MAPF_ERR_INVALID, "mapf_rollout: bad argument");
     if (B == 0 || T == 0) return MAPF_OK;
     if (B > MAPF_LAUNCH_MAX_ENVS) return fail(MAPF_ERR_INVALID, "mapf_rollout: at most 2**30 envs per call");
@@ -1353,7 +1368,8 @@ extern "C" int mapf_step_host_resident(mapf_ctx *ctx, void *states_dev, const in
                                        const double *uniforms, uint64_t seed, uint64_t step_index, int64_t env_offset,
                                        uint32_t options, void *next_states, double *reward, double *prob, uint8_t *done,
                                        uint8_t *collision) {
-    if (B > 0 && !states_dev) return fail(MAPF_ERR_INVALID, "mapf_step_host_resident: bad argument");
+    if (B > 0 && (!states_dev || (ctx && states_misaligned(ctx->sp.words, states_dev))))
+        return fail(MAPF_ERR_INVALID, "mapf_step_host_resident: bad argument");
     return step_host_impl(ctx, nullptr, states_dev, actions, B, uniforms, seed, step_index, env_offset, options, next_states,
                           reward, prob, done, collision);
 }
@@ -1630,7 +1646,8 @@ extern "C" int mapf_group_step(const mapf_group *g, const void *states, const in
                                double *reward, double *prob, uint8_t *done, uint8_t *collision, void *stream) {
     if (!g) return fail(MAPF_ERR_INVALID, "mapf_group_step: NULL group");
     if (g->B == 0) return MAPF_OK;
-    if (!states || !actions || !next_states || !reward || !prob || !done || !collision)
+    if (!states || !actions || !next_states || !reward || !prob || !done || !collision ||
+        states_misaligned(g->words, states) || states_misaligned(g->words, next_states))
         return fail(MAPF_ERR_INVALID, "mapf_group_step: NULL buffer");
     if (!uniforms && !g->philox_ok)
         return fail(MAPF_ERR_UNSUPPORTED, "device-side sampling needs slip probabilities that add up to 1; pass uniforms");
