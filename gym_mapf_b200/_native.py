@@ -17,14 +17,15 @@ OPT_AUTO_RESET = 1
 OPT_SHARE_SM = 2
 OPT_COMPACT = 4
 FLAG_DONE, FLAG_COLLISION = 1, 2
-POLICY_RANDOM, POLICY_JOINT, POLICY_AGENTS = 0, 1, 2
+POLICY_RANDOM, POLICY_JOINT, POLICY_AGENTS, POLICY_GROUPS = 0, 1, 2, 3
+NO_CONFLICT = 0xFF  # conflict byte of an episode that did not end in a collision
 EPISODE_TIMEOUT, EPISODE_COLLISION, EPISODE_GOAL, EPISODE_TERMINAL_START = 0, 1, 2, 3
 
 EXPORTS = ["mapf_ctx_create", "mapf_ctx_destroy", "mapf_ctx_info", "mapf_ctx_moves", "mapf_ctx_reward_table", "mapf_decode_states",
            "mapf_encode_states", "mapf_count_rows", "mapf_scan_scratch_bytes", "mapf_scan_rows", "mapf_count_scan_rows",
            "mapf_count_scan_range", "mapf_expand",
            "mapf_count_range", "mapf_expand_range", "mapf_checksum", "mapf_step", "mapf_rollout", "mapf_step_host", "mapf_step_host_resident",
-           "mapf_evaluate_scratch_bytes", "mapf_evaluate",
+           "mapf_evaluate_scratch_bytes", "mapf_evaluate", "mapf_evaluate_groups",
            "mapf_backup", "mapf_backup_range", "mapf_greedy", "mapf_greedy_bcast", "mapf_count_predecessors", "mapf_predecessors",
            "mapf_projected_words", "mapf_project_states", "mapf_parse_map_text", "mapf_parse_scen_text", "mapf_ctx_create_from_text", "mapf_ctx_grid",
            "mapf_group_create", "mapf_group_destroy", "mapf_group_size", "mapf_group_step", "mapf_last_error",
@@ -102,6 +103,7 @@ def lib():
         L.mapf_evaluate_scratch_bytes.argtypes = []
         L.mapf_evaluate_scratch_bytes.restype = i64
         L.mapf_evaluate.argtypes = [vp, i32, vp, i64, i64, i64, C.c_double, u64, u64, i64, vp, vp, vp, vp, vp]
+        L.mapf_evaluate_groups.argtypes = [vp, vp, vp, i64, i64, i64, C.c_double, u64, u64, i64, vp, vp, vp, vp, vp, vp]
         L.mapf_backup.argtypes = [vp, vp, vp, i64, vp, i64, C.c_double, vp, vp]
         L.mapf_backup_range.argtypes = [vp, C.POINTER(u64 * 2), i64, vp, i64, C.c_double, vp, vp]
         L.mapf_greedy.argtypes = [vp, vp, i64, vp, vp, vp]
@@ -476,8 +478,13 @@ class Engine:
         steps, in one launch (mapf_evaluate).  Episode e draws what env `episode_offset + e` of `step` draws from
         `step_index` on.  `policy`: None (uniformly random joint actions, as `rollout` draws them), an int32[nS] tensor
         of joint actions indexed by the joint state, or an integer [n_agents, L] tensor of per-agent actions indexed by
-        the agent's cell.  Returns (returns f64[E], lengths i32[E], outcomes u8[E]) with outcomes EPISODE_*."""
+        the agent's cell, or a `GroupPolicy` (see `evaluate_groups`).  Returns (returns f64[E], lengths i32[E],
+        outcomes u8[E]) with outcomes EPISODE_*."""
         import torch
+        from .envs.vec_env import GroupPolicy
+        if isinstance(policy, GroupPolicy):
+            return self.evaluate_groups(policy, n_episodes, max_steps, gamma=gamma, seed=seed, step_index=step_index,
+                                        episode_offset=episode_offset, out=out)
         E = int(n_episodes)
         if E < 0:
             raise ValueError("n_episodes must be >= 0 (got %d)" % E)
@@ -515,6 +522,38 @@ class Engine:
         check(lib().mapf_evaluate(self._h, kind, _ptr(table), n_entries, E, int(max_steps), float(gamma), int(seed),
                                   int(step_index), int(episode_offset), _ptr(scratch), _ptr(ret), _ptr(length),
                                   _ptr(outcome), self._stream()))
+        return out
+
+    def evaluate_groups(self, policy, n_episodes, max_steps, gamma=1.0, seed=0, step_index=0, episode_offset=0, out=None,
+                        conflicts=None):
+        """`evaluate` for a `GroupPolicy` (mapf_evaluate_groups): each group of agents acts by its own table, indexed by
+        the group's local state.  `conflicts` (u8[E] device tensor, optional) receives, for every episode that ends in a
+        collision, the pair i | j << 4 (i < j) of its last step's clash -- agents of different groups first -- and
+        NO_CONFLICT for every other episode."""
+        import torch
+        E = int(n_episodes)
+        if E < 0:
+            raise ValueError("n_episodes must be >= 0 (got %d)" % E)
+        if policy.n_agents != self.n or policy.n_cells != self.L or policy.tables[0].device != self.torch_device:
+            raise ValueError("the GroupPolicy is for %d agents on %d cells on %s; this env has %d agents on %d cells on %s"
+                             % (policy.n_agents, policy.n_cells, policy.tables[0].device, self.n, self.L,
+                                self.torch_device))
+        tables = policy.tables[0].contiguous() if len(policy.tables) == 1 else torch.cat(policy.tables)
+        group_of = (C.c_int32 * self.n)(*policy.group_of())
+        dev = self.torch_device
+        if out is None:
+            out = (torch.empty(E, dtype=torch.float64, device=dev), torch.empty(E, dtype=torch.int32, device=dev),
+                   torch.empty(E, dtype=torch.uint8, device=dev))
+        ret, length, outcome = out
+        self._check_tensor("returns", ret, torch.float64, (E,))
+        self._check_tensor("lengths", length, torch.int32, (E,))
+        self._check_tensor("outcomes", outcome, torch.uint8, (E,))
+        if conflicts is not None:
+            self._check_tensor("conflicts", conflicts, torch.uint8, (E,))
+        scratch = torch.empty((int(lib().mapf_evaluate_scratch_bytes()) + 7) // 8, dtype=torch.int64, device=dev)
+        check(lib().mapf_evaluate_groups(self._h, group_of, _ptr(tables), tables.numel(), E, int(max_steps),
+                                         float(gamma), int(seed), int(step_index), int(episode_offset), _ptr(scratch),
+                                         _ptr(ret), _ptr(length), _ptr(outcome), _ptr(conflicts), self._stream()))
         return out
 
     # ---- rows next to the hot path (SURVEY.md 8f) ----------------------------------------------------------

@@ -69,7 +69,7 @@ struct mapf_ctx {
     int threads_step = 0;  // CTA size of k_step (ks.step_threads, else `threads`)
     int grid_step1 = 0, grid_step2 = 0, grid_step_tape = 0, grid_rollout = 0, grid_rollout2 = 0, grid_rollout_tape = 0;
     int grid_expand = 0, grid_expand_range = 0, grid_plain = 0, grid_backup = 0, grid_backup_range = 0;
-    int grid_evaluate[3] = {0, 0, 0};   // k_evaluate by policy kind
+    int grid_evaluate[4] = {0, 0, 0, 0};  // k_evaluate / k_evaluate_groups by policy kind
     KernelSet ks;
     u32 pat_triple[MAPF_MAX_PATTERNS];  // merge patterns (see PatternList)
     int n_patterns = 0;
@@ -554,7 +554,8 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
         {ctx->ks.backup_range, ctx->smem_backup, &ctx->grid_backup_range},
         {ctx->ks.evaluate[MAPF_POLICY_RANDOM], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_RANDOM]},
         {ctx->ks.evaluate[MAPF_POLICY_JOINT], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_JOINT]},
-        {ctx->ks.evaluate[MAPF_POLICY_AGENTS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_AGENTS]}};
+        {ctx->ks.evaluate[MAPF_POLICY_AGENTS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_AGENTS]},
+        {ctx->ks.evaluate[MAPF_POLICY_GROUPS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_GROUPS]}};
     for (auto &pl : plan) {
         if (!pl.fn) continue;  // two-word states have no backup kernels; wide step CTAs have no EPT = 2 k_step
         if (pl.smem > smem_limit) {
@@ -1202,6 +1203,70 @@ extern "C" int mapf_evaluate(const mapf_ctx *ctx, int32_t policy_kind, const voi
     void *args[] = {&sp, &keys, &policy, &E, &T, &gamma, &st, &e0, &scratch, &ret, &length, &outcome};
     LAUNCH(fn, grid_for(n_episodes, ctx->threads, ctx->grid_evaluate[policy_kind]), ctx->threads, ctx->smem_base, stream,
            args);
+    return MAPF_OK;
+}
+
+extern "C" int mapf_evaluate_groups(const mapf_ctx *ctx, const int32_t *group_of, const int32_t *tables,
+                                    int64_t tables_len, int64_t n_episodes, int64_t max_steps, double gamma,
+                                    uint64_t seed, uint64_t step_index0, int64_t episode_offset, void *scratch,
+                                    double *ret, int32_t *length, uint8_t *outcome, uint8_t *conflict, void *stream) {
+    if (!ctx || !group_of || !tables || n_episodes < 0 || (n_episodes > 0 && (!scratch || !ret || !length || !outcome)))
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: bad argument");
+    if (max_steps < 1 || max_steps >= (1ll << 31))
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: max_steps = %lld, must be in [1, 2**31)", (long long)max_steps);
+    if (n_episodes > MAPF_LAUNCH_MAX_ENVS)
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: at most 2**30 episodes per call");
+    const int n = ctx->sp.n;
+    const u64 L = (u64)ctx->sp.L;
+    int size[MAPF_MAXN] = {0}, pos[MAPF_MAXN], n_groups = 0;
+    for (int i = 0; i < n; ++i) {
+        const int g = group_of[i];
+        if (g < 0 || g > n_groups)  // canonical: a new group takes the next id
+            return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: group_of[%d] = %d, must be in [0, %d]", i, g, n_groups);
+        if (g == n_groups) ++n_groups;
+        pos[i] = size[g]++;
+    }
+    // table g holds L**size[g] entries at first[g]; every partial sum stays below 2**63
+    u64 first[MAPF_MAXN], total = 0, powL[MAPF_MAXN + 1];
+    powL[0] = 1;
+    for (int k = 1; k <= n; ++k) powL[k] = powL[k - 1] > (u64)INT64_MAX / L ? (u64)INT64_MAX : powL[k - 1] * L;
+    for (int g = 0; g < n_groups; ++g) {
+        if (powL[size[g]] == (u64)INT64_MAX || total > (u64)INT64_MAX - powL[size[g]])
+            return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: the tables have more than 2**63 - 1 entries");
+        first[g] = total;
+        total += powL[size[g]];
+    }
+    if (tables_len < 0 || (u64)tables_len != total)
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: the groups' tables have %llu entries (tables_len = %lld)",
+                    (unsigned long long)total, (long long)tables_len);
+    if (!ctx->philox_ok)
+        return fail(MAPF_ERR_UNSUPPORTED, "device-side sampling needs slip probabilities that add up to 1");
+    if (n_episodes == 0) return MAPF_OK;
+    const void *fn = ctx->ks.evaluate[MAPF_POLICY_GROUPS];
+    if (!fn) return fail(MAPF_ERR_UNSUPPORTED, "mapf_evaluate_groups: no kernel");
+    GroupLayout gl;
+    memset(&gl, 0, sizeof(gl));
+    for (int i = 0; i < n; ++i) {
+        const int g = group_of[i];
+        for (int j = 0; j < n; ++j) gl.mul[i][j] = group_of[j] == g ? powL[pos[j]] : 0;
+        gl.off[i] = first[g];
+        u64 d = 5;  // 5**(pos[i] + 1) <= 5**13 < 2**32: not a divisor of 2**64, so the ceiling is floor + 1
+        for (int k = 0; k < pos[i]; ++k) d *= 5;
+        gl.frac[i] = ~0ull / d + 1;
+        u32 a = 1;
+        for (int k = 0; k < size[g]; ++k) a *= 5u;
+        gl.amax[i] = a - 1u;
+        gl.group[i] = (u32)g;
+    }
+    DeviceGuard dg(ctx->device);
+    CUDA_TRY(cudaMemsetAsync(scratch, 0, sizeof(u32), (cudaStream_t)stream));
+    DevSpec sp = ctx->sp;
+    PhiloxKeys keys = make_keys(seed);
+    u32 E = (u32)n_episodes, T = (u32)max_steps;
+    u64 st = step_index0, e0 = (u64)episode_offset;
+    void *args[] = {&sp, &keys, &tables, &gl, &E, &T, &gamma, &st, &e0, &scratch, &ret, &length, &outcome, &conflict};
+    LAUNCH(fn, grid_for(n_episodes, ctx->threads, ctx->grid_evaluate[MAPF_POLICY_GROUPS]), ctx->threads, ctx->smem_base,
+           stream, args);
     return MAPF_OK;
 }
 

@@ -22,7 +22,8 @@ struct KernelSet {
     int compact_len_bytes = 0;
     const void *decode = nullptr, *encode = nullptr;
     const void *backup = nullptr, *backup_range = nullptr;  // k_backup<N, LUTS, RANGE>; one-word states only
-    const void *evaluate[3] = {nullptr, nullptr, nullptr};  // k_evaluate<N, W, LUTS, POLICY> by MAPF_POLICY_* kind
+    // by MAPF_POLICY_* kind: k_evaluate<N, W, LUTS, POLICY> for 0..2, k_evaluate_groups<N, W, LUTS> for 3
+    const void *evaluate[4] = {nullptr, nullptr, nullptr, nullptr};
     const void *pred_count = nullptr, *pred_emit = nullptr, *project = nullptr;
     size_t expand_slab_bytes = 0;        // per warp
     int expand_threads = 0;              // CTA size of k_expand (0: the context's)

@@ -61,6 +61,7 @@ static void fill(KernelSet *k) {
     k->evaluate[0] = (const void *)k_evaluate<N, W, LUTS, 0>;
     if constexpr (W == 1) k->evaluate[1] = (const void *)k_evaluate<N, W, LUTS, 1>;  // policy indexed by the joint state
     k->evaluate[2] = (const void *)k_evaluate<N, W, LUTS, 2>;
+    k->evaluate[3] = (const void *)k_evaluate_groups<N, W, LUTS>;
     k->pred_count = (const void *)k_pred_count<N, W>;
     k->pred_emit = (const void *)k_pred_emit<N, W>;
     k->project = (const void *)k_project<N, W>;

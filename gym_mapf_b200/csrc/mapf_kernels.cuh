@@ -1489,15 +1489,47 @@ k_rollout(DevSpec sp, PhiloxKeys keys, u64 *states, const int *__restrict__ acti
 //   POLICY 0 (MAPF_POLICY_RANDOM)  the uniform joint action k_rollout draws (random_action)
 //   POLICY 1 (MAPF_POLICY_JOINT)   int32 policy[s], indexed by the one-word joint state
 //   POLICY 2 (MAPF_POLICY_AGENTS)  u8 policy[i * L + cell of agent i]: each agent's action from its own cell
+//   POLICY 3 (MAPF_POLICY_GROUPS)  int32 tables of agent groups, read through a GroupLayout (k_evaluate_groups)
 // The return G = G + disc * r, disc = disc * gamma is accumulated with single binary64 operations (no FMA), and the
 // episode stops at its first done.  Nothing is stored per step: ret / length / outcome of episode e are written when it
 // ends (outcome = the step's kind: 1 clash, 2 goal, 3 the start state was terminal; 0 = no done within T steps).
 // A lane whose episode ends takes the next episode index of the queue (`counter`, one warp-aggregated atomic per warp
 // and refill), so a warp's lanes stay busy until the queue drains instead of waiting for the warp's longest episode.
+
+// The agent groups of a MAPF_POLICY_GROUPS policy, per agent i (built by mapf_evaluate_groups).  Group g with agents
+// g_0 < g_1 < ... owns L**|g| int32 entries at off[g_0]; entry sum_k cell[g_k] * L**k holds the group's joint action,
+// base 5, agent g_k's digit at 5**k.
+struct GroupLayout {
+    u64 mul[MAPF_MAXN][MAPF_MAXN];  // [i][j]: L**(position of j in its group) when j is in i's group, else 0
+    u64 off[MAPF_MAXN];             // first entry of the table of i's group
+    u64 frac[MAPF_MAXN];            // ceil(2**64 / 5**(position of i + 1)): extracts i's digit (see evaluate_episodes)
+    u32 amax[MAPF_MAXN];            // 5**|i's group| - 1: larger entries are clamped to it
+    u32 group[MAPF_MAXN];           // group id of i
+};
+
+// The pair (i < j) a collision step is attributed to, as i | j << 4: the lexicographically smallest pair of agents in
+// different groups that clashed (a vertex or a swap conflict, the two tests of has_clash), else the smallest pair.
+template <int N>
+__device__ __forceinline__ u32 clash_pair(const GroupLayout &gl, const int (&prev)[N], const int (&nxt)[N]) {
+    u32 any = 0xffu, cross = 0xffu;
+#pragma unroll
+    for (int i = N - 1; i >= 0; --i)
+#pragma unroll
+        for (int j = N - 1; j > i; --j)
+            if (nxt[i] == nxt[j] || (nxt[i] == prev[j] && nxt[j] == prev[i])) {
+                any = (u32)i | (u32)j << 4;
+                if (gl.group[i] != gl.group[j]) cross = any;
+            }
+    return cross != 0xffu ? cross : any;
+}
+
+// The episode loop of every policy kind.  `gl` and `conflict` are used by POLICY 3 only.  (The kernels' parameters
+// carry __restrict__; passing sp and keys by value and no qualifiers here keeps k_evaluate's machine code as it was
+// before this loop was shared.)
 template <int N, int WORDS, bool LUTS, int POLICY>
-__global__ void __launch_bounds__(MAPF_MAX_THREADS, MAPF_MIN_BLOCKS(N))
-k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, u32 T, double gamma, u64 step0, u64 e0,
-           u32 *__restrict__ counter, double *__restrict__ ret, int *__restrict__ length, u8 *__restrict__ outcome) {
+__device__ __forceinline__ void evaluate_episodes(DevSpec sp, PhiloxKeys keys, const void *policy, const GroupLayout *gl,
+                                                  u32 E, u32 T, double gamma, u64 step0, u64 e0, u32 *counter,
+                                                  double *ret, int *length, u8 *outcome, u8 *conflict) {
     extern __shared__ __align__(16) unsigned char smem[];
     SmemTables tb = tables_begin<LUTS>(sp, smem);
     const u32 n_threads = gridDim.x * blockDim.x;
@@ -1517,7 +1549,23 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
         bool ended = false;
         if (live) {
             const u64 env = e0 + (u64)e, stp = step0 + (u64)t;
-            if (POLICY == 0) {
+            if constexpr (POLICY == 3) {
+                // Each agent indexes its own group's table with its group's local state (an unrolled N x N sum whose
+                // multipliers are 0 outside the group: no register array is indexed by a run-time group id) and takes
+                // its digit k of the entry v < 5**13 < 2**31: with f = v * ceil(2**64 / 5**(k + 1)) mod 2**64, f / 2**64
+                // is frac(v / 5**(k + 1)) + eps, eps < 2**-33, and 5 * (the top 32 bits of f, plus 1) / 2**32 has the
+                // digit as its integer part (the rounding stays below 1 / 5**k).
+                const int *tables = reinterpret_cast<const int *>(policy);
+#pragma unroll
+                for (int i = 0; i < N; ++i) {
+                    u64 x = gl->off[i];
+#pragma unroll
+                    for (int j = 0; j < N; ++j) x += (u64)(u32)in.cell[j] * gl->mul[i][j];
+                    const u32 v = min((u32)__ldg(tables + x), gl->amax[i]);
+                    const u32 fhi = (u32)(((u64)v * gl->frac[i]) >> 32);
+                    in.actv[i] = __umulhi(fhi + 1u, 5u) * 8u + tb.act0;
+                }
+            } else if (POLICY == 0) {
                 load_actions<N>(sp, tb, random_action(sp, keys, env, stp), in.actv);
             } else if (POLICY == 1) {
                 load_actions<N>(sp, tb, (u32)__ldg(reinterpret_cast<const int *>(policy) + in.lo), in.actv);
@@ -1531,6 +1579,9 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
             int nxt[N];
             // after a step that was not done the state is not terminal (see env_step): only step 0 needs the test
             const EnvOut o = env_step<N, WORDS, LUTS, false>(sp, tb, in, nullptr, 0u, nxt, t > 0);
+            if constexpr (POLICY == 3)  // the episode ends here: its conflict byte (MAPF_NO_CONFLICT unless a clash)
+                if (conflict && (o.kind != 0u || t + 1u == T))
+                    conflict[e] = (u8)(o.kind == 1u ? clash_pair<N>(*gl, in.cell, nxt) : 0xffu);
             G = __dadd_rn(G, __dmul_rn(disc, o.reward));
             disc = __dmul_rn(disc, gamma);
             ++t;
@@ -1563,6 +1614,25 @@ k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, 
             for (int i = 0; i < N; ++i) in.cell[i] = (int)sp.start[i];
         }
     }
+}
+
+template <int N, int WORDS, bool LUTS, int POLICY>
+__global__ void __launch_bounds__(MAPF_MAX_THREADS, MAPF_MIN_BLOCKS(N))
+k_evaluate(DevSpec sp, PhiloxKeys keys, const void *__restrict__ policy, u32 E, u32 T, double gamma, u64 step0, u64 e0,
+           u32 *__restrict__ counter, double *__restrict__ ret, int *__restrict__ length, u8 *__restrict__ outcome) {
+    evaluate_episodes<N, WORDS, LUTS, POLICY>(sp, keys, policy, nullptr, E, T, gamma, step0, e0, counter, ret, length,
+                                              outcome, nullptr);
+}
+
+// MAPF_POLICY_GROUPS: `tables` holds the groups' tables; `conflict` (may be null) receives, per episode, the pair of
+// its last step's clash (clash_pair) when the episode ends in a collision, else 0xff.
+template <int N, int WORDS, bool LUTS>
+__global__ void __launch_bounds__(MAPF_MAX_THREADS, MAPF_MIN_BLOCKS(N))
+k_evaluate_groups(DevSpec sp, PhiloxKeys keys, const int *__restrict__ tables, const __grid_constant__ GroupLayout gl,
+                  u32 E, u32 T, double gamma, u64 step0, u64 e0, u32 *__restrict__ counter, double *__restrict__ ret,
+                  int *__restrict__ length, u8 *__restrict__ outcome, u8 *__restrict__ conflict) {
+    evaluate_episodes<N, WORDS, LUTS, 3>(sp, keys, tables, &gl, E, T, gamma, step0, e0, counter, ret, length, outcome,
+                                         conflict);
 }
 
 // =====================================================================================================

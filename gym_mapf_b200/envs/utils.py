@@ -1,5 +1,7 @@
 """Factories and parsers (reference gym_mapf/envs/utils.py): MovingAI `.map` / `.scen` parsing, env construction
 by map name, the synthetic multi-room "sanity" env and agent-subset views.  Host-side setup only."""
+import collections
+
 from . import map_name_to_files
 from .grid import MapfGrid
 from .mapf_env import MapfEnv
@@ -106,6 +108,67 @@ def independent_policy(env: MapfEnv, gamma=1.0, eps=1e-6, max_iter=1000):
         _, pi, _ = VecMapfEnv(get_local_view(env, [i]), 1).value_iteration(gamma=gamma, eps=eps, max_iter=max_iter)
         rows.append(pi)
     return torch.stack(rows).contiguous()
+
+
+def _plan_group(env, group, gamma, eps, max_iter, slab):
+    from .vec_env import VecMapfEnv
+    _, pi, _ = VecMapfEnv(get_local_view(env, list(group)), 1).value_iteration(gamma=gamma, eps=eps, max_iter=max_iter,
+                                                                              slab=slab)
+    return pi
+
+
+def group_policy(env: MapfEnv, groups, gamma=1.0, eps=1e-6, max_iter=1000, slab=None):
+    """The product of jointly optimal group policies: for each group g, `value_iteration` of the agent-subset env
+    `get_local_view(env, g)`, whose policy is indexed by g's local state.  `independent_policy` with any grouping:
+    singleton groups give tables equal to its rows.  `slab` bounds the states of one backup launch.  Returns a
+    GroupPolicy (groups in canonical order)."""
+    from .vec_env import GroupPolicy
+    groups = [tuple(sorted(int(a) for a in g)) for g in groups]
+    return GroupPolicy(groups, [_plan_group(env, g, gamma, eps, max_iter, slab) for g in groups])
+
+
+IndependenceDetection = collections.namedtuple("IndependenceDetection", "policy resolved log")
+
+
+def independence_detection(env: MapfEnv, n_episodes=1 << 20, max_steps=256, gamma=1.0, seed=0, max_group_size=3,
+                           max_table_entries=1 << 28, eps=1e-6, max_iter=1000):
+    """Independence detection: plan every agent alone, then repeatedly evaluate the product of the group policies
+    (`VecMapfEnv.find_conflicts`, `n_episodes` episodes of at most `max_steps` steps from Philox stream `seed`), merge
+    the two groups with the most episodes whose collision is attributed to a pair of agents across them (ties: the
+    lowest group ids), and re-plan the merged group jointly with `value_iteration`.  Stops when no episode collides
+    across groups (resolved=True), or when the next merge would make a group of more than `max_group_size` agents or a
+    table of more than `max_table_entries` entries (resolved=False).
+
+    Detection is sampled: a conflict is found only if it occurs in the evaluated episodes, so resolved=True means that
+    none of them collided across groups, not that no reachable state does.  The run is deterministic for a seed.
+    Returns IndependenceDetection(policy: GroupPolicy, resolved, log), with one log record per evaluation round:
+    {"groups", "counts" (int64[n, n] attributed collision episodes per agent pair, on the CPU), "summary"
+    (`evaluation_summary`)}."""
+    from .vec_env import GroupPolicy, VecMapfEnv, evaluation_summary
+    vec = VecMapfEnv(env, 1, seed=seed, auto_reset=False)
+    L = len(env.valid_locations)
+    plans = {(i,): _plan_group(env, (i,), gamma, eps, max_iter, None) for i in range(env.n_agents)}
+    log = []
+    while True:
+        groups = sorted(plans, key=lambda g: g[0])
+        policy = GroupPolicy(groups, [plans[g] for g in groups])
+        found = vec.find_conflicts(policy, n_episodes, max_steps, gamma=gamma)
+        counts = found.counts.cpu()
+        log.append(dict(groups=policy.groups, counts=counts, summary=evaluation_summary(found.evaluation)))
+        gid = policy.group_of()
+        across = collections.Counter()
+        for i in range(env.n_agents):
+            for j in range(i + 1, env.n_agents):
+                if gid[i] != gid[j] and int(counts[i, j]):
+                    across[(min(gid[i], gid[j]), max(gid[i], gid[j]))] += int(counts[i, j])
+        if not across:
+            return IndependenceDetection(policy, True, log)
+        ga, gb = min(across, key=lambda k: (-across[k], k))
+        merged = tuple(sorted(policy.groups[ga] + policy.groups[gb]))
+        if len(merged) > max_group_size or L ** len(merged) > max_table_entries:
+            return IndependenceDetection(policy, False, log)
+        del plans[policy.groups[ga]], plans[policy.groups[gb]]
+        plans[merged] = _plan_group(env, merged, gamma, eps, max_iter, None)
 
 
 def mapf_env_load_from_json(json_str: str) -> MapfEnv:

@@ -14,6 +14,80 @@ Transitions = collections.namedtuple("Transitions", "row_ptr next_state prob rew
 Rollout = collections.namedtuple("Rollout", "next_state reward prob done collision")
 # per episode: return f64, length i32 (steps taken), outcome u8 (0 timeout, 1 collision, 2 goal, 3 the start was terminal)
 Evaluation = collections.namedtuple("Evaluation", "returns lengths outcomes")
+# find_conflicts: the Evaluation, the attributed pair per episode (u8[E], i | j << 4 or NO_CONFLICT) and counts[i, j]
+# (int64[n, n], i < j): the number of episodes attributed to the pair (i, j)
+Conflicts = collections.namedtuple("Conflicts", "evaluation pairs counts")
+
+
+def _int_root(x, k):
+    r = int(round(x ** (1.0 / k)))
+    while r > 0 and r ** k > x:
+        r -= 1
+    while (r + 1) ** k <= x:
+        r += 1
+    return r
+
+
+class GroupPolicy(collections.namedtuple("GroupPolicy", "groups tables")):
+    """A product of group policies: the agents are split into groups, and each group acts jointly by its own table.
+
+    `groups`: a tuple of agent tuples that partitions agents 0..n-1, each ascending, in canonical order (by lowest
+    agent).  `tables[g]`: int32[L**|g|] on the device, the group's joint action (base 5, agent g[k]'s digit at 5**k)
+    indexed by the group's local state sum_k cell[g[k]] * L**k -- exactly the policy `value_iteration` returns on
+    `get_local_view(env, g)`, and what `VecMapfEnv.project(states, g)` computes.  The constructor puts the groups (with
+    their tables) in canonical order and rejects anything else it cannot use: agents out of order inside a group, a set
+    of groups that does not partition 0..n-1, tables of the wrong dtype, length, device, or with entries outside
+    [0, 5**|g|)."""
+    __slots__ = ()
+
+    def __new__(cls, groups, tables):
+        import torch
+        groups = [tuple(int(a) for a in g) for g in groups]
+        tables = list(tables)
+        if not groups or len(tables) != len(groups):
+            raise ValueError("a GroupPolicy needs one table per group (got %d groups, %d tables)"
+                             % (len(groups), len(tables)))
+        for g in groups:
+            if not g or any(a >= b for a, b in zip(g, g[1:])):
+                raise ValueError("the agents of a group must be distinct and ascending (got %s)" % (g,))
+        agents = sorted(a for g in groups for a in g)
+        if agents != list(range(len(agents))):
+            raise ValueError("the groups must partition the agents 0..n-1 (got %s)" % (groups,))
+        order = sorted(range(len(groups)), key=lambda k: groups[k][0])
+        groups, tables = tuple(groups[k] for k in order), [tables[k] for k in order]
+        L, device = None, None
+        for g, t in zip(groups, tables):
+            if not isinstance(t, torch.Tensor) or t.dtype is not torch.int32 or t.dim() != 1 or t.numel() == 0:
+                raise ValueError("the table of group %s must be a non-empty int32[L**%d] tensor" % (g, len(g)))
+            r = _int_root(t.numel(), len(g))
+            if r ** len(g) != t.numel() or (L is not None and r != L):
+                raise ValueError("the table of group %s has %d entries, not L**%d%s"
+                                 % (g, t.numel(), len(g), "" if L is None else " = %d" % L ** len(g)))
+            if device is not None and t.device != device:
+                raise ValueError("all tables must be on one device (got %s and %s)" % (device, t.device))
+            L, device = r, t.device
+            lo, hi = (int(v) for v in torch.aminmax(t))
+            if lo < 0 or hi >= 5 ** len(g):
+                raise ValueError("the entries of group %s's table must lie in [0, %d) (got [%d, %d])"
+                                 % (g, 5 ** len(g), lo, hi))
+        return super().__new__(cls, groups, tables)
+
+    @property
+    def n_agents(self):
+        return sum(len(g) for g in self.groups)
+
+    @property
+    def n_cells(self):
+        """L, the number of free cells the tables are indexed over."""
+        return _int_root(self.tables[0].numel(), len(self.groups[0]))
+
+    def group_of(self):
+        """The group id of every agent (a list of n_agents ints)."""
+        out = [0] * self.n_agents
+        for gid, g in enumerate(self.groups):
+            for a in g:
+                out[a] = gid
+        return out
 
 
 def evaluation_summary(ev):
@@ -134,11 +208,29 @@ class VecMapfEnv:
         batch stepped from a reset with `actions = policy(states)` and no auto-reset, cut at its first done or after
         `max_steps` steps.  It draws from the Philox stream of `self.seed` (or `seed`) at `self.env_offset + e`, from
         step `self.step_count` on.  `policy`: None (uniformly random joint actions), int32[nS] joint actions by joint
-        state (`value_iteration`'s policy), or an integer [n_agents, L] table of per-agent actions by cell
-        (`independent_policy`).  Returns an Evaluation; `self.states` and `step_count` are left as they are."""
+        state (`value_iteration`'s policy), an integer [n_agents, L] table of per-agent actions by cell
+        (`independent_policy`), or a GroupPolicy (`group_policy`).  Returns an Evaluation; `self.states` and
+        `step_count` are left as they are."""
         out = self.engine.evaluate(policy, n_episodes, max_steps, gamma=gamma, seed=self.seed if seed is None else seed,
                                    step_index=self.step_count, episode_offset=self.env_offset)
         return Evaluation(*out)
+
+    def find_conflicts(self, policy, n_episodes, max_steps, gamma=1.0, seed=None):
+        """`evaluate` of a GroupPolicy that also names, for every episode that ends in a collision, the pair of agents
+        (i < j) that clashed on its last step: the lexicographically smallest pair of agents in different groups, else
+        the smallest pair inside one group.  This is sampled: it sees the collisions of these episodes, not every
+        reachable one.  Returns Conflicts(evaluation, pairs u8[E] (i | j << 4, or NO_CONFLICT), counts int64[n, n])."""
+        from .. import _native
+        torch = self._torch
+        if not isinstance(policy, GroupPolicy):
+            raise ValueError("find_conflicts needs a GroupPolicy (got %s)" % type(policy).__name__)
+        E, n = int(n_episodes), self.n_agents
+        pairs = torch.empty(max(E, 0), dtype=torch.uint8, device=self.device)
+        out = self.engine.evaluate_groups(policy, E, max_steps, gamma=gamma, seed=self.seed if seed is None else seed,
+                                          step_index=self.step_count, episode_offset=self.env_offset, conflicts=pairs)
+        p = pairs[pairs != _native.NO_CONFLICT].long()
+        counts = torch.bincount((p & 15) * n + (p >> 4), minlength=n * n).view(n, n)
+        return Conflicts(Evaluation(*out), pairs, counts)
 
     # ---- transition table --------------------------------------------------------------------------------------
     def transitions(self, states, actions):

@@ -181,8 +181,11 @@ enum { MAPF_EPISODE_TIMEOUT = 0, MAPF_EPISODE_COLLISION = 1, MAPF_EPISODE_GOAL =
 enum {
     MAPF_POLICY_RANDOM = 0, /* a uniformly random joint action per step, drawn as mapf_rollout draws it (policy unused) */
     MAPF_POLICY_JOINT = 1,  /* int32 policy[policy_len], indexed by the joint state (policy_len >= nS; one-word states) */
-    MAPF_POLICY_AGENTS = 2  /* uint8 policy[n_agents * L]: agent i on cell c intends action policy[i * L + c] */
+    MAPF_POLICY_AGENTS = 2, /* uint8 policy[n_agents * L]: agent i on cell c intends action policy[i * L + c] */
+    MAPF_POLICY_GROUPS = 3  /* int32 tables of agent groups, one per group (mapf_evaluate_groups) */
 };
+/* conflict[e] of mapf_evaluate_groups for an episode that did not end in a collision */
+#define MAPF_NO_CONFLICT 0xFF
 
 /* Bytes of device scratch mapf_evaluate needs (its work counter).  Concurrent calls need separate scratch. */
 int64_t mapf_evaluate_scratch_bytes(void);
@@ -201,6 +204,33 @@ int64_t mapf_evaluate_scratch_bytes(void);
 int mapf_evaluate(const mapf_ctx *ctx, int32_t policy_kind, const void *policy, int64_t policy_len, int64_t n_episodes,
                   int64_t max_steps, double gamma, uint64_t seed, uint64_t step_index0, int64_t episode_offset,
                   void *scratch, double *ret, int32_t *length, uint8_t *outcome, void *stream);
+
+/* mapf_evaluate for a product of group policies, with the pair of agents each collision episode is attributed to.
+ * group_of (HOST, n_agents entries) splits the agents into groups numbered canonically: group_of[0] = 0, and each
+ * further group takes the next id in the order of its lowest agent.  Group g with agents g_0 < g_1 < ... acts by
+ * int32 table_g[L**|g|]: in joint state s it takes the group joint action
+ *     table_g[sum_k cell(s, g_k) * L**k]        (the local state mapf_project_states(ctx, s, g) computes)
+ * and agent g_k intends digit k of it, base 5 -- so table_g is the policy value iteration returns on the agent-subset
+ * env of g.  `tables` (DEVICE) is table_0, table_1, ... concatenated, tables_len = sum_g L**|g| entries.  Singleton
+ * groups act like MAPF_POLICY_AGENTS, one group of every agent like MAPF_POLICY_JOINT.  Episode e is exactly
+ *     s = start state; G = 0; disc = 1
+ *     for t in range(max_steps):
+ *         a = sum_i 5**i * digit(table_{group_of[i]}[local state of group_of[i] in s], position of i in its group)
+ *         s_prev = s; s, r, done = mapf_step(s, a) with Philox counter (episode_offset + e, step_index0 + t), no auto-reset
+ *         G = G + disc * r; disc = disc * gamma        (single binary64 operations, no fused multiply-add)
+ *         if done: break
+ * with ret / length / outcome as in mapf_evaluate (same draws, queue and scratch; out-of-range entries are clamped to
+ * 5**|g| - 1).  conflict (DEVICE, may be NULL): for an episode whose outcome is MAPF_EPISODE_COLLISION,
+ * conflict[e] = i | j << 4 for the lexicographically smallest pair i < j that clashed in its last step (next_i == next_j,
+ * or next_i == prev_j and next_j == prev_i), where pairs of agents in different groups come before pairs inside one
+ * group; MAPF_NO_CONFLICT for every other episode.
+ * Rejected (MAPF_ERR_INVALID): the arguments mapf_evaluate rejects, a NULL group_of or tables, a group_of that is not
+ * canonical or has an id outside [0, n_agents), and tables_len != sum_g L**|g| (or a sum that overflows int64).
+ * A context whose slip probabilities do not add up to 1 is MAPF_ERR_UNSUPPORTED. */
+int mapf_evaluate_groups(const mapf_ctx *ctx, const int32_t *group_of, const int32_t *tables, int64_t tables_len,
+                         int64_t n_episodes, int64_t max_steps, double gamma, uint64_t seed, uint64_t step_index0,
+                         int64_t episode_offset, void *scratch, double *ret, int32_t *length, uint8_t *outcome,
+                         uint8_t *conflict, void *stream);
 
 /* Host-buffer convenience call (end-to-end path): copies states/actions from HOST memory, steps, copies the five
  * results back to HOST memory, on the context's own streams; returns when the results are in host memory. */
