@@ -420,3 +420,152 @@ def test_evaluate_errors(torch):
     base = eng.evaluate(torch.ones((eng.n, eng.L), dtype=torch.uint8, device=dev), E, 20, seed=1)
     other = eng.evaluate(torch.ones((eng.n, eng.L), dtype=torch.int64, device=dev), E, 20, seed=1)
     assert all(torch.equal(a, b) for a, b in zip(base, other))
+
+
+# ---- 10. out-of-range entries through the C ABI are clamped ------------------------------------------------------------
+def c_evaluate(eng, policy, E, T, out, scratch=None, gamma=0.95, seed=3, step_index=0, episode_offset=0):
+    """One mapf_evaluate (policy = (kind, table)) or mapf_evaluate_groups (policy = (POLICY_GROUPS, tables, group_of))
+    call; `out` is (ret, length, outcome) plus, for groups, the conflict output (or None)."""
+    import torch
+    from gym_mapf_b200._native import POLICY_GROUPS, _ptr, check, lib
+    if scratch is None:
+        scratch = torch.empty(2, dtype=torch.int64, device=eng.torch_device)
+    table = policy[1]
+    n = 0 if table is None else table.numel()
+    if policy[0] == POLICY_GROUPS:
+        gof = (C.c_int32 * eng.n)(*policy[2])
+        check(lib().mapf_evaluate_groups(eng._h, gof, _ptr(table), n, E, T, gamma, seed, step_index, episode_offset,
+                                         _ptr(scratch), *(_ptr(x) for x in out), eng._stream()))
+    else:
+        check(lib().mapf_evaluate(eng._h, policy[0], _ptr(table), n, E, T, gamma, seed, step_index, episode_offset,
+                                  _ptr(scratch), *(_ptr(x) for x in out), eng._stream()))
+    return out
+
+
+def new_outputs(torch, eng, E, conflict=False):
+    dev = eng.torch_device
+    out = (torch.empty(E, dtype=torch.float64, device=dev), torch.empty(E, dtype=torch.int32, device=dev),
+           torch.empty(E, dtype=torch.uint8, device=dev))
+    return out + ((torch.empty(E, dtype=torch.uint8, device=dev),) if conflict else ())
+
+
+def assert_clamped(torch, eng, make_policy, table, bad, top, rng, E=20000, T=100):
+    """Some entries of `table` overwritten with the values `bad` give bit for bit the episodes of the same entries set
+    to `top`, the documented maximum; and those entries are read (the episodes differ from the unmodified table's).
+    `bad` and `top` hold scalars or per-entry arrays."""
+    hit = np.flatnonzero(rng.random(len(table)) < 0.3)
+    cand = np.stack([np.broadcast_to(np.asarray(b, np.int64), table.shape) for b in bad])
+    worst, capped = table.copy(), table.copy()
+    worst[hit] = cand[rng.integers(0, len(bad), len(hit)), hit].astype(table.dtype)
+    capped[hit] = np.broadcast_to(top, table.shape)[hit]
+    dev = eng.torch_device
+    conflict = make_policy(None)[0] == 3
+    got = [c_evaluate(eng, make_policy(torch.from_numpy(t).to(dev)), E, T, new_outputs(torch, eng, E, conflict))
+           for t in (worst, capped, table)]
+    assert all(torch.equal(a, b) for a, b in zip(got[0], got[1]))
+    assert not all(torch.equal(a, b) for a, b in zip(got[1], got[2]))
+
+
+@pytest.mark.parametrize("case", ["joint_c1", "agents_c2", "agents_c4"])
+def test_out_of_range_entries_are_clamped(case, torch):
+    """JOINT entries >= nA or < 0 act as nA - 1; AGENTS entries above 4 act as 4 (LEFT).  The Python layer rejects such
+    tables, so only C callers reach the clamp."""
+    from gym_mapf_b200._native import POLICY_AGENTS, POLICY_JOINT
+    rng = np.random.default_rng(len(case))
+    if case == "joint_c1":
+        eng = c1_env(soc=True).engine
+        nA = int(eng.nA)
+        table = rng.integers(0, nA, int(eng.nS)).astype(np.int32)
+        assert_clamped(torch, eng, lambda t: (POLICY_JOINT, t), table, [nA, (1 << 31) - 1, -1], nA - 1, rng)
+    else:  # planned tables: with random ones the agents never meet or arrive, and every episode is a timeout alike
+        from gym_mapf_b200.envs.utils import independent_policy
+        env = env_of(G.load("rows_" + case[-2:])[0])
+        eng = env.engine
+        table = independent_policy(env).cpu().numpy().astype(np.uint8).reshape(-1)
+        assert_clamped(torch, eng, lambda t: (POLICY_AGENTS, t), table, [5, 17, 255], 4, rng)
+
+
+# ---- 11. the episode queue: lanes refill past the resident threads of a launch -----------------------------------------
+QUEUE_CASES = ["random_c1", "agents_c1", "joint_c1", "groups_c2", "groups_c5_n10"]
+SENTINEL_RET = 0x7FF4DEADBEEF0001  # the bits of a NaN, which no return is
+
+
+def queue_policy(torch, case):
+    """(engine, oracle, C ABI policy, replay policy, replay kind) of a queue case."""
+    from gym_mapf_b200._native import POLICY_AGENTS, POLICY_GROUPS, POLICY_JOINT, POLICY_RANDOM
+    from gym_mapf_b200.envs.vec_env import GroupPolicy
+    rng = np.random.default_rng(len(case))
+    if case.endswith("c1"):
+        env = c1_env(soc=True)
+        spec = dict(rows=["".join("@" if v else "." for v in r) for r in env.grid.obstacles], n_agents=2,
+                    goals=[list(g) for g in env.agents_goals], fail_prob=0.2, r_clash=-1000.0, r_goal=100.0,
+                    r_living=-1.0, soc=True)
+        eng, ora = env.engine, make_oracle(spec)
+    else:
+        spec = G.load("rows_" + case[len("groups_"):])[0]
+        eng, ora = make_engine(spec), make_oracle(spec)
+    dev = eng.torch_device
+    if case.startswith("random"):
+        return eng, ora, (POLICY_RANDOM, None), None, "random"
+    if case.startswith("agents"):
+        table = rng.integers(0, 5, (eng.n, eng.L))
+        return eng, ora, (POLICY_AGENTS, torch.from_numpy(table.astype(np.uint8)).to(dev)), table, "agents"
+    if case.startswith("joint"):
+        table = rng.integers(0, eng.nA, int(eng.nS)).astype(np.int32)
+        return eng, ora, (POLICY_JOINT, torch.from_numpy(table).to(dev)), table, "joint"
+    m = (eng.n + 1) // 2  # pairs of agents i, i + m (and a singleton when n is odd)
+    groups = [tuple(range(g, eng.n, m)) for g in range(m)]
+    tables = [rng.integers(0, 5 ** len(g), eng.L ** len(g), dtype=np.int32) for g in groups]
+    gp = GroupPolicy(groups, [torch.from_numpy(t).to(dev) for t in tables])
+    return eng, ora, (POLICY_GROUPS, torch.cat(gp.tables), gp.group_of()), (groups, tables), "groups"
+
+
+@pytest.mark.timeout(300)
+@pytest.mark.parametrize("case", QUEUE_CASES)
+def test_episode_queue_hands_out_every_episode_once(case, torch):
+    """E = 2**19 + 3 episodes: more than a B200 launch holds resident (148 SMs x 2048 threads = 303 104), so lanes take
+    further episodes from the queue.  Every output is written, with the episode the oracle computes for that index
+    (sampled up to E - 1), in two calls that share one scratch buffer, and three shards give the same records."""
+    from gym_mapf_b200 import sharding
+    from gym_mapf_b200._native import POLICY_GROUPS
+    from gym_mapf_b200.envs.vec_env import GroupPolicy
+    from test_gpu_kernel_matrix import SEED, assert_episodes, replay_episodes
+    eng, ora, policy, table, kind = queue_policy(torch, case)
+    E, T, gamma, step0, off = (1 << 19) + 3, 64, 0.95, 11, 1 << 33
+    groups = policy[0] == POLICY_GROUPS
+    scratch = torch.empty(2, dtype=torch.int64, device=eng.torch_device)
+    runs = []
+    for _ in range(2):
+        out = new_outputs(torch, eng, E, groups)
+        out[0].view(torch.int64).fill_(SENTINEL_RET)
+        out[1].fill_(-1)
+        for x in out[2:]:
+            x.fill_(0xEE)
+        c_evaluate(eng, policy, E, T, out, scratch=scratch, gamma=gamma, seed=SEED, step_index=step0,
+                   episode_offset=off)
+        assert bool((out[0].view(torch.int64) != SENTINEL_RET).all())
+        assert bool(((out[1] >= 1) & (out[1] <= T)).all()) and bool((out[2] <= 3).all())
+        if groups:
+            assert bool(((out[3] != 0xFF) == (out[2] == 1)).all()) and bool(((out[3] & 15) < (out[3] >> 4)).any())
+        runs.append(out)
+    assert all(torch.equal(a, b) for a, b in zip(*runs))
+    out = runs[0]
+    sub = np.unique(np.concatenate([np.arange(0, E, 257), np.arange(303104 - 40, 303104 + 40), [E - 1]]))
+    ep = replay_episodes(eng, ora, table, kind, T, gamma, step0, off, sub)
+    assert_episodes(out, ep, sub, case)
+    if groups:
+        assert np.array_equal(out[3].cpu().numpy()[sub], ep.pair) and (ep.outcome == 1).any()
+    assert (ep.outcome != ep.outcome[0]).any() and (ep.length < T).any()
+    pol = GroupPolicy(table[0], [torch.from_numpy(t).to(eng.torch_device) for t in table[1]]) if groups else policy[1]
+    parts = []
+    for rank in range(3):
+        sh = sharding.split_range(E, 3, rank, begin=off)
+        p = new_outputs(torch, eng, sh.count, groups)
+        if groups:
+            eng.evaluate_groups(pol, sh.count, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=sh.begin,
+                                out=p[:3], conflicts=p[3])
+        else:
+            eng.evaluate(pol, sh.count, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=sh.begin, out=p)
+        parts.append(p)
+    for k in range(len(out)):
+        assert torch.equal(torch.cat([p[k] for p in parts]), out[k])

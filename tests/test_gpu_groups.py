@@ -161,6 +161,40 @@ def test_cross_group_pair_comes_first(torch):
         assert bool((pairs == want).all()), (groups, pairs)
 
 
+def test_attribution_at_13_agents(torch):
+    """Thirteen agents on an open 3 x 13 grid (39**13 >= 2**63: two-word states, staged moves).  Agents 0-9 stand on
+    row 0 and STAY.  Agent 10 on (1, 10) goes RIGHT, 11 on (0, 11) DOWN and 12 on (2, 11) UP: a 3-way vertex clash on
+    (1, 11); or 10 STAYs and only 11 and 12 clash; optionally 4 and 5 swap.  The expected bytes are written out: the
+    high nibble holds agents 10-12."""
+    from gym_mapf_b200.envs.vec_env import GroupPolicy
+    starts = [[0, c] for c in range(10)] + [[1, 10], [0, 11], [2, 11]]
+    goals = [[2, c] for c in range(10)] + [[1, 0], [1, 1], [1, 2]]
+    spec = dict(rows=["." * 13] * 3, n_agents=13, starts=starts, goals=goals, fail_prob=0.0, r_clash=-1000.0,
+                r_goal=100.0, r_living=-1.0, soc=True)
+    eng = make_engine(spec)
+    assert (eng.L, eng.words, eng.moves_in_smem) == (39, 2, True)
+    dev = eng.torch_device
+    STAY, UP, RIGHT, DOWN, LEFT = range(5)
+    three, two = {10: RIGHT, 11: DOWN, 12: UP}, {11: DOWN, 12: UP}
+    swap = {4: RIGHT, 5: LEFT}
+    single = [(i,) for i in range(10)]
+    rest = [(i,) for i in range(10) if i not in (4, 5)]
+    cases = [(three, single + [(10,), (11,), (12,)], 0xBA),
+             (two, single + [(10,), (11,), (12,)], 0xCB),
+             ({**three, **swap}, single + [(10,), (11,), (12,)], 0x54),
+             (three, single + [(10, 11), (12,)], 0xCA),
+             (two, single + [(10, 11, 12)], 0xCB),
+             ({**three, **swap}, rest + [(4, 5), (10,), (11, 12)], 0xBA),
+             ({**three, **swap}, rest + [(4, 5), (10, 11, 12)], 0x54)]
+    for moves, groups, want in cases:
+        tables = [torch.full((eng.L ** len(g),), sum(moves.get(a, STAY) * 5 ** k for k, a in enumerate(g)),
+                             dtype=torch.int32, device=dev) for g in groups]
+        pairs = torch.empty(64, dtype=torch.uint8, device=dev)
+        ret, length, outcome = eng.evaluate_groups(GroupPolicy(groups, tables), 64, 10, conflicts=pairs)
+        assert bool((outcome == 1).all()) and bool((length == 1).all()), (moves, groups)
+        assert bool((pairs == want).all()), (moves, groups, pairs)
+
+
 # ---- 4. the same episodes from the C oracle and the host Philox stream ------------------------------------------------
 def test_groups_replayed_through_the_oracle(torch):
     spec, _ = G.load("rows_c2")
@@ -348,3 +382,49 @@ def test_find_conflicts_counts(mixed, torch):
     assert np.array_equal(found.counts.cpu().numpy(), want) and want.sum() > 0
     ev = vec.evaluate(gp, 20000, 100)
     assert all(torch.equal(a, b) for a, b in zip(ev, found.evaluation))
+
+
+# ---- 10. out-of-range entries through the C ABI are clamped ------------------------------------------------------------
+@pytest.mark.parametrize("name", sorted(PARTITIONS))
+def test_out_of_range_entries_are_clamped(name, mixed, torch):
+    """Entries >= 5**|g| or negative (as u32, above 5**|g| - 1) act as 5**|g| - 1.  GroupPolicy rejects such tables,
+    so only C callers reach the clamp."""
+    from gym_mapf_b200._native import POLICY_GROUPS
+    from test_gpu_evaluate import assert_clamped
+    eng, gp = mixed[name]
+    table = torch.cat(gp.tables).cpu().numpy()
+    size = np.concatenate([np.full(t.numel(), 5 ** len(g), np.int64) for g, t in zip(gp.groups, gp.tables)])
+    assert_clamped(torch, eng, lambda t: (POLICY_GROUPS, t, gp.group_of()), table, [size, -1, -(1 << 31)], size - 1,
+                   np.random.default_rng(5))
+
+
+# ---- 11. 2**30 episodes in one call: the env index crosses 2**32 -------------------------------------------------------
+@pytest.mark.timeout(300)
+def test_largest_call_crosses_2_32(mixed, torch):
+    """n_episodes = 2**30, the most one call takes, from episode_offset 2**32 - 2**29: episode 2**29 is env 2**32.
+    Every record is written, and episodes on both sides of the crossing and the last one are the oracle's."""
+    from test_gpu_evaluate import SENTINEL_RET
+    from test_gpu_kernel_matrix import SEED, assert_episodes, replay_episodes
+    free, _ = torch.cuda.mem_get_info()
+    if free < 24 << 30:
+        pytest.skip("needs 24 GB of free device memory for 15 GB of outputs, %.1f GB free: the device is shared"
+                    % (free / 2 ** 30))
+    eng, gp = mixed["rows_c2"]
+    E, T, gamma, step0, off = 1 << 30, 2, 0.95, (1 << 32) - 1, (1 << 32) - (1 << 29)
+    dev = eng.torch_device
+    ret = torch.full((E,), SENTINEL_RET, dtype=torch.int64, device=dev).view(torch.float64)
+    length = torch.full((E,), -1, dtype=torch.int32, device=dev)
+    outcome = torch.full((E,), 0xEE, dtype=torch.uint8, device=dev)
+    pairs = torch.full((E,), 0xEE, dtype=torch.uint8, device=dev)
+    eng.evaluate_groups(gp, E, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=off,
+                        out=(ret, length, outcome), conflicts=pairs)
+    assert bool((ret.view(torch.int64) != SENTINEL_RET).all())
+    assert bool(((length >= 1) & (length <= T)).all()) and bool((outcome <= 3).all())
+    assert bool(((pairs != 0xFF) == (outcome == 1)).all()) and bool((pairs != 0xEE).all())
+    sub = np.concatenate([np.arange(0, 300), np.arange((1 << 29) - 300, (1 << 29) + 300), np.arange(E - 300, E)])
+    ep = replay_episodes(eng, make_oracle(G.load("rows_c2")[0]), (gp.groups, [t.cpu().numpy() for t in gp.tables]),
+                         "groups", T, gamma, step0, off, sub)
+    got = tuple(x[torch.from_numpy(sub).to(dev)] for x in (ret, length, outcome, pairs))
+    every = np.arange(len(sub))
+    assert_episodes(got, ep, every, "E = 2**30")
+    assert np.array_equal(got[3].cpu().numpy(), ep.pair) and (ep.length == T).any()

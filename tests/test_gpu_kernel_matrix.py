@@ -32,14 +32,20 @@ terminal (every agent on its goal, or two agents on one cell).
 In every cell: step (Philox draws regenerated on the host, given uniforms, one and two envs per thread, compact
 results, auto-reset, shared-SM launches and the device-resident host step), rollout (all instantiated variants,
 auto-reset on and off, starts from s0, random, conflict-dense, goal and terminal states), evaluate (random and per-agent
-policies, joint-state policies where W = 1 and nS <= 2**26), the table path (transitions, checksum; table_range on a
-slab up to N = 6, where a slab of 5**N actions stays small), encode / decode / project and predecessors (up to N = 8:
-a state has up to 5**N predecessors).  Step indices cross 2**32 and env offsets are >= 2**32.
+policies, joint-state policies where W = 1 and nS <= 2**26, and group policies with their conflict bytes: singletons,
+equal to the per-agent kind on the same table; agents dealt round-robin into groups of up to four; {0, N-1} plus
+singletons; one group of every agent where the joint table fits, equal to the joint kind on the same table), the table
+path (transitions, checksum; table_range on a slab up to N = 6, where a slab of 5**N actions stays small), encode /
+decode / project and predecessors (up to N = 8: a state has up to 5**N predecessors).  Step indices cross 2**32 and env
+offsets are >= 2**32.
 
 Backup / greedy need one-word states and V of nS doubles, so they run on their own specs: staged N = 1..9 with small
 grids (N = 9 on nine cells: nS = 9**9, V = 3.1 GB, rows of permutation states, more batches than warps so a warp's
 head cache meets a second batch), unstaged N = 1, 2 on 5000 cells, and staged N = 10..13 on four cells, where L < N
-puts two agents on one cell in every state: every row there is terminal."""
+puts two agents on one cell in every state: every row there is terminal.  The staged N = 8 and 9 specs also run one
+group of every agent (tables of 9**8 and 9**9 entries): the device then takes digits 0..8 of a group's entry.  Digits
+9..12 would need a group of 10 or more agents with L >= 10 (10**10 entries); the host check of the digit arithmetic in
+test_groups_host.py covers them."""
 import math
 
 import numpy as np
@@ -282,6 +288,9 @@ def offset_view(torch, t, offset):
 
 
 SEED = 0x9E3779B97F4A7C15
+# seeds of the group-policy tables that give every partition of these cells a collision episode (the default, 1, does
+# elsewhere)
+GROUP_SEEDS = {(2, 1, True, 34): 250, (3, 1, True, 34): 2, (5, 1, False, 5000): 6}
 GPU_CELLS = [pytest.param(c, id=cell_id(c), marks=pytest.mark.gpu) for c in CELLS]
 
 
@@ -439,54 +448,181 @@ def test_rollout_matches_oracle(c, cells, torch):
 
 
 # ---- evaluate ---------------------------------------------------------------------------------------------------------
-def replay_episodes(cell, policy, kind, E, T, gamma, step0, off, sub):
-    eng, ora = cell.eng, cell.ora
+def gather(table, idx):
+    """table[idx] as int64 numpy, from a host array or a device tensor (tables too large to copy back)."""
+    if isinstance(table, np.ndarray):
+        return table[idx].astype(np.int64)
+    import torch
+    return table[torch.from_numpy(idx).to(table.device)].cpu().numpy().astype(np.int64)
+
+
+def group_actions(cells_, L, groups, tables):
+    """The joint action of a group policy: each group's entry at its local state sum_k cell[g_k] * L**k, split into
+    base-5 digits, agent g_k's at 5**k."""
+    actions = np.zeros(len(cells_), np.int64)
+    for g, table in zip(groups, tables):
+        entry = gather(table, sum(cells_[:, a] * L ** k for k, a in enumerate(g)))
+        for k, a in enumerate(g):
+            actions += entry // 5 ** k % 5 * 5 ** a
+    return actions
+
+
+def replay_episodes(eng, ora, policy, kind, T, gamma, step0, off, sub):
+    """Episodes `sub` of an evaluate call, stepped through the oracle with the host Philox draws.  kind "groups" takes
+    policy = (groups, tables) and also gives ep.pair, the conflict byte of every replayed episode (host_pair of the
+    oracle-decoded cells before and after a collision episode's last step, NO_CONFLICT for every other episode)."""
+    from test_gpu_groups import host_pair
     env = sub.astype(np.uint64) + np.uint64(off)
     s0_lo, s0_hi = split_s0(eng)
     lo, hi = np.full(len(sub), s0_lo), np.full(len(sub), s0_hi)
     ep = Episodes(len(sub), gamma)
+    ep.pair = np.full(len(sub), 0xFF, np.uint8)
+    if kind == "groups":
+        group_of = [next(gi for gi, g in enumerate(policy[0]) if a in g) for a in range(eng.n)]
     for t in range(T):
-        if kind == "agents":
+        if kind in ("agents", "groups"):
             cells_ = ora.decode(lo, hi).astype(np.int64)
+        if kind == "agents":
             actions = sum(policy[i][cells_[:, i]] * 5 ** i for i in range(eng.n))
+        elif kind == "groups":
+            actions = group_actions(cells_, eng.L, *policy)
         elif kind == "joint":
-            actions = policy[lo.astype(np.int64)].astype(np.int64)
+            actions = gather(policy, lo.astype(np.int64))
         else:
             actions = philox_actions(SEED, env, step0 + t, eng.nA)
         w = ora.step(lo, hi, actions, philox_uniforms(SEED, env, step0 + t, eng.n))
         k = np.where(w["collision"] == 1, 1, np.where(w["terminal"] == 1, 3, 2)).astype(np.uint8)
+        if kind == "groups":
+            hit = np.flatnonzero(ep.active & (w["done"] == 1) & (w["collision"] == 1))
+            nxt = ora.decode(w["next_lo"][hit], w["next_hi"][hit])
+            for h, row in zip(hit, nxt):
+                ep.pair[h] = host_pair(cells_[h], row, group_of)
         if not ep.add(t, w["reward"], w["done"].astype(bool), k):
             break
         lo, hi = w["next_lo"], w["next_hi"]
     return ep
 
 
+def cell_partitions(n, L, joint):
+    """The agent partitions a cell's group policies use: singletons; agents dealt round-robin into groups of at most
+    k <= 4 agents with L**k <= 2**25 entries (non-contiguous groups such as (0, 4, 8, 12) at 13 agents, so the whole
+    N x N multiplier matrix is used); {0, n-1} plus singletons; one group of every agent where a joint table fits.
+    Duplicates (small n) are dropped."""
+    k = max(k for k in range(1, min(n, 4) + 1) if L ** k <= 1 << 25)
+    m = -(-n // k)
+    out = [tuple((i,) for i in range(n)), tuple(tuple(range(g, n, m)) for g in range(m))]
+    if n >= 2 and L ** 2 <= 1 << 25:
+        out.append(((0, n - 1),) + tuple((i,) for i in range(1, n - 1)))
+    if joint:
+        out.append((tuple(range(n)),))
+    return list(dict.fromkeys(out))
+
+
+def assert_episodes(got, ep, sub, what):
+    assert np.array_equal(u64(got[0])[sub], ep.G.view(np.uint64)), what
+    assert np.array_equal(got[1].cpu().numpy()[sub], ep.length), what
+    assert np.array_equal(got[2].cpu().numpy()[sub], ep.outcome), what
+
+
 @pytest.mark.timeout(300)
 @pytest.mark.parametrize("c", GPU_CELLS)
 def test_evaluate_matches_oracle(c, cells, torch):
+    from gym_mapf_b200.envs.vec_env import GroupPolicy
     cell = cells(c)
-    eng = cell.eng
+    eng, ora, n, L = cell.eng, cell.ora, cell.n, cell.L
     dev = eng.torch_device
     rng = np.random.default_rng(cell.L + 5 * cell.n)
     policies = [("random", None, None), ("agents", None, rng.integers(0, 5, (eng.n, eng.L)))]
-    if eng.words == 1 and eng.nS <= 1 << 26:
+    joint = eng.words == 1 and eng.nS <= 1 << 26
+    if joint:
         policies.append(("joint", None, rng.integers(0, eng.nA, int(eng.nS))))
     step0, off, gamma = (1 << 32) - 7, (1 << 32) + 3, 0.95
+    cases = ((1500, 50), (257, 1))
+    results = {}
     for kind, _, table in policies:
         pol = None if table is None else torch.from_numpy(table.astype(np.int32)).to(dev)
-        for E, T in ((1500, 50), (257, 1)):
+        for E, T in cases:
             got = eng.evaluate(pol, E, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=off)
             sub = np.arange(E) if E < 1000 else np.arange(0, E, 3)
-            ep = replay_episodes(cell, table, kind, E, T, gamma, step0, off, sub)
-            assert np.array_equal(u64(got[0])[sub], ep.G.view(np.uint64)), (kind, E, T)
-            assert np.array_equal(got[1].cpu().numpy()[sub], ep.length), (kind, E, T)
-            assert np.array_equal(got[2].cpu().numpy()[sub], ep.outcome), (kind, E, T)
+            ep = replay_episodes(eng, ora, table, kind, T, gamma, step0, off, sub)
+            assert_episodes(got, ep, sub, (kind, E, T))
+            results[kind, E] = got
+    # group policies: singletons act as AGENTS on the same table, one group of every agent as JOINT on the same table
+    grng = np.random.default_rng(cell.L + 7 * cell.n + GROUP_SEEDS.get(c, 1))
+    for groups in cell_partitions(n, L, joint):
+        if len(groups) == 1 and joint:
+            tables = [policies[2][2].astype(np.int32)]
+        else:
+            tables = [grng.integers(0, 5 ** len(g), L ** len(g), dtype=np.int32) for g in groups]
+        gp = GroupPolicy(groups, [torch.from_numpy(t).to(dev) for t in tables])
+        for E, T in cases:
+            what = (groups, E, T)
+            pairs = torch.full((E,), 0xEE, dtype=torch.uint8, device=dev)
+            got = eng.evaluate_groups(gp, E, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=off,
+                                      conflicts=pairs)
+            plain = eng.evaluate_groups(gp, E, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=off)
+            assert all(torch.equal(a, b) for a, b in zip(got, plain)), what  # conflicts=None changes nothing else
+            if len(groups) == n:
+                same = eng.evaluate(torch.stack(gp.tables), E, T, gamma=gamma, seed=SEED, step_index=step0,
+                                    episode_offset=off)
+                assert all(torch.equal(a, b) for a, b in zip(got, same)), what
+            elif len(groups) == 1 and joint:
+                assert all(torch.equal(a, b) for a, b in zip(got, results["joint", E])), what
+            sub = np.arange(E) if E < 1000 else np.arange(0, E, 3)
+            ep = replay_episodes(eng, ora, (groups, tables), "groups", T, gamma, step0, off, sub)
+            assert_episodes(got, ep, sub, what)
+            assert np.array_equal(pairs.cpu().numpy()[sub], ep.pair), what
+            if n >= 2 and T > 1:  # attribution is tested only where something collides
+                assert (ep.outcome == 1).any(), what
     for terminal in ("goal", "shared"):
         tw = cells(c, terminal)
         if tw.n == 1 and terminal == "shared":
             continue
         ret, length, outcome = tw.eng.evaluate(None, 300, 20, gamma=gamma, seed=SEED)
         assert np.all(u64(ret) == 0) and bool((length == 1).all()) and bool((outcome == 3).all())
+        gp = GroupPolicy([(i,) for i in range(n)], [torch.from_numpy(t).to(dev) for t in
+                                                     grng.integers(0, 5, (n, L), dtype=np.int32)])
+        pairs = torch.zeros(300, dtype=torch.uint8, device=dev)
+        ret, length, outcome = tw.eng.evaluate_groups(gp, 300, 20, gamma=gamma, seed=SEED, conflicts=pairs)
+        assert np.all(u64(ret) == 0) and bool((length == 1).all()) and bool((outcome == 3).all())
+        assert bool((pairs == 0xFF).all())
+
+
+@pytest.mark.timeout(300)
+@pytest.mark.parametrize("c", [pytest.param(c, id=cell_id(c), marks=pytest.mark.gpu) for c in BACKUP_CELLS
+                               if c[0] in (8, 9)])
+def test_one_group_takes_every_digit(c, cells, torch):
+    """One group of all 8 or 9 agents on nine cells: entries of 9**n states, so the device takes digits 0..8 of an entry
+    (positions 9..12 are covered by the host check of the arithmetic in test_groups_host.py: a group of 10 agents needs
+    L >= 10 for a non-terminal start, and 10**10 entries).  Against JOINT on the same table, and against the oracle
+    with conflict bytes.  Each digit is STAY with probability 3/4: with uniform digits nearly every agent moves on a
+    full grid, and nearly every episode would end on its first step, having read the entry of s0 only.  (At 9 agents
+    the grid is full and fail_prob is 0: every episode is that one step, and its conflict byte names the movers.)"""
+    from gym_mapf_b200.envs.vec_env import GroupPolicy
+    cell = cells(c)
+    eng, ora, n = cell.eng, cell.ora, cell.n
+    dev = eng.torch_device
+    nS = int(eng.nS)
+    assert eng.words == 1 and nS == 9 ** n
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(77 + n)
+    table = torch.zeros(nS, dtype=torch.int32, device=dev)
+    for k in range(n):
+        d = torch.randint(1, 5, (nS,), dtype=torch.int32, device=dev, generator=gen)
+        d.masked_fill_(torch.rand(nS, device=dev, generator=gen) < 0.75, 0)
+        table += d * 5 ** k
+        del d
+    gp = GroupPolicy([tuple(range(n))], [table])
+    E, T, gamma, step0, off = 100003, 40, 0.95, (1 << 32) - 3, (1 << 32) + 11
+    pairs = torch.full((E,), 0xEE, dtype=torch.uint8, device=dev)
+    got = eng.evaluate_groups(gp, E, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=off, conflicts=pairs)
+    want = eng.evaluate(table, E, T, gamma=gamma, seed=SEED, step_index=step0, episode_offset=off)
+    assert all(torch.equal(a, b) for a, b in zip(got, want))
+    sub = np.concatenate([np.arange(0, E, 331), [E - 1]])
+    ep = replay_episodes(eng, ora, (gp.groups, [table]), "groups", T, gamma, step0, off, sub)
+    assert_episodes(got, ep, sub, c)
+    assert np.array_equal(pairs.cpu().numpy()[sub], ep.pair)
+    assert (ep.outcome == 1).any() and (n == 9 or (ep.length > 1).any())
 
 
 # ---- table path -------------------------------------------------------------------------------------------------------
