@@ -1710,6 +1710,11 @@ extern "C" int mapf_group_step(const mapf_group *g, const void *states, const in
                                uint64_t seed, uint64_t step_index, int64_t env_offset, uint32_t options, void *next_states,
                                double *reward, double *prob, uint8_t *done, uint8_t *collision, void *stream) {
     if (!g) return fail(MAPF_ERR_INVALID, "mapf_group_step: NULL group");
+    // k_step_group writes the default result layout and takes no launch-shape option: a compact-sized reward buffer
+    // would be overrun by its 8-byte stores
+    if (options & ~(uint32_t)MAPF_OPT_AUTO_RESET)
+        return fail(MAPF_ERR_UNSUPPORTED, "mapf_group_step: options = %u, only MAPF_OPT_AUTO_RESET is supported (step "
+                                          "with mapf_step for the compact layout)", options);
     if (g->B == 0) return MAPF_OK;
     if (!states || !actions || !next_states || !reward || !prob || !done || !collision ||
         states_misaligned(g->words, states) || states_misaligned(g->words, next_states))

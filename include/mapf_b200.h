@@ -327,8 +327,10 @@ typedef struct mapf_group mapf_group;
 int mapf_group_create(mapf_ctx *const *ctxs, const int64_t *env_counts, int32_t n_specs, mapf_group **out);
 void mapf_group_destroy(mapf_group *group);
 int64_t mapf_group_size(const mapf_group *group);
-/* MapfEnv.step (mapf_env.py:237-266) for every env of the group in ONE launch; buffers and semantics as mapf_step,
- * indexed by the env's position in the concatenated batch (which also keys its Philox stream). */
+/* MapfEnv.step (mapf_env.py:237-266) for every env of the group in ONE launch; buffers and semantics as mapf_step
+ * without options, indexed by the env's position in the concatenated batch (which also keys its Philox stream).
+ * The one option bit it takes is MAPF_OPT_AUTO_RESET; any other bit (MAPF_OPT_COMPACT, MAPF_OPT_SHARE_SM) is
+ * MAPF_ERR_UNSUPPORTED and launches nothing -- step with mapf_step for the compact layout. */
 int mapf_group_step(const mapf_group *group, const void *states, const int32_t *actions, const double *uniforms,
                     uint64_t seed, uint64_t step_index, int64_t env_offset, uint32_t options, void *next_states,
                     double *reward, double *prob, uint8_t *done, uint8_t *collision, void *stream);
