@@ -17,7 +17,9 @@ OPT_AUTO_RESET = 1
 OPT_SHARE_SM = 2
 OPT_COMPACT = 4
 FLAG_DONE, FLAG_COLLISION = 1, 2
-POLICY_RANDOM, POLICY_JOINT, POLICY_AGENTS, POLICY_GROUPS = 0, 1, 2, 3
+POLICY_RANDOM, POLICY_JOINT, POLICY_AGENTS, POLICY_GROUPS, POLICY_TABLE = 0, 1, 2, 3, 4
+VTABLE_EMPTY = (1 << 64) - 1     # key of a free value-table slot
+VTABLE_REFUSED = 1 << 63         # bit of a value table's count word: a store was dropped for lack of room
 NO_CONFLICT = 0xFF  # conflict byte of an episode that did not end in a collision
 EPISODE_TIMEOUT, EPISODE_COLLISION, EPISODE_GOAL, EPISODE_TERMINAL_START = 0, 1, 2, 3
 
@@ -26,6 +28,7 @@ EXPORTS = ["mapf_ctx_create", "mapf_ctx_destroy", "mapf_ctx_info", "mapf_ctx_mov
            "mapf_count_scan_range", "mapf_expand",
            "mapf_count_range", "mapf_expand_range", "mapf_checksum", "mapf_step", "mapf_rollout", "mapf_step_host", "mapf_step_host_resident",
            "mapf_evaluate_scratch_bytes", "mapf_evaluate", "mapf_evaluate_groups",
+           "mapf_rtdp_backup", "mapf_vtable_store", "mapf_vtable_lookup", "mapf_evaluate_table",
            "mapf_backup", "mapf_backup_range", "mapf_greedy", "mapf_greedy_bcast", "mapf_count_predecessors", "mapf_predecessors",
            "mapf_projected_words", "mapf_project_states", "mapf_parse_map_text", "mapf_parse_scen_text", "mapf_ctx_create_from_text", "mapf_ctx_grid",
            "mapf_group_create", "mapf_group_destroy", "mapf_group_size", "mapf_group_step", "mapf_last_error",
@@ -44,6 +47,11 @@ class MapfInfo(C.Structure):
                 ("moves_in_smem", C.c_int32), ("n_actions", C.c_int64), ("n_states", C.c_uint64 * 2),
                 ("start_state", C.c_uint64 * 2), ("goal_state", C.c_uint64 * 2), ("max_row_len", C.c_int64),
                 ("device", C.c_int32), ("sm_count", C.c_int32)]
+
+
+class MapfVtable(C.Structure):
+    _fields_ = [("keys", C.c_void_p), ("values", C.c_void_p), ("actions", C.c_void_p), ("capacity", C.c_int64),
+                ("count", C.c_void_p)]
 
 
 class NativeError(RuntimeError):
@@ -104,6 +112,12 @@ def lib():
         L.mapf_evaluate_scratch_bytes.restype = i64
         L.mapf_evaluate.argtypes = [vp, i32, vp, i64, i64, i64, C.c_double, u64, u64, i64, vp, vp, vp, vp, vp]
         L.mapf_evaluate_groups.argtypes = [vp, vp, vp, i64, i64, i64, C.c_double, u64, u64, i64, vp, vp, vp, vp, vp, vp]
+        vtp = C.POINTER(MapfVtable)
+        L.mapf_rtdp_backup.argtypes = [vp, vp, i64, vp, vp, i64, vtp, C.c_double, vp, vp, vp]
+        L.mapf_vtable_store.argtypes = [vp, vp, i64, vp, vp, vtp, vp]
+        L.mapf_vtable_lookup.argtypes = [vp, vp, i64, vp, vp, i64, vtp, vp, vp, vp]
+        L.mapf_evaluate_table.argtypes = [vp, vtp, vp, vp, i64, i64, i64, C.c_double, u64, u64, i64, vp, vp, vp, vp, vp,
+                                          vp]
         L.mapf_backup.argtypes = [vp, vp, vp, i64, vp, i64, C.c_double, vp, vp]
         L.mapf_backup_range.argtypes = [vp, C.POINTER(u64 * 2), i64, vp, i64, C.c_double, vp, vp]
         L.mapf_greedy.argtypes = [vp, vp, i64, vp, vp, vp]
@@ -478,10 +492,13 @@ class Engine:
         steps, in one launch (mapf_evaluate).  Episode e draws what env `episode_offset + e` of `step` draws from
         `step_index` on.  `policy`: None (uniformly random joint actions, as `rollout` draws them), an int32[nS] tensor
         of joint actions indexed by the joint state, or an integer [n_agents, L] tensor of per-agent actions indexed by
-        the agent's cell, or a `GroupPolicy` (see `evaluate_groups`).  Returns (returns f64[E], lengths i32[E],
+        the agent's cell, a `GroupPolicy` (see `evaluate_groups`) or a `TablePolicy` (see `evaluate_table`).  Returns (returns f64[E], lengths i32[E],
         outcomes u8[E]) with outcomes EPISODE_*."""
         import torch
-        from .envs.vec_env import GroupPolicy
+        from .envs.vec_env import GroupPolicy, TablePolicy
+        if isinstance(policy, TablePolicy):
+            return self.evaluate_table(policy, n_episodes, max_steps, gamma=gamma, seed=seed, step_index=step_index,
+                                       episode_offset=episode_offset, out=out)
         if isinstance(policy, GroupPolicy):
             return self.evaluate_groups(policy, n_episodes, max_steps, gamma=gamma, seed=seed, step_index=step_index,
                                         episode_offset=episode_offset, out=out)
@@ -555,6 +572,95 @@ class Engine:
                                          float(gamma), int(seed), int(step_index), int(episode_offset), _ptr(scratch),
                                          _ptr(ret), _ptr(length), _ptr(outcome), _ptr(conflicts), self._stream()))
         return out
+
+    def evaluate_table(self, policy, n_episodes, max_steps, gamma=1.0, seed=0, step_index=0, episode_offset=0, out=None,
+                       conflicts=None):
+        """`evaluate_groups` for a `TablePolicy` (mapf_evaluate_table): in a state that is a key of the policy's value
+        table an episode takes the action stored with it, anywhere else the fallback GroupPolicy's action.  Same draws,
+        outputs and `conflicts` as `evaluate_groups`."""
+        import torch
+        E = int(n_episodes)
+        if E < 0:
+            raise ValueError("n_episodes must be >= 0 (got %d)" % E)
+        if policy.table.engine is not self:
+            raise ValueError("the TablePolicy's value table belongs to another env")
+        group_of, tables = self._group_args(policy.fallback.groups, policy.fallback.tables, "fallback GroupPolicy")
+        dev = self.torch_device
+        if out is None:
+            out = (torch.empty(E, dtype=torch.float64, device=dev), torch.empty(E, dtype=torch.int32, device=dev),
+                   torch.empty(E, dtype=torch.uint8, device=dev))
+        ret, length, outcome = out
+        self._check_tensor("returns", ret, torch.float64, (E,))
+        self._check_tensor("lengths", length, torch.int32, (E,))
+        self._check_tensor("outcomes", outcome, torch.uint8, (E,))
+        if conflicts is not None:
+            self._check_tensor("conflicts", conflicts, torch.uint8, (E,))
+        scratch = torch.empty((int(lib().mapf_evaluate_scratch_bytes()) + 7) // 8, dtype=torch.int64, device=dev)
+        check(lib().mapf_evaluate_table(self._h, C.byref(policy.table.c_struct()), group_of, _ptr(tables),
+                                        tables.numel(), E, int(max_steps), float(gamma), int(seed), int(step_index),
+                                        int(episode_offset), _ptr(scratch), _ptr(ret), _ptr(length), _ptr(outcome),
+                                        _ptr(conflicts), self._stream()))
+        return out
+
+    # ---- RTDP over a value table (one-word states) -------------------------------------------------------------
+    def _group_args(self, groups, tables, what):
+        """(group_of as a C array, the per-group tables concatenated) of a GroupPolicy's or GroupValues' tensors."""
+        import torch
+        n = sum(len(g) for g in groups)
+        if n != self.n or any(t.numel() != self.L ** len(g) for g, t in zip(groups, tables)) or \
+                tables[0].device != self.torch_device:
+            raise ValueError("the %s is for %d agents with tables of %s entries on %s; this env has %d agents on %d cells "
+                             "on %s" % (what, n, [t.numel() for t in tables], tables[0].device, self.n, self.L,
+                                        self.torch_device))
+        group_of = [0] * n
+        for gid, g in enumerate(groups):
+            for a in g:
+                group_of[a] = gid
+        flat = tables[0].contiguous() if len(tables) == 1 else torch.cat(tables)
+        return (C.c_int32 * n)(*group_of), flat
+
+    def _check_keys(self, states):
+        import torch
+        if self.words != 1:
+            raise ValueError("value tables are keyed by one-word states; this env's states take two words")
+        self._check_tensor("states", states, torch.int64, (states.shape[0],))
+
+    def rtdp_backup(self, states, heuristic, table, gamma):
+        """(v f64[B], a i32[B]) (mapf_rtdp_backup): v[b] = max over actions of the Bellman backup of states[b], every
+        successor valued by `table` when it is a key and by `heuristic` (GroupValues) otherwise; a[b] = the first
+        action attaining it.  `table` is only read."""
+        import torch
+        self._check_keys(states)
+        B = states.shape[0]
+        group_of, hv = self._group_args(heuristic.groups, heuristic.values, "GroupValues")
+        v = torch.empty(B, dtype=torch.float64, device=self.torch_device)
+        a = torch.empty(B, dtype=torch.int32, device=self.torch_device)
+        check(lib().mapf_rtdp_backup(self._h, _ptr(states), B, group_of, _ptr(hv), hv.numel(),
+                                     C.byref(table.c_struct()), float(gamma), _ptr(v), _ptr(a), self._stream()))
+        return v, a
+
+    def vtable_store(self, states, v, a, table):
+        """Stores (states[b], v[b], a[b]) in `table`, overwriting present keys; the states must be distinct
+        (mapf_vtable_store)."""
+        import torch
+        self._check_keys(states)
+        B = states.shape[0]
+        self._check_tensor("v", v, torch.float64, (B,))
+        self._check_tensor("a", a, torch.int32, (B,))
+        check(lib().mapf_vtable_store(self._h, _ptr(states), B, _ptr(v), _ptr(a), C.byref(table.c_struct()),
+                                      self._stream()))
+
+    def vtable_lookup(self, states, heuristic, table):
+        """(value_of(states) f64[B], the stored action or -1 i32[B]) (mapf_vtable_lookup)."""
+        import torch
+        self._check_keys(states)
+        B = states.shape[0]
+        group_of, hv = self._group_args(heuristic.groups, heuristic.values, "GroupValues")
+        v = torch.empty(B, dtype=torch.float64, device=self.torch_device)
+        a = torch.empty(B, dtype=torch.int32, device=self.torch_device)
+        check(lib().mapf_vtable_lookup(self._h, _ptr(states), B, group_of, _ptr(hv), hv.numel(),
+                                       C.byref(table.c_struct()), _ptr(v), _ptr(a), self._stream()))
+        return v, a
 
     # ---- rows next to the hot path (SURVEY.md 8f) ----------------------------------------------------------
     def backup(self, states, actions, V, gamma, out=None):

@@ -70,6 +70,7 @@ struct mapf_ctx {
     int grid_step1 = 0, grid_step2 = 0, grid_step_tape = 0, grid_rollout = 0, grid_rollout2 = 0, grid_rollout_tape = 0;
     int grid_expand = 0, grid_expand_range = 0, grid_plain = 0, grid_backup = 0, grid_backup_range = 0;
     int grid_evaluate[4] = {0, 0, 0, 0};  // k_evaluate / k_evaluate_groups by policy kind
+    int grid_rtdp = 0, grid_evaluate_table = 0;
     KernelSet ks;
     u32 pat_triple[MAPF_MAX_PATTERNS];  // merge patterns (see PatternList)
     int n_patterns = 0;
@@ -555,7 +556,9 @@ extern "C" int mapf_ctx_create(const mapf_spec *spec, int device, mapf_ctx **out
         {ctx->ks.evaluate[MAPF_POLICY_RANDOM], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_RANDOM]},
         {ctx->ks.evaluate[MAPF_POLICY_JOINT], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_JOINT]},
         {ctx->ks.evaluate[MAPF_POLICY_AGENTS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_AGENTS]},
-        {ctx->ks.evaluate[MAPF_POLICY_GROUPS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_GROUPS]}};
+        {ctx->ks.evaluate[MAPF_POLICY_GROUPS], ctx->smem_base, &ctx->grid_evaluate[MAPF_POLICY_GROUPS]},
+        {ctx->ks.rtdp_backup, ctx->smem_backup, &ctx->grid_rtdp},
+        {ctx->ks.evaluate_table, ctx->smem_base, &ctx->grid_evaluate_table}};
     for (auto &pl : plan) {
         if (!pl.fn) continue;  // two-word states have no backup kernels; wide step CTAs have no EPT = 2 k_step
         if (pl.smem > smem_limit) {
@@ -1206,6 +1209,51 @@ extern "C" int mapf_evaluate(const mapf_ctx *ctx, int32_t policy_kind, const voi
     return MAPF_OK;
 }
 
+// The agent groups of a group_of / table-length pair (mapf_evaluate_groups' rules), as the per-agent GroupLayout of the
+// kernels; *heads gets bit i set when agent i is the first agent of its group.  `who` names the entry point in errors.
+static int group_layout(const mapf_ctx *ctx, const char *who, const int32_t *group_of, int64_t tables_len, GroupLayout *gl,
+                        u32 *heads) {
+    const int n = ctx->sp.n;
+    const u64 L = (u64)ctx->sp.L;
+    int size[MAPF_MAXN] = {0}, pos[MAPF_MAXN], n_groups = 0;
+    for (int i = 0; i < n; ++i) {
+        const int g = group_of[i];
+        if (g < 0 || g > n_groups)  // canonical: a new group takes the next id
+            return fail(MAPF_ERR_INVALID, "%s: group_of[%d] = %d, must be in [0, %d]", who, i, g, n_groups);
+        if (g == n_groups) ++n_groups;
+        pos[i] = size[g]++;
+    }
+    // table g holds L**size[g] entries at first[g]; every partial sum stays below 2**63
+    u64 first[MAPF_MAXN], total = 0, powL[MAPF_MAXN + 1];
+    powL[0] = 1;
+    for (int k = 1; k <= n; ++k) powL[k] = powL[k - 1] > (u64)INT64_MAX / L ? (u64)INT64_MAX : powL[k - 1] * L;
+    for (int g = 0; g < n_groups; ++g) {
+        if (powL[size[g]] == (u64)INT64_MAX || total > (u64)INT64_MAX - powL[size[g]])
+            return fail(MAPF_ERR_INVALID, "%s: the tables have more than 2**63 - 1 entries", who);
+        first[g] = total;
+        total += powL[size[g]];
+    }
+    if (tables_len < 0 || (u64)tables_len != total)
+        return fail(MAPF_ERR_INVALID, "%s: the groups' tables have %llu entries (tables_len = %lld)", who,
+                    (unsigned long long)total, (long long)tables_len);
+    memset(gl, 0, sizeof(*gl));
+    *heads = 0;
+    for (int i = 0; i < n; ++i) {
+        const int g = group_of[i];
+        for (int j = 0; j < n; ++j) gl->mul[i][j] = group_of[j] == g ? powL[pos[j]] : 0;
+        gl->off[i] = first[g];
+        u64 d = 5;  // 5**(pos[i] + 1) <= 5**13 < 2**32: not a divisor of 2**64, so the ceiling is floor + 1
+        for (int k = 0; k < pos[i]; ++k) d *= 5;
+        gl->frac[i] = ~0ull / d + 1;
+        u32 a = 1;
+        for (int k = 0; k < size[g]; ++k) a *= 5u;
+        gl->amax[i] = a - 1u;
+        gl->group[i] = (u32)g;
+        if (pos[i] == 0) *heads |= 1u << i;
+    }
+    return MAPF_OK;
+}
+
 extern "C" int mapf_evaluate_groups(const mapf_ctx *ctx, const int32_t *group_of, const int32_t *tables,
                                     int64_t tables_len, int64_t n_episodes, int64_t max_steps, double gamma,
                                     uint64_t seed, uint64_t step_index0, int64_t episode_offset, void *scratch,
@@ -1216,48 +1264,15 @@ extern "C" int mapf_evaluate_groups(const mapf_ctx *ctx, const int32_t *group_of
         return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: max_steps = %lld, must be in [1, 2**31)", (long long)max_steps);
     if (n_episodes > MAPF_LAUNCH_MAX_ENVS)
         return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: at most 2**30 episodes per call");
-    const int n = ctx->sp.n;
-    const u64 L = (u64)ctx->sp.L;
-    int size[MAPF_MAXN] = {0}, pos[MAPF_MAXN], n_groups = 0;
-    for (int i = 0; i < n; ++i) {
-        const int g = group_of[i];
-        if (g < 0 || g > n_groups)  // canonical: a new group takes the next id
-            return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: group_of[%d] = %d, must be in [0, %d]", i, g, n_groups);
-        if (g == n_groups) ++n_groups;
-        pos[i] = size[g]++;
-    }
-    // table g holds L**size[g] entries at first[g]; every partial sum stays below 2**63
-    u64 first[MAPF_MAXN], total = 0, powL[MAPF_MAXN + 1];
-    powL[0] = 1;
-    for (int k = 1; k <= n; ++k) powL[k] = powL[k - 1] > (u64)INT64_MAX / L ? (u64)INT64_MAX : powL[k - 1] * L;
-    for (int g = 0; g < n_groups; ++g) {
-        if (powL[size[g]] == (u64)INT64_MAX || total > (u64)INT64_MAX - powL[size[g]])
-            return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: the tables have more than 2**63 - 1 entries");
-        first[g] = total;
-        total += powL[size[g]];
-    }
-    if (tables_len < 0 || (u64)tables_len != total)
-        return fail(MAPF_ERR_INVALID, "mapf_evaluate_groups: the groups' tables have %llu entries (tables_len = %lld)",
-                    (unsigned long long)total, (long long)tables_len);
+    GroupLayout gl;
+    u32 heads;
+    const int rc = group_layout(ctx, "mapf_evaluate_groups", group_of, tables_len, &gl, &heads);
+    if (rc) return rc;
     if (!ctx->philox_ok)
         return fail(MAPF_ERR_UNSUPPORTED, "device-side sampling needs slip probabilities that add up to 1");
     if (n_episodes == 0) return MAPF_OK;
     const void *fn = ctx->ks.evaluate[MAPF_POLICY_GROUPS];
     if (!fn) return fail(MAPF_ERR_UNSUPPORTED, "mapf_evaluate_groups: no kernel");
-    GroupLayout gl;
-    memset(&gl, 0, sizeof(gl));
-    for (int i = 0; i < n; ++i) {
-        const int g = group_of[i];
-        for (int j = 0; j < n; ++j) gl.mul[i][j] = group_of[j] == g ? powL[pos[j]] : 0;
-        gl.off[i] = first[g];
-        u64 d = 5;  // 5**(pos[i] + 1) <= 5**13 < 2**32: not a divisor of 2**64, so the ceiling is floor + 1
-        for (int k = 0; k < pos[i]; ++k) d *= 5;
-        gl.frac[i] = ~0ull / d + 1;
-        u32 a = 1;
-        for (int k = 0; k < size[g]; ++k) a *= 5u;
-        gl.amax[i] = a - 1u;
-        gl.group[i] = (u32)g;
-    }
     DeviceGuard dg(ctx->device);
     CUDA_TRY(cudaMemsetAsync(scratch, 0, sizeof(u32), (cudaStream_t)stream));
     DevSpec sp = ctx->sp;
@@ -1267,6 +1282,122 @@ extern "C" int mapf_evaluate_groups(const mapf_ctx *ctx, const int32_t *group_of
     void *args[] = {&sp, &keys, &tables, &gl, &E, &T, &gamma, &st, &e0, &scratch, &ret, &length, &outcome, &conflict};
     LAUNCH(fn, grid_for(n_episodes, ctx->threads, ctx->grid_evaluate[MAPF_POLICY_GROUPS]), ctx->threads, ctx->smem_base,
            stream, args);
+    return MAPF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// RTDP: value table, its Bellman update and its policy
+// ---------------------------------------------------------------------------------------------------------------
+static_assert(MAPF_VTABLE_EMPTY == VT_EMPTY && MAPF_VTABLE_REFUSED == VT_REFUSED, "value-table constants");
+
+// The checks every value-table call makes: a one-word context and a well-formed table.
+static int vtable_view(const mapf_ctx *ctx, const char *who, const mapf_vtable *t, VTableView *vt) {
+    if (!ctx || !t || !t->keys || !t->values || !t->actions || !t->count)
+        return fail(MAPF_ERR_INVALID, "%s: bad argument", who);
+    if (t->capacity < 64 || (t->capacity & (t->capacity - 1)) != 0)
+        return fail(MAPF_ERR_INVALID, "%s: capacity = %lld, must be a power of two >= 64", who, (long long)t->capacity);
+    if (ctx->sp.words != 1)
+        return fail(MAPF_ERR_UNSUPPORTED, "%s: the value table is keyed by one-word states; L**n = %d**%d needs two", who,
+                    ctx->sp.L, ctx->sp.n);
+    vt->keys = (const u64 *)t->keys;
+    vt->values = t->values;
+    vt->actions = t->actions;
+    vt->mask = (u64)t->capacity - 1;
+    return MAPF_OK;
+}
+
+static inline bool bad_states(int64_t B, const void *states) {
+    return B < 0 || (B > 0 && (!states || ((uintptr_t)states & 7u) != 0));
+}
+
+extern "C" int mapf_rtdp_backup(const mapf_ctx *ctx, const void *states, int64_t B, const int32_t *group_of,
+                                const double *hvalues, int64_t hvalues_len, const mapf_vtable *table, double gamma,
+                                double *v_out, int32_t *a_out, void *stream) {
+    VTableView vt = {};
+    int rc = vtable_view(ctx, "mapf_rtdp_backup", table, &vt);
+    if (rc) return rc;
+    if (bad_states(B, states) || !group_of || !hvalues || (B > 0 && (!v_out || !a_out)))
+        return fail(MAPF_ERR_INVALID, "mapf_rtdp_backup: bad argument");
+    GroupLayout gl;
+    u32 heads;
+    rc = group_layout(ctx, "mapf_rtdp_backup", group_of, hvalues_len, &gl, &heads);
+    if (rc) return rc;
+    if (B == 0) return MAPF_OK;
+    DeviceGuard g(ctx->device);
+    DevSpec sp = ctx->sp;
+    // a warp takes G = max(1, 32 / nA) states per pass
+    u32 G = ctx->sp.nA >= 32 ? 1u : (u32)(32 / ctx->sp.nA), rcp_nA = G > 1 ? (u32)(0xffffffffu / ctx->sp.nA + 1) : 0u;
+    void *args[] = {&sp, &states, &B, &gl, &hvalues, &heads, &vt, &gamma, &G, &rcp_nA, &v_out, &a_out};
+    const int64_t lanes = (B + G - 1) / G * 32;
+    LAUNCH(ctx->ks.rtdp_backup, grid_for(lanes, ctx->threads, ctx->grid_rtdp), ctx->threads, ctx->smem_backup, stream,
+           args);
+    return MAPF_OK;
+}
+
+extern "C" int mapf_vtable_store(const mapf_ctx *ctx, const void *states, int64_t B, const double *v, const int32_t *a,
+                                 const mapf_vtable *table, void *stream) {
+    VTableView vt = {};
+    int rc = vtable_view(ctx, "mapf_vtable_store", table, &vt);
+    if (rc) return rc;
+    if (bad_states(B, states) || (B > 0 && (!v || !a))) return fail(MAPF_ERR_INVALID, "mapf_vtable_store: bad argument");
+    if (B == 0) return MAPF_OK;
+    DeviceGuard g(ctx->device);
+    k_vtable_store<<<grid_for(B, 256, ctx->grid_plain), 256, 0, (cudaStream_t)stream>>>(
+        (const u64 *)states, B, v, a, (u64 *)table->keys, table->values, table->actions, vt.mask, (u64 *)table->count);
+    CUDA_TRY(cudaGetLastError());
+    return MAPF_OK;
+}
+
+extern "C" int mapf_vtable_lookup(const mapf_ctx *ctx, const void *states, int64_t B, const int32_t *group_of,
+                                  const double *hvalues, int64_t hvalues_len, const mapf_vtable *table, double *v_out,
+                                  int32_t *a_out, void *stream) {
+    VTableView vt = {};
+    int rc = vtable_view(ctx, "mapf_vtable_lookup", table, &vt);
+    if (rc) return rc;
+    if (bad_states(B, states) || !group_of || !hvalues || (B > 0 && (!v_out || !a_out)))
+        return fail(MAPF_ERR_INVALID, "mapf_vtable_lookup: bad argument");
+    GroupLayout gl;
+    u32 heads;
+    rc = group_layout(ctx, "mapf_vtable_lookup", group_of, hvalues_len, &gl, &heads);
+    if (rc) return rc;
+    if (B == 0) return MAPF_OK;
+    DeviceGuard g(ctx->device);
+    DevSpec sp = ctx->sp;
+    void *args[] = {&sp, &states, &B, &gl, &hvalues, &heads, &vt, &v_out, &a_out};
+    LAUNCH(ctx->ks.vtable_lookup, grid_for(B, 256, ctx->grid_plain), 256, 0, stream, args);
+    return MAPF_OK;
+}
+
+extern "C" int mapf_evaluate_table(const mapf_ctx *ctx, const mapf_vtable *table, const int32_t *group_of,
+                                   const int32_t *tables, int64_t tables_len, int64_t n_episodes, int64_t max_steps,
+                                   double gamma, uint64_t seed, uint64_t step_index0, int64_t episode_offset,
+                                   void *scratch, double *ret, int32_t *length, uint8_t *outcome, uint8_t *conflict,
+                                   void *stream) {
+    VTableView vt = {};
+    int rc = vtable_view(ctx, "mapf_evaluate_table", table, &vt);
+    if (rc) return rc;
+    if (!group_of || !tables || n_episodes < 0 || (n_episodes > 0 && (!scratch || !ret || !length || !outcome)))
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_table: bad argument");
+    if (max_steps < 1 || max_steps >= (1ll << 31))
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_table: max_steps = %lld, must be in [1, 2**31)", (long long)max_steps);
+    if (n_episodes > MAPF_LAUNCH_MAX_ENVS)
+        return fail(MAPF_ERR_INVALID, "mapf_evaluate_table: at most 2**30 episodes per call");
+    GroupLayout gl;
+    u32 heads;
+    rc = group_layout(ctx, "mapf_evaluate_table", group_of, tables_len, &gl, &heads);
+    if (rc) return rc;
+    if (!ctx->philox_ok)
+        return fail(MAPF_ERR_UNSUPPORTED, "device-side sampling needs slip probabilities that add up to 1");
+    if (n_episodes == 0) return MAPF_OK;
+    DeviceGuard dg(ctx->device);
+    CUDA_TRY(cudaMemsetAsync(scratch, 0, sizeof(u32), (cudaStream_t)stream));
+    DevSpec sp = ctx->sp;
+    PhiloxKeys keys = make_keys(seed);
+    u32 E = (u32)n_episodes, T = (u32)max_steps;
+    u64 st = step_index0, e0 = (u64)episode_offset;
+    void *args[] = {&sp, &keys, &tables, &gl, &vt, &E, &T, &gamma, &st, &e0, &scratch, &ret, &length, &outcome, &conflict};
+    LAUNCH(ctx->ks.evaluate_table, grid_for(n_episodes, ctx->threads, ctx->grid_evaluate_table), ctx->threads,
+           ctx->smem_base, stream, args);
     return MAPF_OK;
 }
 

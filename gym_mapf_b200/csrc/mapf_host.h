@@ -24,6 +24,8 @@ struct KernelSet {
     const void *backup = nullptr, *backup_range = nullptr;  // k_backup<N, LUTS, RANGE>; one-word states only
     // by MAPF_POLICY_* kind: k_evaluate<N, W, LUTS, POLICY> for 0..2, k_evaluate_groups<N, W, LUTS> for 3
     const void *evaluate[4] = {nullptr, nullptr, nullptr, nullptr};
+    // RTDP over a value table (one-word states only): k_rtdp_backup<N, LUTS>, k_vtable_lookup<N>, k_evaluate_table<N, LUTS>
+    const void *rtdp_backup = nullptr, *vtable_lookup = nullptr, *evaluate_table = nullptr;
     const void *pred_count = nullptr, *pred_emit = nullptr, *project = nullptr;
     size_t expand_slab_bytes = 0;        // per warp
     int expand_threads = 0;              // CTA size of k_expand (0: the context's)

@@ -57,6 +57,9 @@ static void fill(KernelSet *k) {
     if (W == 1) {
         k->backup = (const void *)k_backup<N, LUTS, false>;
         k->backup_range = (const void *)k_backup<N, LUTS, true>;
+        k->rtdp_backup = (const void *)k_rtdp_backup<N, LUTS>;
+        k->vtable_lookup = (const void *)k_vtable_lookup<N>;
+        k->evaluate_table = (const void *)k_evaluate_table<N, LUTS>;
     }
     k->evaluate[0] = (const void *)k_evaluate<N, W, LUTS, 0>;
     if constexpr (W == 1) k->evaluate[1] = (const void *)k_evaluate<N, W, LUTS, 1>;  // policy indexed by the joint state

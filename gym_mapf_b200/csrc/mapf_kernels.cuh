@@ -1523,13 +1523,79 @@ __device__ __forceinline__ u32 clash_pair(const GroupLayout &gl, const int (&pre
     return cross != 0xffu ? cross : any;
 }
 
-// The episode loop of every policy kind.  `gl` and `conflict` are used by POLICY 3 only.  (The kernels' parameters
-// carry __restrict__; passing sp and keys by value and no qualifiers here keeps k_evaluate's machine code as it was
-// before this loop was shared.)
+// =====================================================================================================
+// The value table of RTDP (mapf_vtable): open addressing with linear probing, keyed by the one-word joint state
+// =====================================================================================================
+// `capacity` (a power of two) slots; a free slot holds VT_EMPTY, which no state equals (states are < 2**63).  Entries are
+// never deleted and at most capacity / 2 slots are ever occupied, so a probe sequence meets a free slot long before it
+// wraps; the probe loops are still bounded by the capacity, so that a table whose keys were never cleared cannot hang.
+#define VT_EMPTY 0xffffffffffffffffull
+#define VT_REFUSED 0x8000000000000000ull  // bit of the count word: a store was dropped for lack of room
+struct VTableView {
+    const u64 *keys;
+    const double *values;
+    const int *actions;
+    u64 mask;  // capacity - 1
+};
+
+// the splitmix64 finalizer: the home slot of a key is vt_hash(key) & mask
+__device__ __forceinline__ u64 vt_hash(u64 z) {
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+    return z ^ (z >> 31);
+}
+
+// the slot holding `key`, or -1
+__device__ __forceinline__ i64 vt_find(const VTableView &vt, u64 key) {
+    u64 slot = vt_hash(key) & vt.mask;
+    for (u64 i = 0; i <= vt.mask; ++i, slot = (slot + 1) & vt.mask) {
+        const u64 k = __ldg(vt.keys + slot);
+        if (k == key) return (i64)slot;
+        if (k == VT_EMPTY) break;
+    }
+    return -1;
+}
+
+// The additive group heuristic of a one-word state: 0.0 when s is terminal, else
+//     ((0.0 + V_0[l_0(s)]) + V_1[l_1(s)]) + ...      (groups in canonical order, single binary64 additions)
+// where l_g(s) is group g's local state and V_g its table at gl.off of the first agent of g.  `heads`: bit i is set when
+// agent i is the first agent of its group, so walking the agents in order visits the groups in canonical order.
+template <int N, bool EXACT>
+__device__ __forceinline__ double vt_heuristic(const DevSpec &sp, const GroupLayout &gl, const double *hv, u32 heads,
+                                               u64 s) {
+    int cell[N];
+    decode_state<N, 1, EXACT>(sp, s, 0ull, cell);
+    if (is_terminal<N>(sp, cell, s, 0ull)) return 0.0;
+    double h = 0.0;
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+        if ((heads >> i) & 1u) {
+            u64 x = gl.off[i];
+#pragma unroll
+            for (int j = 0; j < N; ++j) x += (u64)(u32)cell[j] * gl.mul[i][j];
+            h = __dadd_rn(h, __ldg(hv + x));
+        }
+    }
+    return h;
+}
+
+// value_of(s): the stored value when s is a key of the table, else the heuristic
+template <int N, bool EXACT>
+__device__ __forceinline__ double vt_value(const DevSpec &sp, const GroupLayout &gl, const double *hv, u32 heads,
+                                           const VTableView &vt, u64 s) {
+    const i64 slot = vt_find(vt, s);
+    return slot >= 0 ? __ldg(vt.values + slot) : vt_heuristic<N, EXACT>(sp, gl, hv, heads, s);
+}
+
+// The episode loop of every policy kind.  `gl` and `conflict` are used by POLICY 3 and 4 only, `vt` by POLICY 4 only.
+// (The kernels' parameters carry __restrict__; passing sp and keys by value and no qualifiers here keeps k_evaluate's
+// machine code as it was before this loop was shared.)
+//   POLICY 4 (MAPF_POLICY_TABLE)   the action stored with the state in a value table, else the POLICY 3 group action
 template <int N, int WORDS, bool LUTS, int POLICY>
 __device__ __forceinline__ void evaluate_episodes(DevSpec sp, PhiloxKeys keys, const void *policy, const GroupLayout *gl,
                                                   u32 E, u32 T, double gamma, u64 step0, u64 e0, u32 *counter,
-                                                  double *ret, int *length, u8 *outcome, u8 *conflict) {
+                                                  double *ret, int *length, u8 *outcome, u8 *conflict,
+                                                  const VTableView *vt = nullptr) {
     extern __shared__ __align__(16) unsigned char smem[];
     SmemTables tb = tables_begin<LUTS>(sp, smem);
     const u32 n_threads = gridDim.x * blockDim.x;
@@ -1549,21 +1615,31 @@ __device__ __forceinline__ void evaluate_episodes(DevSpec sp, PhiloxKeys keys, c
         bool ended = false;
         if (live) {
             const u64 env = e0 + (u64)e, stp = step0 + (u64)t;
-            if constexpr (POLICY == 3) {
+            if constexpr (POLICY == 3 || POLICY == 4) {
+                bool stored = false;
+                if constexpr (POLICY == 4) {
+                    const i64 slot = vt_find(*vt, in.lo);
+                    if (slot >= 0) {
+                        stored = true;
+                        load_actions<N>(sp, tb, (u32)__ldg(vt->actions + slot), in.actv);
+                    }
+                }
                 // Each agent indexes its own group's table with its group's local state (an unrolled N x N sum whose
                 // multipliers are 0 outside the group: no register array is indexed by a run-time group id) and takes
                 // its digit k of the entry v < 5**13 < 2**31: with f = v * ceil(2**64 / 5**(k + 1)) mod 2**64, f / 2**64
                 // is frac(v / 5**(k + 1)) + eps, eps < 2**-33, and 5 * (the top 32 bits of f, plus 1) / 2**32 has the
                 // digit as its integer part (the rounding stays below 1 / 5**k).
-                const int *tables = reinterpret_cast<const int *>(policy);
+                if (!stored) {
+                    const int *tables = reinterpret_cast<const int *>(policy);
 #pragma unroll
-                for (int i = 0; i < N; ++i) {
-                    u64 x = gl->off[i];
+                    for (int i = 0; i < N; ++i) {
+                        u64 x = gl->off[i];
 #pragma unroll
-                    for (int j = 0; j < N; ++j) x += (u64)(u32)in.cell[j] * gl->mul[i][j];
-                    const u32 v = min((u32)__ldg(tables + x), gl->amax[i]);
-                    const u32 fhi = (u32)(((u64)v * gl->frac[i]) >> 32);
-                    in.actv[i] = __umulhi(fhi + 1u, 5u) * 8u + tb.act0;
+                        for (int j = 0; j < N; ++j) x += (u64)(u32)in.cell[j] * gl->mul[i][j];
+                        const u32 v = min((u32)__ldg(tables + x), gl->amax[i]);
+                        const u32 fhi = (u32)(((u64)v * gl->frac[i]) >> 32);
+                        in.actv[i] = __umulhi(fhi + 1u, 5u) * 8u + tb.act0;
+                    }
                 }
             } else if (POLICY == 0) {
                 load_actions<N>(sp, tb, random_action(sp, keys, env, stp), in.actv);
@@ -1579,7 +1655,7 @@ __device__ __forceinline__ void evaluate_episodes(DevSpec sp, PhiloxKeys keys, c
             int nxt[N];
             // after a step that was not done the state is not terminal (see env_step): only step 0 needs the test
             const EnvOut o = env_step<N, WORDS, LUTS, false>(sp, tb, in, nullptr, 0u, nxt, t > 0);
-            if constexpr (POLICY == 3)  // the episode ends here: its conflict byte (MAPF_NO_CONFLICT unless a clash)
+            if constexpr (POLICY == 3 || POLICY == 4)  // the episode ends here: its conflict byte (MAPF_NO_CONFLICT unless a clash)
                 if (conflict && (o.kind != 0u || t + 1u == T))
                     conflict[e] = (u8)(o.kind == 1u ? clash_pair<N>(*gl, in.cell, nxt) : 0xffu);
             G = __dadd_rn(G, __dmul_rn(disc, o.reward));
@@ -1633,6 +1709,187 @@ k_evaluate_groups(DevSpec sp, PhiloxKeys keys, const int *__restrict__ tables, c
                   int *__restrict__ length, u8 *__restrict__ outcome, u8 *__restrict__ conflict) {
     evaluate_episodes<N, WORDS, LUTS, 3>(sp, keys, tables, &gl, E, T, gamma, step0, e0, counter, ret, length, outcome,
                                          conflict);
+}
+
+// MAPF_POLICY_TABLE (one-word states): the action stored with the state in the value table `vt`, else the group action
+// of `tables` exactly as k_evaluate_groups takes it.
+template <int N, bool LUTS>
+__global__ void __launch_bounds__(MAPF_MAX_THREADS, MAPF_MIN_BLOCKS(N))
+k_evaluate_table(DevSpec sp, PhiloxKeys keys, const int *__restrict__ tables, const __grid_constant__ GroupLayout gl,
+                 const __grid_constant__ VTableView vt, u32 E, u32 T, double gamma, u64 step0, u64 e0,
+                 u32 *__restrict__ counter, double *__restrict__ ret, int *__restrict__ length, u8 *__restrict__ outcome,
+                 u8 *__restrict__ conflict) {
+    evaluate_episodes<N, 1, LUTS, 4>(sp, keys, tables, &gl, E, T, gamma, step0, e0, counter, ret, length, outcome,
+                                     conflict, &vt);
+}
+
+// =====================================================================================================
+// RTDP: the Bellman update of B states over the value table, max over actions folded in
+// =====================================================================================================
+//   v_out[b] = max_a Q(s_b, a),  a_out[b] = the first a attaining it (np.argmax),
+//   Q(s, a) = 0; for ((p, c), s2, r, done) in P[s][a]:  Q += p * (r + gamma * value_of(s2))
+// with single binary64 operations in the row's order: k_backup's sum with V[s2] replaced by value_of(s2) (vt_value).
+// A warp takes G = max(1, 32 / nA) consecutive input states (rcp_nA = ceil(2**32 / nA) when G > 1) and walks their G * nA (state, action) rows 32 at a time,
+// rows generated from the row index; each pass is one k_backup batch (phase A, ordered per-row sums in the slab), after
+// which lane j folds the Q values of state j's rows in this pass into its running (max, first argmax).  No Q buffer
+// exists.  The table is only read, so a launch is a synchronous (Jacobi) update whatever the scheduling.
+// (The explicit one-CTA launch bound lets ptxas use the registers it needs: with the bare thread bound it spilled at
+// 1, 4, 5 and 8 agents at 32 to 64 registers.)
+template <int N, bool LUTS>
+__global__ void __launch_bounds__(MAPF_MAX_THREADS, 1)
+k_rtdp_backup(DevSpec sp, const u64 *__restrict__ states, i64 B, const __grid_constant__ GroupLayout gl,
+              const double *__restrict__ hv, u32 heads, const __grid_constant__ VTableView vt, double gamma, u32 G,
+              u32 rcp_nA, double *__restrict__ v_out, int *__restrict__ a_out) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    SmemTables tb = tables_begin<LUTS>(sp, smem);
+    const u32 FULL = 0xffffffffu;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const u32 lane_le = 0xffffffffu >> (31 - lane);
+    BackupSlab<N> &bs = reinterpret_cast<BackupSlab<N> *>(smem + MAPF_SMEM_LUT + staged_table_bytes<LUTS>(sp))[wid];
+    ExpandSlab<N> &sl = bs.sl;
+    const u32 nA = (u32)sp.nA;  // <= 5**13 < 2**31
+    const i64 stride = (i64)gridDim.x * (blockDim.x >> 5) * G;
+    tables_wait<LUTS>(smem);
+    for (i64 s_first = ((i64)blockIdx.x * (blockDim.x >> 5) + wid) * G; s_first < B; s_first += stride) {
+        const u32 n_s = B - s_first < (i64)G ? (u32)(B - s_first) : G;
+        const u32 rows = n_s * nA;
+        double best = 0.0;
+        int arg = -1;
+        for (u32 r0 = 0; r0 < rows; r0 += 32) {
+            const u32 r = r0 + (u32)lane;
+            const bool need = r < rows;
+            const u32 js = G == 1u ? 0u : __umulhi(r, rcp_nA);  // the lane's state within the group: r / nA (r < 32)
+            HeadCache hc;
+            hc.row = -1;
+            // the lane's (state, action) row, staged in slab words phase A does not use (the explicit-row source: no
+            // 64-bit division by nA per row as the RANGE source makes)
+            u64 *row_state = reinterpret_cast<u64 *>(bs.term);
+            int *row_action = reinterpret_cast<int *>(sl.pref);
+            if (need) {
+                row_state[lane] = states[s_first + js];
+                row_action[lane] = (int)(r - js * nA);
+            }
+            const u32 len = need ? expand_row_setup<N, 1, LUTS, false>(sp, tb, sl, lane, row_state, row_action, 0ull, 0ull,
+                                                                       (i64)lane)
+                                 : 0u;
+            u32 incl = len;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const u32 y = __shfl_up_sync(FULL, incl, o);
+                if (lane >= o) incl += y;
+            }
+            const int total = (int)__shfl_sync(FULL, incl, 31);
+            const int myrel = (int)(incl - len), myend = (int)incl;
+            sl.pref[lane] = (u32)myrel;
+            __syncwarp();
+            double mine = 0.0;
+            int rows_before = 0;
+            for (int wrel = 0; wrel < total; wrel += 32) {
+                const bool inwin = need && myrel >= wrel && myrel < wrel + 32;
+                const u32 starts = __reduce_or_sync(FULL, inwin ? 1u << (myrel - wrel) : 0u);
+                const int row = rows_before + __popc(starts & lane_le) - 1;
+                rows_before += __popc(starts);
+                const int rel = wrel + lane;
+                if (rel < total) {
+                    const u32 flag = sl.flag[row];
+                    double term;
+                    if (flag & 1u) {  // the single record of a terminal state: (1.0, s, 0, True)
+                        const double v = vt_value<N, false>(sp, gl, hv, heads, vt, sl.st[0][row]);
+                        term = __dmul_rn(1.0, __dadd_rn(0.0, __dmul_rn(gamma, v)));
+                    } else {
+                        const RecordOut rec = expand_record_any<N, 1>(sp, tb, sl, row, flag, (u32)rel - sl.pref[row], hc);
+                        const double v = vt_value<N, false>(sp, gl, hv, heads, vt, rec.lo);
+                        term = __dmul_rn(rec.p, __dadd_rn(rec.reward, __dmul_rn(gamma, v)));
+                    }
+                    bs.term[lane] = term;
+                }
+                __syncwarp();
+                const int ja = (myrel > wrel ? myrel : wrel) - wrel, jb = (myend < wrel + 32 ? myend : wrel + 32) - wrel;
+                for (int j = ja; j < jb; ++j) mine = __dadd_rn(mine, bs.term[j]);
+                __syncwarp();
+            }
+            // fold: lane j takes the Q values of its state's rows in this pass, in action order
+            bs.term[lane] = mine;
+            __syncwarp();
+            if ((u32)lane < n_s) {
+                const u32 first = (u32)lane * nA, end = first + nA;
+                const u32 ja = first > r0 ? first - r0 : 0u;
+                const u32 jb = end <= r0 ? 0u : (end - r0 < 32u ? end - r0 : 32u);
+                for (u32 j = ja; j < jb; ++j) {
+                    const double q = bs.term[j];
+                    if (arg < 0 || q > best) {  // strictly greater: the first maximum stays
+                        best = q;
+                        arg = (int)(r0 + j - first);
+                    }
+                }
+            }
+            __syncwarp();
+        }
+        if ((u32)lane < n_s) {
+            v_out[s_first + lane] = best;
+            a_out[s_first + lane] = arg;
+        }
+    }
+}
+
+// Inserts or overwrites B (key, value, action) triples; the keys of one launch are distinct.  A thread that meets a free
+// slot first reserves one unit of the count word (refused, with VT_REFUSED set and the triple dropped, when capacity / 2
+// slots are already taken), then claims the slot with a 64-bit compare-and-swap on its key, probing on when another
+// thread claimed it first.  A key stored by an earlier launch lies before any free slot of its probe sequence and is
+// overwritten in place.
+static __global__ void __launch_bounds__(256)
+k_vtable_store(const u64 *__restrict__ states, i64 B, const double *__restrict__ v, const int *__restrict__ a,
+               u64 *keys, double *values, int *actions, u64 mask, u64 *count) {
+    const u64 limit = (mask + 1) >> 1;
+    unsigned long long *cnt = reinterpret_cast<unsigned long long *>(count);
+    for (i64 b = (i64)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (i64)gridDim.x * blockDim.x) {
+        const u64 key = states[b];
+        u64 slot = vt_hash(key) & mask;
+        bool reserved = false;
+        for (u64 i = 0; i <= mask; ++i, slot = (slot + 1) & mask) {
+            u64 k = *reinterpret_cast<volatile u64 *>(keys + slot);
+            if (k == VT_EMPTY) {
+                if (!reserved) {
+                    u64 c = *reinterpret_cast<volatile u64 *>(count);
+                    while ((c & ~VT_REFUSED) < limit) {
+                        const u64 prev = atomicCAS(cnt, c, c + 1);
+                        if (prev == c) { reserved = true; break; }
+                        c = prev;
+                    }
+                    if (!reserved) {
+                        atomicOr(cnt, VT_REFUSED);
+                        break;
+                    }
+                }
+                k = atomicCAS(reinterpret_cast<unsigned long long *>(keys + slot), VT_EMPTY, key);
+                if (k == VT_EMPTY) k = key;  // claimed
+            }
+            if (k == key) {
+                values[slot] = v[b];
+                actions[slot] = a[b];
+                break;
+            }
+        }
+    }
+}
+
+// value_of(s) and the stored action (-1 when s is not a key) of B states
+template <int N>
+__global__ void __launch_bounds__(256)
+k_vtable_lookup(DevSpec sp, const u64 *__restrict__ states, i64 B, const __grid_constant__ GroupLayout gl,
+                const double *__restrict__ hv, u32 heads, const __grid_constant__ VTableView vt,
+                double *__restrict__ v_out, int *__restrict__ a_out) {
+    for (i64 b = (i64)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (i64)gridDim.x * blockDim.x) {
+        const u64 s = states[b];
+        const i64 slot = vt_find(vt, s);
+        if (slot >= 0) {
+            v_out[b] = __ldg(vt.values + slot);
+            a_out[b] = __ldg(vt.actions + slot);
+        } else {
+            v_out[b] = vt_heuristic<N, false>(sp, gl, hv, heads, s);
+            a_out[b] = -1;
+        }
+    }
 }
 
 // =====================================================================================================

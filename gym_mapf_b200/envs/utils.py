@@ -110,11 +110,15 @@ def independent_policy(env: MapfEnv, gamma=1.0, eps=1e-6, max_iter=1000):
     return torch.stack(rows).contiguous()
 
 
-def _plan_group(env, group, gamma, eps, max_iter, slab):
+def _solve_group(env, group, gamma, eps, max_iter, slab):
     from .vec_env import VecMapfEnv
-    _, pi, _ = VecMapfEnv(get_local_view(env, list(group)), 1).value_iteration(gamma=gamma, eps=eps, max_iter=max_iter,
+    V, pi, _ = VecMapfEnv(get_local_view(env, list(group)), 1).value_iteration(gamma=gamma, eps=eps, max_iter=max_iter,
                                                                               slab=slab)
-    return pi
+    return V, pi
+
+
+def _plan_group(env, group, gamma, eps, max_iter, slab):
+    return _solve_group(env, group, gamma, eps, max_iter, slab)[1]
 
 
 def group_policy(env: MapfEnv, groups, gamma=1.0, eps=1e-6, max_iter=1000, slab=None):
@@ -125,6 +129,16 @@ def group_policy(env: MapfEnv, groups, gamma=1.0, eps=1e-6, max_iter=1000, slab=
     from .vec_env import GroupPolicy
     groups = [tuple(sorted(int(a) for a in g)) for g in groups]
     return GroupPolicy(groups, [_plan_group(env, g, gamma, eps, max_iter, slab) for g in groups])
+
+
+def group_values(env: MapfEnv, groups, gamma=1.0, eps=1e-6, max_iter=1000, slab=None):
+    """`group_policy` that also keeps each group's values: the same per-group `value_iteration`, returned as
+    GroupValues(groups, values, policy) with values[g] = V of `get_local_view(env, g)` (float64[L**|g|]) and `policy`
+    equal to `group_policy(env, groups, ...)`.  The heuristic of `VecMapfEnv.rtdp`."""
+    from .vec_env import GroupPolicy, GroupValues
+    groups = [tuple(sorted(int(a) for a in g)) for g in groups]
+    solved = [_solve_group(env, g, gamma, eps, max_iter, slab) for g in groups]
+    return GroupValues(groups, [V for V, _ in solved], GroupPolicy(groups, [pi for _, pi in solved]))
 
 
 IndependenceDetection = collections.namedtuple("IndependenceDetection", "policy resolved log")

@@ -90,6 +90,123 @@ class GroupPolicy(collections.namedtuple("GroupPolicy", "groups tables")):
         return out
 
 
+def _canonical_groups(groups):
+    """The groups as ascending agent tuples, and the order that sorts them by lowest agent; raises unless they
+    partition the agents 0..n-1."""
+    groups = [tuple(int(a) for a in g) for g in groups]
+    for g in groups:
+        if not g or any(a >= b for a, b in zip(g, g[1:])):
+            raise ValueError("the agents of a group must be distinct and ascending (got %s)" % (g,))
+    agents = sorted(a for g in groups for a in g)
+    if not groups or agents != list(range(len(agents))):
+        raise ValueError("the groups must partition the agents 0..n-1 (got %s)" % (groups,))
+    return groups, sorted(range(len(groups)), key=lambda k: groups[k][0])
+
+
+class GroupValues(collections.namedtuple("GroupValues", "groups values policy")):
+    """Values of agent groups planned apart, the additive heuristic of `VecMapfEnv.rtdp`.
+
+    `groups` partitions the agents as in GroupPolicy; `values[g]` is a float64[L**|g|] device tensor indexed by group g's
+    local state (the V `value_iteration` returns on `get_local_view(env, g)`); `policy` is the GroupPolicy of the same
+    groups (the fallback of the RTDP policy).  The heuristic of a joint state s is 0.0 when s is terminal, else
+    ((0.0 + values[0][l_0(s)]) + values[1][l_1(s)]) + ... in group order.  The constructor puts groups and values in
+    canonical order and rejects groups that do not partition the agents, values of the wrong dtype, shape or device,
+    and a policy over other groups."""
+    __slots__ = ()
+
+    def __new__(cls, groups, values, policy):
+        import torch
+        values = list(values)
+        if len(values) != len(groups):
+            raise ValueError("GroupValues needs one value table per group (got %d groups, %d tables)"
+                             % (len(groups), len(values)))
+        groups, order = _canonical_groups(groups)
+        groups, values = tuple(groups[k] for k in order), [values[k] for k in order]
+        L, device = None, None
+        for g, v in zip(groups, values):
+            if not isinstance(v, torch.Tensor) or v.dtype is not torch.float64 or v.dim() != 1 or v.numel() == 0:
+                raise ValueError("the values of group %s must be a non-empty float64[L**%d] tensor" % (g, len(g)))
+            r = _int_root(v.numel(), len(g))
+            if r ** len(g) != v.numel() or (L is not None and r != L):
+                raise ValueError("the values of group %s have %d entries, not L**%d%s"
+                                 % (g, v.numel(), len(g), "" if L is None else " = %d" % L ** len(g)))
+            if device is not None and v.device != device:
+                raise ValueError("all value tables must be on one device (got %s and %s)" % (device, v.device))
+            L, device = r, v.device
+        if not isinstance(policy, GroupPolicy) or policy.groups != groups or policy.n_cells != L or \
+                policy.tables[0].device != device:
+            raise ValueError("the policy must be a GroupPolicy of the groups %s on %d cells on %s" % (groups, L, device))
+        return super().__new__(cls, groups, values, policy)
+
+
+class ValueTable:
+    """A device-resident value table for RTDP (C ABI `mapf_vtable`): `capacity` slots (a power of two, >= 64) of
+    (key = one-word joint state, float64 value, int32 greedy joint action), open addressing with linear probing, at
+    most capacity / 2 of them occupied.  Owns the five device tensors; the keys start as VTABLE_EMPTY."""
+
+    def __init__(self, engine, capacity):
+        capacity = int(capacity)
+        if capacity < 64 or capacity & (capacity - 1):
+            raise ValueError("capacity must be a power of two >= 64 (got %d)" % capacity)
+        if engine.words != 1:
+            raise ValueError("a value table is keyed by one-word states; this env's states take two words")
+        import torch
+        dev = engine.torch_device
+        self.engine, self.capacity = engine, capacity
+        self.keys = torch.full((capacity,), -1, dtype=torch.int64, device=dev)  # VTABLE_EMPTY as int64
+        self.values = torch.zeros(capacity, dtype=torch.float64, device=dev)
+        self.actions = torch.zeros(capacity, dtype=torch.int32, device=dev)
+        self.count = torch.zeros(1, dtype=torch.int64, device=dev)
+
+    def c_struct(self):
+        from .. import _native
+        return _native.MapfVtable(self.keys.data_ptr(), self.values.data_ptr(), self.actions.data_ptr(), self.capacity,
+                                  self.count.data_ptr())
+
+    def _count(self):
+        return int(self.count.item()) & ((1 << 64) - 1)
+
+    def __len__(self):
+        """Occupied slots (synchronises with the device)."""
+        return self._count() & ~(1 << 63)
+
+    def overflowed(self):
+        """True once a store was dropped because capacity / 2 slots were taken (synchronises with the device)."""
+        return bool(self._count() >> 63)
+
+    def lookup(self, states, heuristic):
+        """(values f64[B], actions i32[B]): the stored value of each state, or `heuristic`'s (GroupValues) when it is not
+        a key, and the stored action, or -1."""
+        return self.engine.vtable_lookup(states, heuristic, self)
+
+    def store(self, states, values, actions):
+        """Stores (states[b], values[b], actions[b]); the states must be distinct."""
+        self.engine.vtable_store(states, values, actions, self)
+
+    def items(self):
+        """(keys int64[K], values, actions) of the occupied slots, sorted by key (for inspection)."""
+        occ = self.keys != -1
+        keys, order = self.keys[occ].sort()
+        return keys, self.values[occ][order], self.actions[occ][order]
+
+
+class TablePolicy(collections.namedtuple("TablePolicy", "table fallback")):
+    """The policy of a value table: in a state that is a key of `table` (ValueTable) take the action stored with it,
+    anywhere else the action of `fallback` (GroupPolicy)."""
+    __slots__ = ()
+
+    def __new__(cls, table, fallback):
+        if not isinstance(table, ValueTable):
+            raise ValueError("table must be a ValueTable (got %s)" % type(table).__name__)
+        if not isinstance(fallback, GroupPolicy):
+            raise ValueError("fallback must be a GroupPolicy (got %s)" % type(fallback).__name__)
+        return super().__new__(cls, table, fallback)
+
+
+# rtdp: the value table, its TablePolicy (fallback: the heuristic's GroupPolicy) and one log record per iteration
+Rtdp = collections.namedtuple("Rtdp", "table policy log")
+
+
 def evaluation_summary(ev):
     """dict of the usual policy statistics of an Evaluation: mean / (population) standard deviation of the return, the
     shares of episodes that reached the goal, collided or ran out of steps, and the mean episode length."""
@@ -209,25 +326,26 @@ class VecMapfEnv:
         `max_steps` steps.  It draws from the Philox stream of `self.seed` (or `seed`) at `self.env_offset + e`, from
         step `self.step_count` on.  `policy`: None (uniformly random joint actions), int32[nS] joint actions by joint
         state (`value_iteration`'s policy), an integer [n_agents, L] table of per-agent actions by cell
-        (`independent_policy`), or a GroupPolicy (`group_policy`).  Returns an Evaluation; `self.states` and
+        (`independent_policy`), a GroupPolicy (`group_policy`) or a TablePolicy (`rtdp`).  Returns an Evaluation; `self.states` and
         `step_count` are left as they are."""
         out = self.engine.evaluate(policy, n_episodes, max_steps, gamma=gamma, seed=self.seed if seed is None else seed,
                                    step_index=self.step_count, episode_offset=self.env_offset)
         return Evaluation(*out)
 
     def find_conflicts(self, policy, n_episodes, max_steps, gamma=1.0, seed=None):
-        """`evaluate` of a GroupPolicy that also names, for every episode that ends in a collision, the pair of agents
+        """`evaluate` of a GroupPolicy or TablePolicy that also names, for every episode that ends in a collision, the pair of agents
         (i < j) that clashed on its last step: the lexicographically smallest pair of agents in different groups, else
         the smallest pair inside one group.  This is sampled: it sees the collisions of these episodes, not every
         reachable one.  Returns Conflicts(evaluation, pairs u8[E] (i | j << 4, or NO_CONFLICT), counts int64[n, n])."""
         from .. import _native
         torch = self._torch
-        if not isinstance(policy, GroupPolicy):
-            raise ValueError("find_conflicts needs a GroupPolicy (got %s)" % type(policy).__name__)
+        if not isinstance(policy, (GroupPolicy, TablePolicy)):
+            raise ValueError("find_conflicts needs a GroupPolicy or a TablePolicy (got %s)" % type(policy).__name__)
         E, n = int(n_episodes), self.n_agents
         pairs = torch.empty(max(E, 0), dtype=torch.uint8, device=self.device)
-        out = self.engine.evaluate_groups(policy, E, max_steps, gamma=gamma, seed=self.seed if seed is None else seed,
-                                          step_index=self.step_count, episode_offset=self.env_offset, conflicts=pairs)
+        run = self.engine.evaluate_table if isinstance(policy, TablePolicy) else self.engine.evaluate_groups
+        out = run(policy, E, max_steps, gamma=gamma, seed=self.seed if seed is None else seed,
+                  step_index=self.step_count, episode_offset=self.env_offset, conflicts=pairs)
         p = pairs[pairs != _native.NO_CONFLICT].long()
         counts = torch.bincount((p & 15) * n + (p >> 4), minlength=n * n).view(n, n)
         return Conflicts(Evaluation(*out), pairs, counts)
@@ -286,6 +404,76 @@ class VecMapfEnv:
             if delta <= eps:
                 break
         return V, pi, it
+
+    def rtdp(self, heuristic, n_trials, max_depth, max_iterations, gamma=1.0, eps=1e-6, capacity=1 << 24, seed=None):
+        """Real-time dynamic programming from the start state over a device-resident ValueTable, for joint spaces whose
+        values do not fit in memory (one-word states).  `heuristic` (GroupValues) values every state the table does not
+        hold.  The run is exactly
+            every trial t in [0, n_trials) starts at s0
+            for it in range(max_iterations):
+                residual = 0
+                for d in range(max_depth):
+                    S = the distinct states of the live trials, sorted
+                    v, a = rtdp_backup(S); old = lookup(S).values      (both read the table before the store)
+                    residual = max(residual, max |v - old|); store(S, v, a)
+                    every live trial steps with the a of its state (Philox stream `seed` (default self.seed), step
+                        index it * max_depth + d, env index t, no auto-reset); one whose next state is terminal
+                        (two agents on one cell, or every agent on its goal) stops for this iteration
+                log one record; raise if the table overflowed
+                if residual <= eps: stop
+        A trial runs on through a done that is not terminal (a swap clash ends on distinct cells): in the MDP that
+        `value_iteration` solves such a state keeps its future value.
+        The value of s0 converges to the optimum V*(s0) only when the heuristic is optimistic, h >= V* at every state;
+        under SoC with `reward_of_clash` below any path cost, the sum of the single-agent values (`group_values` of
+        singleton groups) is such a heuristic.
+        Returns Rtdp(table, policy = TablePolicy(table, heuristic.policy), log), one log record per iteration:
+        {"residual", "v_s0", "table_size", "backups" (states backed up), "seconds"}."""
+        import time
+        torch = self._torch
+        eng = self.engine
+        if not isinstance(heuristic, GroupValues):
+            raise ValueError("the heuristic must be a GroupValues (got %s)" % type(heuristic).__name__)
+        n_trials, max_depth, max_iterations = int(n_trials), int(max_depth), int(max_iterations)
+        if n_trials < 1 or max_depth < 1 or max_iterations < 1:
+            raise ValueError("n_trials, max_depth and max_iterations must be >= 1")
+        seed = self.seed if seed is None else int(seed)
+        table = ValueTable(eng, capacity)
+        s0 = eng.states_from_ints([eng.s0])
+        goal = int(eng.goal_state)
+        log = []
+        for it in range(max_iterations):
+            t_start = time.perf_counter()
+            states = s0.repeat(n_trials)
+            live = torch.ones(n_trials, dtype=torch.bool, device=self.device)
+            residual = torch.zeros((), dtype=torch.float64, device=self.device)
+            backups = 0
+            for d in range(max_depth):
+                idx = live.nonzero().squeeze(1)
+                if idx.numel() == 0:
+                    break
+                S, inv = torch.unique(states[idx], sorted=True, return_inverse=True)
+                v, a = eng.rtdp_backup(S, heuristic, table, gamma)
+                old, _ = eng.vtable_lookup(S, heuristic, table)
+                residual = torch.maximum(residual, (v - old).abs().max())
+                eng.vtable_store(S, v, a, table)
+                backups += S.numel()
+                actions = torch.zeros(n_trials, dtype=torch.int32, device=self.device)
+                actions[idx] = a[inv]
+                ns = eng.step(states, actions, seed=seed, step_index=it * max_depth + d, env_offset=0)[0]
+                states = torch.where(live, ns, states)
+                cells = eng.decode(ns).sort(dim=1).values
+                terminal = (ns == goal) | (cells[:, 1:] == cells[:, :-1]).any(dim=1)
+                live = live & ~terminal
+            res = float(residual.item())
+            v_s0 = float(eng.vtable_lookup(s0, heuristic, table)[0].item())
+            if table.overflowed():
+                raise RuntimeError("rtdp: the value table of capacity %d is full (more than %d states); pass a larger "
+                                   "capacity" % (table.capacity, table.capacity // 2))
+            log.append(dict(residual=res, v_s0=v_s0, table_size=len(table), backups=backups,
+                            seconds=time.perf_counter() - t_start))
+            if res <= eps:
+                break
+        return Rtdp(table, TablePolicy(table, heuristic.policy), log)
 
     def predecessors(self, states):
         """(row_ptr, pred_states): the CSR of `MapfEnv.predecessors` (reference mapf_env.py:373-376) per state."""

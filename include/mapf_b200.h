@@ -182,7 +182,8 @@ enum {
     MAPF_POLICY_RANDOM = 0, /* a uniformly random joint action per step, drawn as mapf_rollout draws it (policy unused) */
     MAPF_POLICY_JOINT = 1,  /* int32 policy[policy_len], indexed by the joint state (policy_len >= nS; one-word states) */
     MAPF_POLICY_AGENTS = 2, /* uint8 policy[n_agents * L]: agent i on cell c intends action policy[i * L + c] */
-    MAPF_POLICY_GROUPS = 3  /* int32 tables of agent groups, one per group (mapf_evaluate_groups) */
+    MAPF_POLICY_GROUPS = 3, /* int32 tables of agent groups, one per group (mapf_evaluate_groups) */
+    MAPF_POLICY_TABLE = 4   /* the actions of a value table, group tables where it has none (mapf_evaluate_table) */
 };
 /* conflict[e] of mapf_evaluate_groups for an episode that did not end in a collision */
 #define MAPF_NO_CONFLICT 0xFF
@@ -272,6 +273,57 @@ int mapf_greedy(const mapf_ctx *ctx, const double *Q, int64_t n_states, double *
  * separate all-gather after the sweep.  The caller synchronises the ranks before the vector is read again. */
 int mapf_greedy_bcast(const mapf_ctx *ctx, const double *Q, int64_t n_states, int64_t s_begin, double *const *peer_values,
                       int32_t n_peers, int32_t *policy, void *stream);
+
+/* ---- real-time dynamic programming (RTDP) over a sparse value table; one-word states only ---------------------- */
+
+/* A value table: a HOST struct of DEVICE pointers, all owned by the caller (the library never allocates or frees them).
+ * Open addressing with linear probing over `capacity` slots keyed by the one-word joint state; the home slot of key s
+ * is splitmix64_finalizer(s) & (capacity - 1).  Entries are never deleted.  Before its first use the caller sets every
+ * key to MAPF_VTABLE_EMPTY and *count to 0.  *count holds the number of occupied slots; a store that would take more
+ * than capacity / 2 slots is dropped and sets bit 63 of *count (MAPF_VTABLE_REFUSED), which stays set.  The calls below
+ * are asynchronous on their stream: read *count after the stream has reached them. */
+#define MAPF_VTABLE_EMPTY 0xFFFFFFFFFFFFFFFFull
+#define MAPF_VTABLE_REFUSED 0x8000000000000000ull
+typedef struct mapf_vtable {
+    uint64_t *keys;     /* capacity slots; MAPF_VTABLE_EMPTY = free */
+    double *values;     /* capacity: the value stored with the key */
+    int32_t *actions;   /* capacity: the greedy joint action stored with the value */
+    int64_t capacity;   /* a power of two, >= 64 */
+    uint64_t *count;    /* one word: occupied slots | MAPF_VTABLE_REFUSED once a store was dropped */
+} mapf_vtable;
+
+/* The heuristic of the table calls: group_of (HOST) and hvalues (DEVICE f64[hvalues_len]) follow mapf_evaluate_groups'
+ * group_of and tables -- canonical group ids, table_g of L**|g| doubles indexed by g's local state, concatenated in
+ * group order, hvalues_len = sum_g L**|g| -- with values in place of actions.  For a one-word state s
+ *     h(s) = 0.0 when s is terminal (two agents on one cell, or every agent on its goal), else
+ *     h(s) = ((0.0 + table_0[l_0(s)]) + table_1[l_1(s)]) + ...     (group order, single binary64 additions)
+ *     value_of(s) = the value stored with s when s is a key of the table, else h(s).
+ * Rejected (MAPF_ERR_INVALID) by every call below: a NULL table or table pointer, a capacity that is not a power of two
+ * or is below 64, B < 0, NULL or misaligned (not 8-byte) state arrays, the group_of / length errors of
+ * mapf_evaluate_groups.  A context whose states take two words is MAPF_ERR_UNSUPPORTED. */
+
+/* The Bellman update of B states over the table, with the max over actions folded in (no Q buffer exists):
+ *     v_out[b] = max_a Q(states[b], a),  a_out[b] = the first action attaining it (np.argmax)
+ *     Q(s, a) = 0;  for ((p, collision), s2, r, done) in P[s][a]:  Q += p * (r + gamma * value_of(s2))
+ * every operation one IEEE binary64 operation in this order (mapf_backup's sum with V[s2] replaced by value_of(s2)).
+ * The table is only read: the outputs do not depend on how the launch is scheduled. */
+int mapf_rtdp_backup(const mapf_ctx *ctx, const void *states, int64_t B, const int32_t *group_of, const double *hvalues,
+                     int64_t hvalues_len, const mapf_vtable *table, double gamma, double *v_out, int32_t *a_out,
+                     void *stream);
+/* Stores (states[b], v[b], a[b]) for b < B, overwriting the value and action of a key that is already present.  The
+ * states of one call must be distinct.  Stores that do not fit are dropped as described at mapf_vtable. */
+int mapf_vtable_store(const mapf_ctx *ctx, const void *states, int64_t B, const double *v, const int32_t *a,
+                      const mapf_vtable *table, void *stream);
+/* v_out[b] = value_of(states[b]); a_out[b] = the action stored with states[b], or -1 when it is not a key. */
+int mapf_vtable_lookup(const mapf_ctx *ctx, const void *states, int64_t B, const int32_t *group_of, const double *hvalues,
+                       int64_t hvalues_len, const mapf_vtable *table, double *v_out, int32_t *a_out, void *stream);
+/* mapf_evaluate_groups with the MAPF_POLICY_TABLE policy: in state s an episode takes the action stored with s when s
+ * is a key of the table, else the group action of `tables` exactly as mapf_evaluate_groups takes it.  Draws, queue,
+ * scratch, ret / length / outcome and conflict are those of mapf_evaluate_groups, and so are its rejections. */
+int mapf_evaluate_table(const mapf_ctx *ctx, const mapf_vtable *table, const int32_t *group_of, const int32_t *tables,
+                        int64_t tables_len, int64_t n_episodes, int64_t max_steps, double gamma, uint64_t seed,
+                        uint64_t step_index0, int64_t episode_offset, void *scratch, double *ret, int32_t *length,
+                        uint8_t *outcome, uint8_t *conflict, void *stream);
 
 /* MapfEnv.predecessors (mapf_env.py:373-376, 414-434) for B states as CSR: row_len[b] = |predecessors(states[b])|;
  * after mapf_scan_rows, pred[row_ptr[b] ..] holds the set (state_words * 8 bytes each, cartesian-product order with
